@@ -643,6 +643,26 @@ def blockcyclic_measurement(n, world, rank):
     return out
 
 
+DUMP_SAMPLES = 1 << 20
+
+
+def dump_outputs(directory, out, Kbuf, n, m, eta, flags):
+    """Writes what the last timed step of this rank computed as DIR/<name>.npy (float64), so that two builds can be
+    compared output for output. run_ours calls it on rank 0 only: under torchrun the files hold rank 0's last cell and
+    nothing from the other ranks. fused_out = the evaluator's out[] (logdet, traces, Gram matrices; include/gpgp.h), loglik_grad = the
+    (l^, d l^/d eta, d l^/d rho) a caller of ProfileLikelihood.log_likelihood_and_gradient gets from it, and
+    correlation_sample = the generated K at DUMP_SAMPLES (row, column) pairs drawn with numpy.random.RandomState(0)."""
+    import torch
+    from gaussian_proc._likelihood import ProfileLikelihood, _fused
+    os.makedirs(directory, exist_ok=True)
+    q = _fused.FusedQuantities(out, n, m, eta, flags)
+    ij = torch.from_numpy(numpy.random.RandomState(0).randint(0, n, size=(2, DUMP_SAMPLES))).cuda()
+    arrays = {'fused_out': out, 'loglik_grad': numpy.array(ProfileLikelihood._gradient_from(q, (n, m), True)),
+              'correlation_sample': Kbuf[ij[0], ij[1]].cpu().numpy()}
+    for name, a in arrays.items():
+        numpy.save(os.path.join(directory, name + '.npy'), numpy.ascontiguousarray(a, dtype=numpy.float64))
+
+
 # ---------------------------------------------------------------------------------------------------- GPU arm
 def run_ours(args):
     import torch
@@ -751,6 +771,9 @@ def run_ours(args):
     host = stacked.cpu().numpy()
     if not numpy.isfinite(host[:, :4]).all() or (host[:, 4] != 0).any():
         raise SystemExit('bench.py: non-finite result or Cholesky breakdown in the timed region')
+    if args.dump_outputs and rank == 0:
+        eta_last = cell((args.warmup + args.steps - 1) * world + rank)[0]
+        dump_outputs(args.dump_outputs, host[-1], slots[(counter[0] - 1) % C]['Kbuf'], n, m, eta_last, flags)
 
     value = args.steps * world / (ms * 1e-3)
 
@@ -889,7 +912,12 @@ def main():
                     help='independent evaluations kept in flight per GPU (own buffers and stream each)')
     ap.add_argument('--no-cpu', action='store_true', help='skip the cpu_baseline leg')
     ap.add_argument('--no-secondary', action='store_true', help='skip the sparse / sweep secondary measurements')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step computed to DIR/<name>.npy (float64, about 8 MB in all); under '
+                         'torchrun only rank 0 writes, so the files hold rank 0\'s last cell')
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the CUDA path (--impl ours)')
     if args.impl == 'reference':
         run_reference(args)
     else:

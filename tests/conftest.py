@@ -24,8 +24,18 @@ def golden_likelihood():
 
 @pytest.fixture(scope='session')
 def golden_generate():
+    """The dense matrices are exactly symmetric and stored as their packed lower triangles (`<key>_tril`, row-major
+    numpy.tril_indices order) to keep the file small; they are mirrored back to the full matrices here, bit for bit."""
     import numpy
-    return numpy.load(os.path.join(GOLDEN, 'golden_generate.npz'))
+    g = dict(numpy.load(os.path.join(GOLDEN, 'golden_generate.npz')))
+    for key in [k for k in g if k.endswith('_tril')]:
+        v = g.pop(key)
+        n = int(round((numpy.sqrt(8.0 * v.size + 1.0) - 1.0) / 2.0))
+        K = numpy.zeros((n, n))
+        K[numpy.tril_indices(n)] = v
+        K.T[numpy.tril_indices(n)] = v
+        g[key[:-len('_tril')]] = K
+    return g
 
 
 @pytest.fixture(scope='session')

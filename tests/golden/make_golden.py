@@ -114,6 +114,11 @@ def generate():
             S = quiet(cy.generate_sparse_correlation, p, numpy.array([0.03, 0.03]), nu, 0.01, False)
             key = 'sparse_%s_nu%g_' % (tag, nu)
             out[key + 'indptr'], out[key + 'indices'], out[key + 'data'] = S.indptr, S.indices, S.data
+    # the dense matrices are exactly symmetric: keep the packed lower triangles (tests/conftest.py mirrors them back)
+    for key in [k for k in out if k.startswith('dense')]:
+        K = out.pop(key)
+        assert (K == K.T).all()
+        out[key + '_tril'] = K[numpy.tril_indices(K.shape[0])]
     numpy.savez_compressed(os.path.join(HERE, 'golden_generate.npz'), **out)
     print('golden_generate.npz', len(out), 'arrays')
 

@@ -62,16 +62,24 @@ def test_bad_arguments_are_rejected_before_any_launch():
 
 
 def test_no_cpu_fallback():
-    """The product must fail loudly without a CUDA device (and must never import the oracle)."""
-    import torch
-    from gaussian_proc import _device as dev
-    if torch.cuda.is_available():
-        pytest.skip('GPU present')
-    import numpy
-    import gaussian_proc
-    with pytest.raises(dev.GpgpError):
-        gaussian_proc.generate_correlation(numpy.random.rand(10, 2))
+    """The product must fail loudly without a CUDA device (and must never import the oracle). The call runs in a child
+    process that is shown no device, so that the check holds on a machine with a GPU as well."""
+    import subprocess
+    import sys
     pkg = os.path.join(ROOT, 'gaussian-process-param-estimation_b200')
+    code = ('import sys\n'
+            'sys.path.insert(0, %r)\n'
+            'import numpy\n'
+            'import gaussian_proc\n'
+            'from gaussian_proc import _device as dev\n'
+            'try:\n'
+            '    gaussian_proc.generate_correlation(numpy.random.rand(10, 2))\n'
+            'except dev.GpgpError:\n'
+            '    sys.exit(0)\n'
+            'sys.exit("generate_correlation ran without a CUDA device")\n' % pkg)
+    res = subprocess.run([sys.executable, '-c', code], env=dict(os.environ, CUDA_VISIBLE_DEVICES=''),
+                         capture_output=True, text=True, timeout=600)
+    assert res.returncode == 0, res.stderr[-2000:]
     for base, _, files in os.walk(pkg):
         for f in files:
             if f.endswith(('.py', '.cu', '.cuh', '.h')):

@@ -1,8 +1,7 @@
 """CPU tests that PIN the oracle: the restatement in oracle/ against
   (A) numbers from the reference's shipped pickles (tests/golden/golden_pickles.npz),
   (B) vectors produced by the reference's own Python modules (tests/golden/golden_likelihood.npz),
-  (C) matrices produced by the reference's compiled Cython generators (tests/golden/golden_generate.npz),
-and, when oracle/_ref is built, live against the compiled reference itself."""
+  (C) matrices produced by the reference's compiled Cython generators (tests/golden/golden_generate.npz)."""
 
 import os
 
@@ -52,22 +51,6 @@ def test_sparse_csr_bit_identical(golden_generate, tag, nu):
 def test_sparse_density_too_small_raises():
     with pytest.raises(ValueError):
         matern.generate_sparse_correlation(numpy.random.rand(50, 2), 0.1, 0.5, 1e-3)   # density * n < 1
-
-
-def test_live_compiled_reference_if_built():
-    from oracle import ref_loader
-    try:
-        cy = ref_loader.load_cython()
-    except Exception:  # noqa: BLE001
-        pytest.skip('oracle/_ref not built')
-    numpy.random.seed(3)
-    p = numpy.random.rand(257, 2)
-    for nu in (0.5, 1.5, 2.5, 150.0):
-        assert (cy.generate_dense_correlation(p, numpy.array([0.07, 0.2]), nu, False)
-                == matern.generate_dense_correlation(p, numpy.array([0.07, 0.2]), nu)).all()
-    S1 = cy.generate_sparse_correlation(p, numpy.array([0.05, 0.05]), 1.5, 0.05, False)
-    S2 = matern.generate_sparse_correlation(p, 0.05, 1.5, 0.05)
-    assert (S1.indptr == S2.indptr).all() and (S1.indices == S2.indices).all() and (S1.data == S2.data).all()
 
 
 # ---- (B) likelihood vectors from the reference's own Python ---------------------------------------------------
