@@ -624,9 +624,11 @@ static int launch_tma_inst(double* C, int64_t ldc, const double* A, int64_t lda,
     if (tiles_m == 0 || tiles_n == 0) return 0;
     int rc = configure_once((const void*)dgemm_tma_kernel<AT, BT, BN_, WM_>, G::SMEM);
     if (rc) return rc;
+    // K == 0 (C = beta C): the driver refuses a zero extent, so the maps get a dummy one that no load touches (KT = 0)
+    const int Kmap = K > 0 ? K : 32;
     CUtensorMap mapA, mapB;
-    if ((rc = make_map(&mapA, AT, A, lda, M, K, BM))) return rc;
-    if ((rc = make_map(&mapB, BT, B, ldb, N, K, BN_))) return rc;
+    if ((rc = make_map(&mapA, AT, A, lda, M, Kmap, BM))) return rc;
+    if ((rc = make_map(&mapB, BT, B, ldb, N, Kmap, BN_))) return rc;
     cudaEvent_t e1 = profile_begin(tile_flops(tiles_m, tiles_n, BN_, K, krange, tmask), stream);
     dgemm_tma_kernel<AT, BT, BN_, WM_><<<tiles_m * tiles_n, G::THREADS, G::SMEM, stream>>>(
         mapA, mapB, C, ldc, tiles_m, tiles_n, K, alpha, beta, krange, tmask, kbeg_tab, kend_tab);
@@ -685,7 +687,7 @@ int launch_dgemm(int at, int bt, double* C, int64_t ldc, const double* A, int64_
 }
 
 // GEMM with per-row-tile k ranges: tile row tm (128 rows) uses k in [kbeg_tab[tm], kend_tab[tm]) (device int arrays, either
-// may be null). TMA kernel only.
+// may be null; entries multiples of 16, the k-slab of the kernel). TMA kernel only.
 int launch_dgemm_ktab(int at, int bt, double* C, int64_t ldc, const double* A, int64_t lda, const double* B, int64_t ldb,
                       int M, int N, int K, double alpha, double beta, const int* kbeg_tab, const int* kend_tab,
                       cudaStream_t stream) {
@@ -694,7 +696,6 @@ int launch_dgemm_ktab(int at, int bt, double* C, int64_t ldc, const double* A, i
     if (((uintptr_t)A | (uintptr_t)B | (uintptr_t)C) & 15) return -3;
     if (C == A || C == B) return -6;
     if (encode_init() != 1) return -7;
-    if (K == 0) K = 32;   // a zero k extent still has to scale C by beta: the tables (or kend = 0) keep the loop empty
     return launch_tma_bn<64, 64>(at, bt, C, ldc, A, lda, B, ldb, M, N, K, alpha, beta, KR_FULL, TM_ALL, stream, kbeg_tab, kend_tab);
 }
 

@@ -90,9 +90,12 @@ class NumpyOps(object):
         Bm = B.numpy().T if bt == 0 else B.numpy()          # K x N
         M, K = Am.shape
         assert M % 128 == 0 and C.shape[1] % 128 == 0 and K % 32 == 0 and Bm.shape == (K, C.shape[1])
+        # gp_dgemm_ktab_f64 takes table entries that are multiples of its 16-wide k-slab (include/gpgp.h)
+        for tab in (kbeg, kend):
+            assert tab is None or all(int(v) % 16 == 0 for v in tab), 'k tables must hold multiples of 16'
         prod = numpy.zeros((M, C.shape[1]))
         for t in range(M // 128):
-            kb = 0 if kbeg is None else min(int(kbeg[t]), K) // 16 * 16
+            kb = 0 if kbeg is None else min(int(kbeg[t]), K)
             ke = K if kend is None else min(int(kend[t]), K)
             if ke > kb:
                 prod[128 * t:128 * t + 128] = Am[128 * t:128 * t + 128, kb:ke] @ Bm[kb:ke]
