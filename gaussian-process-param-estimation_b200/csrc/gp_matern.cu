@@ -191,6 +191,67 @@ static int launch_cross(const double* prow, const double* pcol, const int* rg, c
     return 0;
 }
 
+// ---- cross-correlation P[i][j] = K(p_i, q_j) between two point sets (prediction at new points) ---------------------
+// Same distance expression and k order as matern_dense_kernel, so P(points, points) equals the dense K bit for bit.
+// Nothing can be mirrored: every 64 x 128 tile is evaluated. Entries with i >= n or j >= m are exactly 0.
+template <int MODE>
+__global__ void __launch_bounds__(256)
+matern_cross_points_kernel(const double* __restrict__ p, int n, const double* __restrict__ q, int m, int d, int64_t ldp,
+                           double* __restrict__ P, MaternParams mp) {
+    __shared__ double sr[MAXD][64];
+    __shared__ double sc[MAXD][128];
+    const int r0 = blockIdx.y * 64, c0 = blockIdx.x * 128, tid = threadIdx.x;
+    for (int idx = tid; idx < 64 * d; idx += 256) {
+        int r = idx / d, k = idx - r * d;
+        sr[k][r] = (r0 + r < n) ? p[(int64_t)(r0 + r) * d + k] : 0.0;
+    }
+    for (int idx = tid; idx < 128 * d; idx += 256) {
+        int r = idx / d, k = idx - r * d;
+        sc[k][r] = (c0 + r < m) ? q[(int64_t)(c0 + r) * d + k] : 0.0;
+    }
+    __syncthreads();
+    const int tx = tid & 31, ty = tid >> 5;   // tx: 4 consecutive columns; ty: rows ty + 8*rr
+    double cx[MAXD][4];
+#pragma unroll
+    for (int k = 0; k < MAXD; ++k)
+        if (k < d)
+#pragma unroll
+            for (int e = 0; e < 4; ++e) cx[k][e] = sc[k][tx * 4 + e];
+    for (int rr = ty; rr < 64; rr += 8) {
+        const int gi = r0 + rr;
+        double v[4];
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+            const int gj = c0 + tx * 4 + e;
+            double val = 0.0;
+            if (gi < n && gj < m) {
+                double s = 0.0;
+#pragma unroll
+                for (int k = 0; k < MAXD; ++k)
+                    if (k < d) {
+                        double t = (sr[k][rr] - cx[k][e]) * mp.inv_scale[k];
+                        s += t * t;
+                    }
+                val = matern_value<MODE>(sqrt(s), mp);
+            }
+            v[e] = val;
+        }
+        double* dst = P + (int64_t)gi * ldp + c0 + tx * 4;
+        reinterpret_cast<double2*>(dst)[0] = make_double2(v[0], v[1]);
+        reinterpret_cast<double2*>(dst)[1] = make_double2(v[2], v[3]);
+    }
+}
+
+template <int MODE>
+static int launch_cross_points(const double* p, int n, const double* q, int m, int d, int64_t ldp, double* P,
+                               const MaternParams& mp, cudaStream_t s) {
+    dim3 grid((unsigned)(gp_padded_size(m) / 128), (unsigned)(gp_padded_size(n) / 64));
+    matern_cross_points_kernel<MODE><<<grid, 256, 0, s>>>(p, n, q, m, d, ldp, P, mp);
+    GP_COUNT(1);
+    GP_LAUNCH_CHECK();
+    return 0;
+}
+
 }  // namespace gp
 
 extern "C" int gp_matern_dense(const double* points, int64_t n, int64_t d, const double* scale_host, double nu,
@@ -268,4 +329,32 @@ extern "C" int gp_matern_cross_dk(const double* prow, const double* pcol, const 
                                   int64_t nc, int64_t n, int64_t d, const double* scale_host, double nu, double* out,
                                   int64_t ld, void* stream) {
     return matern_cross_impl(prow, pcol, row_gidx, col_gidx, nr, nc, n, d, scale_host, nu, 0.0, out, ld, stream, true);
+}
+
+extern "C" int gp_matern_cross_points(const double* p, int64_t n, const double* q, int64_t m, int64_t d,
+                                      const double* scale_host, double nu, double* P, int64_t ldp, void* stream) {
+    using namespace gp;
+    if (!p || !q || !P || !scale_host || n <= 0 || m <= 0 || d <= 0 || d > MAXD) return -1;
+    int64_t npad = gp_padded_size(n), mpad = gp_padded_size(m);
+    if (ldp < mpad || (ldp & 1) || ((uintptr_t)P & 15) || npad > INT32_MAX || mpad > INT32_MAX) return -2;
+    MaternParams mp;
+    for (int k = 0; k < d; ++k) {
+        if (!(scale_host[k] > 0.0)) return -3;
+        mp.inv_scale[k] = 1.0 / scale_host[k];
+    }
+    mp.nu = nu; mp.coef = 0.0; mp.sq2nu = 0.0; mp.inv_rho = 1.0 / scale_host[0];
+    int mode = matern_mode_of(nu);
+    if (mode == MAT_GENERAL) {
+        if (!(nu > 0.0)) return -5;
+        mp.coef = pow(2.0, 1.0 - nu) / tgamma(nu);
+        mp.sq2nu = sqrt(2.0 * nu);
+    }
+    cudaStream_t s = (cudaStream_t)stream;
+    switch (mode) {
+        case MAT_05: return launch_cross_points<MAT_05>(p, (int)n, q, (int)m, (int)d, ldp, P, mp, s);
+        case MAT_15: return launch_cross_points<MAT_15>(p, (int)n, q, (int)m, (int)d, ldp, P, mp, s);
+        case MAT_25: return launch_cross_points<MAT_25>(p, (int)n, q, (int)m, (int)d, ldp, P, mp, s);
+        case MAT_GAUSS: return launch_cross_points<MAT_GAUSS>(p, (int)n, q, (int)m, (int)d, ldp, P, mp, s);
+        default: return launch_cross_points<MAT_GENERAL>(p, (int)n, q, (int)m, (int)d, ldp, P, mp, s);
+    }
 }

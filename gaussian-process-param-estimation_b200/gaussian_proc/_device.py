@@ -45,6 +45,9 @@ SIGNATURES = {
     'gp_gemm_profile_read': (_int, [_vp, _vp, _vp, _vp]),
     'gp_matern_dense': (_int, [_vp, _i64, _i64, _vp, _f64, _vp, _i64, _vp, _vp]),
     'gp_matern_cross': (_int, [_vp, _vp, _vp, _vp, _i64, _i64, _i64, _i64, _vp, _f64, _f64, _vp, _i64, _vp]),
+    'gp_matern_cross_points': (_int, [_vp, _i64, _vp, _i64, _i64, _vp, _f64, _vp, _i64, _vp]),
+    'gp_predict_workspace_bytes': (_i64, [_i64, _i64, _i64]),
+    'gp_predict_dense': (_int, [_vp, _i64, _i64, _vp, _i64, _vp, _i64, _i64, _vp, _i64, _vp, _vp, _vp]),
     'gp_kernel_threshold': (_int, [_i64, _i64, _f64, _vp, _f64, _vp]),
     'gp_sparse_workspace_bytes': (_i64, [_i64, _i64]),
     'gp_matern_sparse_count': (_int, [_vp, _vp, _i64, _i64, _vp, _f64, _f64, _vp, _vp, _vp, _vp]),

@@ -63,6 +63,13 @@ int gp_matern_cross(const double* prow, const double* pcol, const int* row_gidx,
 int gp_matern_cross_dk(const double* prow, const double* pcol, const int* row_gidx, const int* col_gidx, int64_t nr,
                        int64_t nc, int64_t n, int64_t d, const double* scale_host, double nu, double* out, int64_t ld,
                        void* stream);
+/* Cross-correlation between two point sets (prediction at new points): P[i][j] = matern(||(p_i - q_j) / scale||, nu) for the
+ * n points p (n, d) and the m points q (m, d), row-major npad x mpad (npad = gp_padded_size(n), mpad = gp_padded_size(m)),
+ * ldp >= mpad and even, P 16-byte aligned. Entries with i >= n or j >= m are exactly 0 (no identity padding); a zero
+ * distance gives exactly 1. The distance is evaluated like gp_matern_dense's, so P(points, points) equals its K bit for bit.
+ * scale_host: d entries (anisotropic allowed), d <= 8. */
+int gp_matern_cross_points(const double* p, int64_t n, const double* q, int64_t m, int64_t d, const double* scale_host,
+                           double nu, double* P, int64_t ldp, void* stream);
 
 /* ---- helpers of the distributed dense path (gaussian_proc/_blockcyclic.py; replaces what a ScaLAPACK-style build of the
  * reference's dposv / inverse would provide; the reference itself is single-node, _linear_solver.py:71) ---------------- */
@@ -361,6 +368,21 @@ int gp_loglik_dense(const double* K, int64_t n, int64_t npad, const double* R, i
  * out_dim[0] = tr(Kn^-1 dK/d scale[dim]), out_dim[1..] = S^T (dK/d scale[dim]) S. */
 int gp_loglik_dense_dscale(const double* Ainv, int64_t n, int64_t npad, int64_t p, const double* points, int64_t d,
                            const double* scale_host, double nu, int64_t dim, void* ws, double* out_dim, void* stream);
+
+/* ---------------------------------------------------------------------------------------------------------
+ * Kriging at new points (gaussian_proc/_predict.py; the reference has no prediction). For mc test points with
+ * cross block P = gp_matern_cross_points(training points, test points) and the factor of Kn = K + eta I:
+ *   V = W P                      (V: npad x mcpad, ldv; W = inv(L) from gp_trtri_f64, identity padding)
+ *   out[j*(p+1) + c] = P[:, j]^T S[:, c]  for c < p,    out[j*(p+1) + p] = ||V[:, j]||^2      (j < mc)
+ * S = Kn^-1 [X z] (npad x p, ld = p, rows >= n zero; gp_potrs_f64), p = m + 1 <= 16. mcpad = ceil(mc / 128) * 128; P and V
+ * have ld >= mcpad (even) and P's columns mc .. mcpad zero, as gp_matern_cross_points leaves them. A column's results do
+ * not depend on mc (fixed-order reduction over 2048-row chunks). ws: gp_predict_workspace_bytes(npad, mc, p) bytes
+ * (-1 for invalid sizes). No host synchronisation. The host turns out[] into mean and variance; the covariance is
+ * K** - V^T V plus a rank-m term, two more gp_dgemm_f64 calls.
+ * ------------------------------------------------------------------------------------------------------- */
+int64_t gp_predict_workspace_bytes(int64_t npad, int64_t mc, int64_t p);
+int gp_predict_dense(const double* W, int64_t n, int64_t npad, const double* S, int64_t p, const double* P, int64_t mc,
+                     int64_t ldp, double* V, int64_t ldv, double* out, void* ws, void* stream);
 
 #ifdef __cplusplus
 }
