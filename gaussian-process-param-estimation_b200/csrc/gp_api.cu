@@ -25,8 +25,6 @@ int gp_dgemm_ktab_f64(int at, int bt, double* C, int64_t ldc, const double* A, i
                                  (cudaStream_t)stream);
 }
 
-int gp_gemm_set_impl(int impl) { return gp::set_gemm_impl(impl ? 1 : 0); }
-
 unsigned long long gp_launch_count(void) { return gp::g_launch_count.load(std::memory_order_relaxed); }
 
 int gp_gemm_profile_enable(int on) { return gp::profile_enable(on); }

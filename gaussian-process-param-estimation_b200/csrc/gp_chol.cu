@@ -11,7 +11,6 @@
 #include "../../include/gpgp.h"
 #include "gp_common.cuh"
 #include "gp_internal.h"
-#include <stdlib.h>
 #include <map>
 #include <mutex>
 #include <utility>
@@ -22,7 +21,7 @@ namespace gp {
 constexpr int DB = 128;         // diagonal block
 constexpr int DPITCH = DB + 1;  // shared pitch (odd -> conflict-free column walks)
 constexpr int DIAG_THREADS = 256;  // 255 registers per thread: the unrolled warp-level factorisation must not spill
-static int OUTER_NB = 512;   // outer panel width (multiple of 128); GP_POTRF_NB overrides it for tuning
+constexpr int OUTER_NB = 512;  // outer panel width (multiple of 128)
 
 // Factor the 128x128 diagonal block at `Ajj` (lower, in place) and write inv(L_jj) (lower, zero above) to `Linv`.
 //
@@ -530,13 +529,6 @@ int gp_potrf_f64(double* A, int64_t n, int64_t npad, int* info_dev, void* ws, vo
     if (int rc0 = configure_once((const void*)chol_diag_block_kernel, diag_smem)) return rc0;
     int rc = side_streams_init(s);
     if (rc) return rc;
-    static bool nb_read = false;
-    if (!nb_read) {
-        const char* e = getenv("GP_POTRF_NB");
-        int v = e ? atoi(e) : 0;
-        if (v >= DB && v % DB == 0) OUTER_NB = v;
-        nb_read = true;
-    }
     cudaStream_t ps = g_side.s[0];  // high-priority panel stream (look-ahead)
     GP_CUDA_CHECK(cudaMemsetAsync(info_dev, 0, sizeof(int), s));
     const int N = (int)npad;

@@ -24,16 +24,6 @@ namespace gp {
 extern std::atomic<unsigned long long> g_launch_count;
 #define GP_COUNT(k) (gp::g_launch_count.fetch_add((unsigned long long)(k), std::memory_order_relaxed))
 
-__device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src) {
-    unsigned s = (unsigned)__cvta_generic_to_shared(smem_dst);
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(s), "l"(gmem_src));
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() {
-    asm volatile("cp.async.wait_group %0;\n" ::"n"(N));
-}
-
 // FP64 tensor-core MMA, D(8x8) += A(8x4) * B(4x8); lowers to DMMA.8x8x4 on sm_100a.
 __device__ __forceinline__ void dmma884(double& d0, double& d1, double a, double b) {
     asm volatile(

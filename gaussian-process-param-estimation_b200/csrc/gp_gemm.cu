@@ -1,19 +1,24 @@
-// FP64 tensor-core (DMMA) GEMM for the Cholesky / inverse hot path.
+// FP64 tensor-core (DMMA) GEMM for the Cholesky / inverse hot path: C = beta C + alpha op(A) op(B).
 //
-// One 128 x BN output tile per CTA (BN = 64: 4 warps, two CTAs per SM; BN = 128: 8 warps), warp tile 64x32 built from
-// m8n8k4 DMMA fragments, k-slabs moved global->shared with cp.async through a multi-stage ring (measured: the per-slab
-// CTA barrier is the main loss against the raw DMMA issue rate, ~7 %; see Cfg below). Shared tiles are XOR-swizzled
-// so that both the 16-byte cp.async stores and the 8-byte fragment loads are bank-conflict free for
-// K-major ([mn][k]) as well as MN-major ([k][mn]) operands; this lets one kernel serve
+// One 128 x BN output tile per CTA, warp tile 64 x 32 built from m8n8k4 DMMA fragments. The k-slabs (16 deep) are moved
+// by ONE producer warp with cp.async.bulk.tensor (SASS: UTMALDG) into a ring of 128-byte-swizzled shared tiles guarded
+// by full/empty mbarriers, so the consumer warps never meet in a CTA barrier inside the main loop. Both operand layouts
+// are read bank-conflict free (see the shared layouts below), which lets one kernel serve
 //   NT: trailing SYRK/GEMM update and the panel TRSM-by-inverse   (potrf)
 //   NN: triangular products of the recursive inverse               (trtri)
 //   TN: W^T W                                                      (lauum)
 // Triangular operands are exploited by restricting each tile's k-range, never by element masks.
+//
+// Shared layouts (hardware SWIZZLE_128B: 16-byte chunk index ^= row & 7 inside 1024-byte groups):
+//   K-major operand  ([mn][k], T = 0): one 2-D box {16 k, ROWS mn}; row = mn (128 B each).
+//   MN-major operand ([k][mn], T = 1): ROWS/16 boxes of a 5-D view {16 mn, kbit1, kbit0, k>>3, kbit2} (2 KB each); the box
+//                    row is r = kbit1 | kbit0<<1 | kbit3<<2 | kbit2<<3.
+// Inside a slab of 16 k the MMA step kk (0..3) gives lane t (0..3) the logical k = (t&1) | kk<<1 | (t>>1)<<3 - the same
+// permutation for A and B, so the product is unchanged - which makes the 8-byte fragment loads of both layouts
+// bank-conflict free (each half-warp covers 16 distinct 8-byte bank groups).
 #include "gp_common.cuh"
 #include "gp_internal.h"
 #include <cuda.h>
-#include <stdlib.h>
-#include <string.h>
 #include <algorithm>
 #include <mutex>
 #include <set>
@@ -88,211 +93,17 @@ constexpr int BM = 128, WM = 64, WN = 32, MI = WM / 8, NI = WN / 8;
 constexpr int RASTER_GROUP = 8;
 
 // Two tile shapes share one kernel body:
-//   BN = 128: 8 warps, BK = 32 x 3 stages (192 KB), one CTA per SM. Needed where C aliases an operand (in-place panel
-//             solve: a CTA must own the full row block it overwrites).
-//   BN = 64 : 4 warps, BK = 16 x 4 stages (96 KB), TWO CTAs per SM: while one CTA sits in its per-slab barrier, its
-//             prologue or its C read-modify-write epilogue, the other keeps the FP64 tensor pipe busy.
+//   BN = 64 : 4 consumer warps, 4 stages (96 KB), TWO CTAs per SM: while one CTA sits in its prologue or its C
+//             read-modify-write epilogue, the other keeps the FP64 tensor pipe busy. Every product but the one below.
+//   BN = 128: 8 consumer warps, 6 stages (192 KB), one CTA per SM. Only for the in-place panel solve, where C aliases A
+//             and a CTA must own the full row block it overwrites (see check_args).
 template <int BN_>
-struct Cfg {
-    static constexpr int BN = BN_;
-    static constexpr int BK = (BN_ == 128) ? 32 : 16;
-    static constexpr int STAGES = (BN_ == 128) ? 3 : 4;
-    static constexpr int WARPS_N = BN_ / WN;
-    static constexpr int THREADS = (BM / WM) * WARPS_N * 32;
-    static constexpr int A_ELEMS = BM * BK, B_ELEMS = BN_ * BK, STAGE_ELEMS = A_ELEMS + B_ELEMS;
-    static constexpr int SMEM = STAGES * STAGE_ELEMS * (int)sizeof(double);
-    static constexpr int MIN_CTAS = (BN_ == 128) ? 1 : 2;
-};
-
-// shared-memory offset (in doubles) of logical element (mn, k) of an operand tile with ROWS mn-rows
-template <int T, int ROWS, int BK>
-__device__ __forceinline__ int soff(int mn, int k) {
-    if (T == 0) return mn * BK + (((k >> 2) ^ (mn & 3)) << 2) + (k & 3);  // [ROWS][BK], 4-double chunks swizzled by row
-    return k * ROWS + (mn ^ ((k & 3) << 2));                               // [BK][ROWS], mn bits 2..3 swizzled by k
-}
-
-// copy one operand tile (ROWS mn x BK k) into shared memory; g points at logical element (mn0, k0)
-template <int T, int ROWS, int BK, int THREADS>
-__device__ __forceinline__ void load_tile(double* tile, const double* g, int64_t ld, int tid) {
-    constexpr int CHUNKS = ROWS * BK / 2;
-#pragma unroll
-    for (int i = 0; i < CHUNKS / THREADS; ++i) {
-        int idx = tid + i * THREADS;
-        if (T == 0) {
-            int r = idx / (BK / 2), c = idx % (BK / 2);  // row r, 16-byte chunk c (k = 2c, 2c+1)
-            cp_async16(tile + r * BK + ((c >> 1) ^ (r & 3)) * 4 + ((c & 1) << 1), g + (int64_t)r * ld + 2 * c);
-        } else {
-            int kr = idx / (ROWS / 2), c = idx % (ROWS / 2);  // k-row kr, chunk c (mn = 2c, 2c+1)
-            cp_async16(tile + kr * ROWS + ((2 * c) ^ ((kr & 3) << 2)), g + (int64_t)kr * ld + 2 * c);
-        }
-    }
-}
-
-template <int AT, int BT, int BN_>
-__global__ void __launch_bounds__(Cfg<BN_>::THREADS, Cfg<BN_>::MIN_CTAS)
-dgemm_dmma_kernel(double* C, int64_t ldc, const double* A, int64_t lda, const double* B, int64_t ldb,
-                  int tiles_m, int tiles_n, int K, double alpha, double beta, int krange, int tmask) {
-    using G = Cfg<BN_>;
-    constexpr int BN = G::BN, BK = G::BK, STAGES = G::STAGES, THREADS = G::THREADS;
-    extern __shared__ __align__(16) double smem[];
-
-    // grouped rasterisation: RASTER_GROUP tile-rows share each B tile while it is hot in L2
-    int bid = blockIdx.x;
-    int group_sz = RASTER_GROUP * tiles_n;
-    int grp = bid / group_sz;
-    int first_m = grp * RASTER_GROUP;
-    int rows_in_grp = min(RASTER_GROUP, tiles_m - first_m);
-    int rem = bid - grp * group_sz;
-    int tm = first_m + rem % rows_in_grp;
-    int tn = rem / rows_in_grp;
-    const int m0 = tm * BM, n0 = tn * BN;
-    if (tmask == TM_LOWER && n0 >= m0 + BM) return;
-
-    int kbeg = 0, kend = K;
-    if (krange == KR_A_LOWER) kend = min(K, m0 + BM);
-    else if (krange == KR_B_LOWER) kbeg = min(n0, K);
-    else if (krange == KR_TN_LOWER) kbeg = min(max(m0, n0), K);
-    kbeg = (kbeg / BK) * BK;
-    const int KT = (kend - kbeg) / BK;
-
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int g = lane >> 2, t = lane & 3;
-    const int wm = (warp / G::WARPS_N) * WM, wn = (warp % G::WARPS_N) * WN;
-
-    const double* Ag = (AT == 0) ? A + (int64_t)m0 * lda + kbeg : A + (int64_t)kbeg * lda + m0;
-    const double* Bg = (BT == 0) ? B + (int64_t)n0 * ldb + kbeg : B + (int64_t)kbeg * ldb + n0;
-    const int64_t a_step = (AT == 0) ? BK : (int64_t)BK * lda;
-    const int64_t b_step = (BT == 0) ? BK : (int64_t)BK * ldb;
-
-    double acc[MI][NI][2];
-#pragma unroll
-    for (int i = 0; i < MI; ++i)
-#pragma unroll
-        for (int j = 0; j < NI; ++j) acc[i][j][0] = acc[i][j][1] = 0.0;
-
-    if (beta != 0.0) {
-        // the epilogue read-modify-writes a tile of C that streams from HBM: pull it into L2 now so those loads cost
-        // an L2 hit instead of a DRAM round trip each (128 rows x BN/16 lines of 128 B)
-        constexpr int LINES = BM * BN / 16;
-#pragma unroll
-        for (int i = 0; i < LINES / THREADS; ++i) {
-            int line = tid + i * THREADS;
-            const double* pc = C + (int64_t)(m0 + line / (BN / 16)) * ldc + n0 + ((line % (BN / 16)) << 4);
-            asm volatile("prefetch.global.L2 [%0];" ::"l"(pc));
-        }
-    }
-
-    // prologue: fill STAGES-1 slabs
-#pragma unroll
-    for (int s = 0; s < STAGES - 1; ++s) {
-        if (s < KT) {
-            load_tile<AT, BM, BK, THREADS>(smem + s * G::STAGE_ELEMS, Ag + s * a_step, lda, tid);
-            load_tile<BT, BN, BK, THREADS>(smem + s * G::STAGE_ELEMS + G::A_ELEMS, Bg + s * b_step, ldb, tid);
-        }
-        cp_async_commit();
-    }
-
-    for (int kt = 0; kt < KT; ++kt) {
-        cp_async_wait<STAGES - 2>();
-        __syncthreads();
-        {   // refill the slot consumed in the previous iteration
-            int nk = kt + STAGES - 1;
-            if (nk < KT) {
-                int s = nk % STAGES;
-                load_tile<AT, BM, BK, THREADS>(smem + s * G::STAGE_ELEMS, Ag + nk * a_step, lda, tid);
-                load_tile<BT, BN, BK, THREADS>(smem + s * G::STAGE_ELEMS + G::A_ELEMS, Bg + nk * b_step, ldb, tid);
-            }
-            cp_async_commit();
-        }
-        const double* As = smem + (kt % STAGES) * G::STAGE_ELEMS;
-        const double* Bs = As + G::A_ELEMS;
-#pragma unroll
-        for (int kk = 0; kk < BK / 4; ++kk) {
-            double a[MI], b[NI];
-#pragma unroll
-            for (int i = 0; i < MI; ++i) a[i] = As[soff<AT, BM, BK>(wm + i * 8 + g, kk * 4 + t)];
-#pragma unroll
-            for (int j = 0; j < NI; ++j) b[j] = Bs[soff<BT, BN, BK>(wn + j * 8 + g, kk * 4 + t)];
-#pragma unroll
-            for (int i = 0; i < MI; ++i)
-#pragma unroll
-                for (int j = 0; j < NI; ++j) dmma884(acc[i][j][0], acc[i][j][1], a[i], b[j]);
-        }
-    }
-    cp_async_wait<0>();
-
-    // epilogue: each thread owns (row, 2 consecutive cols) of every 8x8 fragment -> 16-byte accesses
-    const bool diag = (tmask == TM_LOWER) && (n0 + BN - 1 > m0);   // tile crosses the diagonal: mask col > row
-    if (beta != 0.0 && !diag) {
-        // full tile with accumulate: issue all loads of a row group before using them (memory-level parallelism)
-#pragma unroll
-        for (int i = 0; i < MI; i += 2) {
-            double2 o[2][NI];
-#pragma unroll
-            for (int ii = 0; ii < 2; ++ii)
-#pragma unroll
-                for (int j = 0; j < NI; ++j)
-                    o[ii][j] = *reinterpret_cast<const double2*>(C + (int64_t)(m0 + wm + (i + ii) * 8 + g) * ldc + n0 + wn + j * 8 + 2 * t);
-#pragma unroll
-            for (int ii = 0; ii < 2; ++ii)
-#pragma unroll
-                for (int j = 0; j < NI; ++j) {
-                    double2 v;
-                    v.x = alpha * acc[i + ii][j][0] + beta * o[ii][j].x;
-                    v.y = alpha * acc[i + ii][j][1] + beta * o[ii][j].y;
-                    *reinterpret_cast<double2*>(C + (int64_t)(m0 + wm + (i + ii) * 8 + g) * ldc + n0 + wn + j * 8 + 2 * t) = v;
-                }
-        }
-        return;
-    }
-#pragma unroll
-    for (int i = 0; i < MI; ++i) {
-        const int grow = m0 + wm + i * 8 + g;
-        double* crow = C + (int64_t)grow * ldc;
-#pragma unroll
-        for (int j = 0; j < NI; ++j) {
-            const int gcol = n0 + wn + j * 8 + 2 * t;
-            if (diag && gcol > grow) continue;
-            double2 v;
-            v.x = alpha * acc[i][j][0];
-            v.y = alpha * acc[i][j][1];
-            double2* p = reinterpret_cast<double2*>(crow + gcol);
-            if (beta != 0.0) {
-                double2 o = *p;
-                v.x += beta * o.x;
-                v.y += beta * o.y;
-            }
-            if (diag && gcol + 1 > grow) {
-                crow[gcol] = v.x;  // keep the strictly-upper neighbour untouched
-            } else {
-                *p = v;
-            }
-        }
-    }
-}
-
-
-// =====================================================================================================================
-// TMA + mbarrier variant (the default): the same tile shapes, warp tiles, k-range logic and epilogue, but the k-slabs
-// are moved by ONE producer warp with cp.async.bulk.tensor (SASS: UTMALDG) into a ring of 128-byte-swizzled shared tiles
-// guarded by full/empty mbarriers; the consumer warps never meet in a CTA barrier inside the main loop.
-//
-// Shared layouts (hardware SWIZZLE_128B: 16-byte chunk index ^= row & 7 inside 1024-byte groups):
-//   K-major operand  ([mn][k], T = 0): one 2-D box {16 k, ROWS mn}; row = mn (128 B each).
-//   MN-major operand ([k][mn], T = 1): ROWS/16 boxes of a 5-D view {16 mn, kbit1, kbit0, k>>3, kbit2} (2 KB each); the box
-//                    row is r = kbit1 | kbit0<<1 | kbit3<<2 | kbit2<<3.
-// Inside a slab of 16 k the MMA step kk (0..3) gives lane t (0..3) the logical k = (t&1) | kk<<1 | (t>>1)<<3 - the same
-// permutation for A and B, so the product is unchanged - which makes the 8-byte fragment loads of both layouts
-// bank-conflict free (each half-warp covers 16 distinct 8-byte bank groups).
-// =====================================================================================================================
-template <int BN_, int WM_>
 struct TCfg {
     static constexpr int BN = BN_;
     static constexpr int BK = 16;
     static constexpr int STAGES = (BN_ == 128) ? 6 : 4;
     static constexpr int WARPS_N = BN_ / WN;
-    static constexpr int WM = WM_, MI = WM_ / 8;         // warp tile WM x 32: 64 (2 warps / SM sub-partition at two CTAs per SM) or 32 (4)
-    static constexpr int CONSUMER_WARPS = (BM / WM_) * WARPS_N;
+    static constexpr int CONSUMER_WARPS = (BM / WM) * WARPS_N;
     static constexpr int THREADS = (CONSUMER_WARPS + 1) * 32;            // + the TMA producer warp
     static constexpr int A_BYTES = BM * BK * 8, B_BYTES = BN_ * BK * 8, STAGE_BYTES = A_BYTES + B_BYTES;
     static constexpr int SMEM = STAGES * STAGE_BYTES + 2048;   // tiles + 1 KB alignment slack + barriers (whole KB)
@@ -360,15 +171,16 @@ __device__ __forceinline__ double lds_f64(uint32_t addr) {
     return v;
 }
 
-template <int AT, int BT, int BN_, int WM_>
-__global__ void __launch_bounds__(TCfg<BN_, WM_>::THREADS, TCfg<BN_, WM_>::MIN_CTAS)
+template <int AT, int BT, int BN_>
+__global__ void __launch_bounds__(TCfg<BN_>::THREADS, TCfg<BN_>::MIN_CTAS)
 dgemm_tma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB, double* C, int64_t ldc,
                  int tiles_m, int tiles_n, int K, double alpha, double beta, int krange, int tmask,
                  const int* __restrict__ kbeg_tab, const int* __restrict__ kend_tab) {
-    using G = TCfg<BN_, WM_>;
-    constexpr int BN = G::BN, BK = G::BK, STAGES = G::STAGES, WM = G::WM, MI = G::MI;
+    using G = TCfg<BN_>;
+    constexpr int BN = G::BN, BK = G::BK, STAGES = G::STAGES;
     extern __shared__ __align__(16) unsigned char smem_raw[];
 
+    // grouped rasterisation: RASTER_GROUP tile-rows share each B tile while it is hot in L2
     int bid = blockIdx.x;
     int group_sz = RASTER_GROUP * tiles_n;
     int grp = bid / group_sz;
@@ -444,6 +256,8 @@ dgemm_tma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
         for (int j = 0; j < NI; ++j) acc[i][j][0] = acc[i][j][1] = 0.0;
 
     if (beta != 0.0) {
+        // the epilogue read-modify-writes a tile of C that streams from HBM: pull it into L2 now so those loads cost
+        // an L2 hit instead of a DRAM round trip each (128 rows x BN/16 lines of 128 B)
         constexpr int LINES = BM * BN / 16;
         constexpr int CT = G::CONSUMER_WARPS * 32;
 #pragma unroll
@@ -501,9 +315,10 @@ dgemm_tma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
         if (lane == 0) mbar_arrive_after(bars + 8 * (STAGES + s), dep);
     }
 
-    // epilogue (identical to the cp.async variant)
-    const bool diag = (tmask == TM_LOWER) && (n0 + BN - 1 > m0);
+    // epilogue: each thread owns (row, 2 consecutive cols) of every 8x8 fragment -> 16-byte accesses
+    const bool diag = (tmask == TM_LOWER) && (n0 + BN - 1 > m0);   // tile crosses the diagonal: mask col > row
     if (beta != 0.0 && !diag) {
+        // full tile with accumulate: issue all loads of a row group before using them (memory-level parallelism)
 #pragma unroll
         for (int i = 0; i < MI; i += 2) {
             double2 o[2][NI];
@@ -542,7 +357,7 @@ dgemm_tma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
                 v.y += beta * o.y;
             }
             if (diag && gcol + 1 > grow) {
-                crow[gcol] = v.x;
+                crow[gcol] = v.x;  // keep the strictly-upper neighbour untouched
             } else {
                 *p = v;
             }
@@ -592,37 +407,15 @@ static int make_map(CUtensorMap* map, int T, const double* P, int64_t ld, int mn
     return r == CUDA_SUCCESS ? 0 : -(int)r - 2000;
 }
 
-static int g_force_bn = -1;  // GP_GEMM_BN=64|128 overrides the tile-shape choice (tuning / A-B measurements)
-
 template <int AT, int BT, int BN_>
-static int launch_inst(double* C, int64_t ldc, const double* A, int64_t lda, const double* B, int64_t ldb,
-                       int M, int N, int K, double alpha, double beta, int krange, int tmask, cudaStream_t stream) {
-    using G = Cfg<BN_>;
-    if (K % G::BK) return -1;
-    int tiles_m = M / BM, tiles_n = N / BN_;
-    if (tiles_m == 0 || tiles_n == 0) return 0;
-    int rc = configure_once((const void*)dgemm_dmma_kernel<AT, BT, BN_>, G::SMEM);
-    if (rc) return rc;
-    cudaEvent_t e1 = profile_begin(tile_flops(tiles_m, tiles_n, BN_, K, krange, tmask), stream);
-    dgemm_dmma_kernel<AT, BT, BN_><<<tiles_m * tiles_n, G::THREADS, G::SMEM, stream>>>(
-        C, ldc, A, lda, B, ldb, tiles_m, tiles_n, K, alpha, beta, krange, tmask);
-    if (e1) cudaEventRecord(e1, stream);
-    GP_COUNT(1);
-    GP_LAUNCH_CHECK();
-    return 0;
-}
-
-static int g_impl = -1;      // GP_GEMM_IMPL=cpasync selects the older cp.async kernel (A-B measurements); default: TMA
-
-template <int AT, int BT, int BN_, int WM_>
 static int launch_tma_inst(double* C, int64_t ldc, const double* A, int64_t lda, const double* B, int64_t ldb,
                            int M, int N, int K, double alpha, double beta, int krange, int tmask, cudaStream_t stream,
                            const int* kbeg_tab, const int* kend_tab) {
-    using G = TCfg<BN_, WM_>;
+    using G = TCfg<BN_>;
     if (K % G::BK) return -1;
     int tiles_m = M / BM, tiles_n = N / BN_;
     if (tiles_m == 0 || tiles_n == 0) return 0;
-    int rc = configure_once((const void*)dgemm_tma_kernel<AT, BT, BN_, WM_>, G::SMEM);
+    int rc = configure_once((const void*)dgemm_tma_kernel<AT, BT, BN_>, G::SMEM);
     if (rc) return rc;
     // K == 0 (C = beta C): the driver refuses a zero extent, so the maps get a dummy one that no load touches (KT = 0)
     const int Kmap = K > 0 ? K : 32;
@@ -630,7 +423,7 @@ static int launch_tma_inst(double* C, int64_t ldc, const double* A, int64_t lda,
     if ((rc = make_map(&mapA, AT, A, lda, M, Kmap, BM))) return rc;
     if ((rc = make_map(&mapB, BT, B, ldb, N, Kmap, BN_))) return rc;
     cudaEvent_t e1 = profile_begin(tile_flops(tiles_m, tiles_n, BN_, K, krange, tmask), stream);
-    dgemm_tma_kernel<AT, BT, BN_, WM_><<<tiles_m * tiles_n, G::THREADS, G::SMEM, stream>>>(
+    dgemm_tma_kernel<AT, BT, BN_><<<tiles_m * tiles_n, G::THREADS, G::SMEM, stream>>>(
         mapA, mapB, C, ldc, tiles_m, tiles_n, K, alpha, beta, krange, tmask, kbeg_tab, kend_tab);
     if (e1) cudaEventRecord(e1, stream);
     GP_COUNT(1);
@@ -638,68 +431,52 @@ static int launch_tma_inst(double* C, int64_t ldc, const double* A, int64_t lda,
     return 0;
 }
 
-template <int BN_, int WM_>
-static int launch_tma_bn(int at, int bt, double* C, int64_t ldc, const double* A, int64_t lda, const double* B, int64_t ldb,
-                         int M, int N, int K, double alpha, double beta, int krange, int tmask, cudaStream_t stream,
-                         const int* kbeg_tab = nullptr, const int* kend_tab = nullptr) {
-    if (at == 0 && bt == 0) return launch_tma_inst<0, 0, BN_, WM_>(C, ldc, A, lda, B, ldb, M, N, K, alpha, beta, krange, tmask, stream, kbeg_tab, kend_tab);
-    if (at == 0 && bt == 1) return launch_tma_inst<0, 1, BN_, WM_>(C, ldc, A, lda, B, ldb, M, N, K, alpha, beta, krange, tmask, stream, kbeg_tab, kend_tab);
-    if (at == 1 && bt == 1) return launch_tma_inst<1, 1, BN_, WM_>(C, ldc, A, lda, B, ldb, M, N, K, alpha, beta, krange, tmask, stream, kbeg_tab, kend_tab);
-    if (at == 1 && bt == 0) return launch_tma_inst<1, 0, BN_, WM_>(C, ldc, A, lda, B, ldb, M, N, K, alpha, beta, krange, tmask, stream, kbeg_tab, kend_tab);
+static int launch_tma_bn64(int at, int bt, double* C, int64_t ldc, const double* A, int64_t lda, const double* B, int64_t ldb,
+                           int M, int N, int K, double alpha, double beta, int krange, int tmask, cudaStream_t stream,
+                           const int* kbeg_tab, const int* kend_tab) {
+    if (at == 0 && bt == 0) return launch_tma_inst<0, 0, 64>(C, ldc, A, lda, B, ldb, M, N, K, alpha, beta, krange, tmask, stream, kbeg_tab, kend_tab);
+    if (at == 0 && bt == 1) return launch_tma_inst<0, 1, 64>(C, ldc, A, lda, B, ldb, M, N, K, alpha, beta, krange, tmask, stream, kbeg_tab, kend_tab);
+    if (at == 1 && bt == 1) return launch_tma_inst<1, 1, 64>(C, ldc, A, lda, B, ldb, M, N, K, alpha, beta, krange, tmask, stream, kbeg_tab, kend_tab);
+    if (at == 1 && bt == 0) return launch_tma_inst<1, 0, 64>(C, ldc, A, lda, B, ldb, M, N, K, alpha, beta, krange, tmask, stream, kbeg_tab, kend_tab);
     return -4;
 }
 
-template <int BN_>
-static int launch_bn(int at, int bt, double* C, int64_t ldc, const double* A, int64_t lda, const double* B, int64_t ldb,
-                     int M, int N, int K, double alpha, double beta, int krange, int tmask, cudaStream_t stream) {
-    if (at == 0 && bt == 0) return launch_inst<0, 0, BN_>(C, ldc, A, lda, B, ldb, M, N, K, alpha, beta, krange, tmask, stream);
-    if (at == 0 && bt == 1) return launch_inst<0, 1, BN_>(C, ldc, A, lda, B, ldb, M, N, K, alpha, beta, krange, tmask, stream);
-    if (at == 1 && bt == 1) return launch_inst<1, 1, BN_>(C, ldc, A, lda, B, ldb, M, N, K, alpha, beta, krange, tmask, stream);
-    if (at == 1 && bt == 0) return launch_inst<1, 0, BN_>(C, ldc, A, lda, B, ldb, M, N, K, alpha, beta, krange, tmask, stream);
-    return -4;
+// Argument checks shared by launch_dgemm and launch_dgemm_ktab, all made before any launch. Returns the tile width to
+// launch (64, or 128 for the in-place form below) or a negative error code.
+// The one aliased form allowed is the in-place panel solve of factor_panel (gp_chol.cu): C == A with the same leading
+// dimension, at = bt = 0, a single 128-wide column tile and no k tables. There each BN = 128 CTA reads exactly the row
+// block it overwrites. In every other aliased form CTAs read rows or columns that other CTAs write, and the result
+// would depend on their timing: -6.
+static int check_args(int at, int bt, const double* C, int64_t ldc, const double* A, int64_t lda, const double* B,
+                      int64_t ldb, int M, int N, int K, bool ktab) {
+    if (M < 0 || N < 0 || K < 0 || (M % BM) || (N % 128) || (K % 32)) return -1;
+    if ((lda & 1) || (ldb & 1) || (ldc & 1)) return -2;
+    if (((uintptr_t)A | (uintptr_t)B | (uintptr_t)C) & 15) return -3;
+    const bool in_place = !ktab && C == A && C != B && ldc == lda && at == 0 && bt == 0 && N == 128;
+    if ((C == A || C == B) && !in_place) return -6;
+    if (encode_init() != 1) return -7;
+    return in_place ? 128 : 64;
 }
 
 int launch_dgemm(int at, int bt, double* C, int64_t ldc, const double* A, int64_t lda, const double* B, int64_t ldb,
                  int M, int N, int K, double alpha, double beta, int krange, int tmask, cudaStream_t stream) {
-    if (M < 0 || N < 0 || K < 0 || (M % BM) || (N % 128) || (K % 32)) return -1;
-    if ((lda & 1) || (ldb & 1) || (ldc & 1)) return -2;
-    if (((uintptr_t)A | (uintptr_t)B | (uintptr_t)C) & 15) return -3;
-    if (g_force_bn < 0) {
-        const char* e = getenv("GP_GEMM_BN");
-        g_force_bn = e ? atoi(e) : 0;
-    }
-    // a CTA that overwrites an operand must own the whole row block it reads: the in-place panel solve needs BN = 128
-    bool aliased = (C == A) || (C == B);
-    int bn = aliased ? 128 : (g_force_bn == 128 ? 128 : 64);
-    if (g_impl < 0) {
-        const char* e = getenv("GP_GEMM_IMPL");
-        g_impl = (e && !strcmp(e, "cpasync")) ? 0 : 1;
-    }
-    if (g_impl == 1 && encode_init() == 1) {
-        static int wm32 = -1;     // GP_GEMM_WM=32: 32 x 32 warp tiles, 8 consumer warps per CTA (4 warps per sub-partition)
-        if (wm32 < 0) { const char* e = getenv("GP_GEMM_WM"); wm32 = (e && atoi(e) == 32) ? 1 : 0; }
-        if (bn == 128) return launch_tma_bn<128, 64>(at, bt, C, ldc, A, lda, B, ldb, M, N, K, alpha, beta, krange, tmask, stream);
-        if (wm32) return launch_tma_bn<64, 32>(at, bt, C, ldc, A, lda, B, ldb, M, N, K, alpha, beta, krange, tmask, stream);
-        return launch_tma_bn<64, 64>(at, bt, C, ldc, A, lda, B, ldb, M, N, K, alpha, beta, krange, tmask, stream);
-    }
-    if (bn == 128) return launch_bn<128>(at, bt, C, ldc, A, lda, B, ldb, M, N, K, alpha, beta, krange, tmask, stream);
-    return launch_bn<64>(at, bt, C, ldc, A, lda, B, ldb, M, N, K, alpha, beta, krange, tmask, stream);
+    const int bn = check_args(at, bt, C, ldc, A, lda, B, ldb, M, N, K, false);
+    if (bn < 0) return bn;
+    if (bn == 128)
+        return launch_tma_inst<0, 0, 128>(C, ldc, A, lda, B, ldb, M, N, K, alpha, beta, krange, tmask, stream, nullptr, nullptr);
+    return launch_tma_bn64(at, bt, C, ldc, A, lda, B, ldb, M, N, K, alpha, beta, krange, tmask, stream, nullptr, nullptr);
 }
 
 // GEMM with per-row-tile k ranges: tile row tm (128 rows) uses k in [kbeg_tab[tm], kend_tab[tm]) (device int arrays, either
-// may be null; entries multiples of 16, the k-slab of the kernel). TMA kernel only.
+// may be null; entries multiples of 16, the k-slab of the kernel).
 int launch_dgemm_ktab(int at, int bt, double* C, int64_t ldc, const double* A, int64_t lda, const double* B, int64_t ldb,
                       int M, int N, int K, double alpha, double beta, const int* kbeg_tab, const int* kend_tab,
                       cudaStream_t stream) {
-    if (M < 0 || N < 0 || K < 0 || (M % BM) || (N % 128) || (K % 32)) return -1;
-    if ((lda & 1) || (ldb & 1) || (ldc & 1)) return -2;
-    if (((uintptr_t)A | (uintptr_t)B | (uintptr_t)C) & 15) return -3;
-    if (C == A || C == B) return -6;
-    if (encode_init() != 1) return -7;
-    return launch_tma_bn<64, 64>(at, bt, C, ldc, A, lda, B, ldb, M, N, K, alpha, beta, KR_FULL, TM_ALL, stream, kbeg_tab, kend_tab);
+    const int bn = check_args(at, bt, C, ldc, A, lda, B, ldb, M, N, K, true);
+    if (bn < 0) return bn;
+    return launch_tma_bn64(at, bt, C, ldc, A, lda, B, ldb, M, N, K, alpha, beta, KR_FULL, TM_ALL, stream, kbeg_tab, kend_tab);
 }
 
-int set_gemm_impl(int impl) { g_impl = impl; return 0; }
 
 int profile_enable(int on) {
     g_prof.on = on != 0;

@@ -20,7 +20,8 @@ enum TileMask {
 // C[M x N] (row-major, ldc) = beta*C + alpha * op(A) * op(B)
 //   at == 0: A(m,k) = A[m*lda + k]   at == 1: A(m,k) = A[k*lda + m]
 //   bt == 0: B(k,n) = B[n*ldb + k]   bt == 1: B(k,n) = B[k*ldb + n]
-// M, N multiples of 128; K multiple of 32; all ld even; pointers 16-byte aligned.
+// M, N multiples of 128; K multiple of 32; all ld even; pointers 16-byte aligned. C may alias an operand only in the
+// in-place panel solve (C == A, lda == ldc, at == bt == 0, N == 128); any other aliasing returns -6.
 int launch_dgemm(int at, int bt, double* C, int64_t ldc, const double* A, int64_t lda,
                  const double* B, int64_t ldb, int M, int N, int K, double alpha, double beta,
                  int krange, int tmask, cudaStream_t stream);
@@ -32,7 +33,6 @@ int launch_dgemm_ktab(int at, int bt, double* C, int64_t ldc, const double* A, i
                       int M, int N, int K, double alpha, double beta, const int* kbeg_tab, const int* kend_tab,
                       cudaStream_t stream);
 
-int set_gemm_impl(int impl);   // 1 = TMA + mbarrier kernel (default), 0 = cp.async kernel (A-B measurements)
 int profile_enable(int on);
 int profile_read(double* ms_sum, double* ms_union, double* flops, long long* launches);
 

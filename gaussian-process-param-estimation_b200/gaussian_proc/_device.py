@@ -74,7 +74,6 @@ SIGNATURES = {
     'gp_dgemm_f64': (_int, [_int, _int, _vp, _i64, _vp, _i64, _vp, _i64, _i64, _i64, _i64, _f64, _f64, _int, _int,
                             _vp]),
     'gp_dgemm_ktab_f64': (_int, [_int, _int, _vp, _i64, _vp, _i64, _vp, _i64, _i64, _i64, _i64, _f64, _f64, _vp, _vp, _vp]),
-    'gp_gemm_set_impl': (_int, [_int]),
     'gp_matern_cross_dk': (_int, [_vp, _vp, _vp, _vp, _i64, _i64, _i64, _i64, _vp, _f64, _vp, _i64, _vp]),
     'gp_rect_apply': (_int, [_vp, _i64, _i64, _i64, _vp, _i64, _i64, _vp, _i64, _f64, _f64, _vp]),
     'gp_rect_workspace_bytes': (_i64, [_i64, _i64, _i64]),

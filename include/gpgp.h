@@ -135,7 +135,11 @@ int gp_csr_sort_rows(int64_t n, const int* indptr_dev, int* indices_dev, double*
 /* General DMMA GEMM used by everything below; exported for tests and the roofline microbenchmark.
  * C[MxN] = beta*C + alpha*op(A)*op(B); at/bt: 0 -> operand stored [mn][k], 1 -> stored [k][mn].
  * krange / tmask: see gp_internal.h (0 / 0 = plain GEMM). M,N multiples of 128, K multiple of 32; K == 0 gives
- * C = beta*C on the tiles tmask covers (beta == 0: C is not read). */
+ * C = beta*C on the tiles tmask covers (beta == 0: C is not read).
+ * C may alias an operand in one form only, the in-place C = beta*C + alpha*C*op(B) with C == A, ldc == lda,
+ * at == bt == 0 and N == 128 (a 128-wide block column, e.g. a Cholesky panel times an inverted diagonal block). Any
+ * other C == A or C == B returns -6 before anything is launched, since tiles would read what other tiles write.
+ * Returns -7 when the driver's tensor-map encoder (cuTensorMapEncodeTiled) is unavailable. */
 int gp_dgemm_f64(int at, int bt, double* C, int64_t ldc, const double* A, int64_t lda, const double* B,
                  int64_t ldb, int64_t M, int64_t N, int64_t K, double alpha, double beta, int krange, int tmask,
                  void* stream);
@@ -143,12 +147,10 @@ int gp_dgemm_f64(int at, int bt, double* C, int64_t ldc, const double* A, int64_
  * (DEVICE int arrays of M / 128 entries, either may be NULL): the staircase operands of the distributed inverse
  * (gaussian_proc/_blockcyclic.py). Table entries must be multiples of 16 (the kernel's k-slab; a kbeg is rounded down
  * to one and a partial slab before kend is dropped); a kbeg beyond K or a kend beyond K is clamped to K, and an empty
- * range (kend <= kbeg), like K == 0, gives C = beta*C for that row tile. C must not alias an operand. */
+ * range (kend <= kbeg), like K == 0, gives C = beta*C for that row tile. C must not alias an operand (-6). */
 int gp_dgemm_ktab_f64(int at, int bt, double* C, int64_t ldc, const double* A, int64_t lda, const double* B,
                       int64_t ldb, int64_t M, int64_t N, int64_t K, double alpha, double beta, const int* kbeg_tab,
                       const int* kend_tab, void* stream);
-/* developer switch for A-B measurements: 1 = TMA + mbarrier GEMM kernel (default), 0 = the cp.async kernel */
-int gp_gemm_set_impl(int impl);
 
 /* A (npad x npad, lower triangle referenced) := K + eta*I on the first n diagonal entries (padding diagonal
  * stays exactly 1); replaces `Kn = K + eta*I` of mixed_correlation.py:184,251,296. */

@@ -61,6 +61,25 @@ def test_bad_arguments_are_rejected_before_any_launch():
     assert dev.check(5, 'x') == 5
 
 
+def test_aliased_gemm_is_rejected_before_any_launch():
+    """C may alias an operand only as C == A with lda == ldc, at = bt = 0 and N = 128 (the in-place panel solve, where
+    each CTA owns the rows it overwrites). Every other aliased form returns -6 before anything is launched, so fake
+    16-byte-aligned pointers are never dereferenced."""
+    from gaussian_proc import _device as dev
+    lib = dev.lib
+    P, Q = ctypes.c_void_p(1 << 20), ctypes.c_void_p(2 << 20)
+
+    def gemm(at, bt, C, ldc, A, lda, B, N=128):
+        return lib.gp_dgemm_f64(at, bt, C, ldc, A, lda, B, 256, 256, N, 128, 1.0, 0.0, 0, 0, None)
+    assert gemm(0, 0, P, 256, Q, 256, P) == -6                 # C == B
+    assert gemm(1, 0, P, 256, P, 256, Q) == -6                 # at = 1
+    assert gemm(0, 1, P, 256, P, 256, Q) == -6                 # bt = 1
+    assert gemm(0, 0, P, 256, P, 256, Q, N=256) == -6          # two column tiles
+    assert gemm(0, 0, P, 256, P, 512, Q) == -6                 # ldc != lda
+    # the k-table entry point takes no aliased form at all
+    assert lib.gp_dgemm_ktab_f64(0, 0, P, 256, P, 256, Q, 256, 256, 128, 128, 1.0, 0.0, None, None, None) == -6
+
+
 def test_no_cpu_fallback():
     """The product must fail loudly without a CUDA device (and must never import the oracle). The call runs in a child
     process that is shown no device, so that the check holds on a machine with a GPU as well."""

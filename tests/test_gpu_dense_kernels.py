@@ -15,9 +15,6 @@ The tests marked gpu need a CUDA device; the unmarked ones check on the CPU that
 
 import ctypes
 import math
-import os
-import subprocess
-import sys
 
 import numpy
 import pytest
@@ -246,7 +243,7 @@ LAYOUTS = [(0, 0), (0, 1), (1, 0), (1, 1)]
 
 
 def gemm_suite(dev, cases=GEMM_CASES):
-    """every case in every operand layout (also run in child processes for the GP_GEMM_* variants)"""
+    """every case in every operand layout"""
     for i, case in enumerate(cases):
         M, N, K, alpha, beta, kr, tm, pad, off = case
         for at, bt in LAYOUTS:
@@ -267,56 +264,38 @@ def test_gemm_tma_default(cu):
 
 
 @gpu
-def test_gemm_cp_async_kernel(cu):
-    assert cu.lib.gp_gemm_set_impl(0) == 0
-    try:
-        gemm_suite(cu)
-    finally:
-        cu.lib.gp_gemm_set_impl(1)
-
-
-@gpu
-@pytest.mark.parametrize('impl', [1, 0])
-def test_gemm_in_place_panel_solve(cu, impl):
-    """factor_panel's panel solve L21 = A21 inv(L_jj)^T: C aliases A (the BN = 128 tile, a CTA owns its row block)"""
-    npad, j = 2048, 128
-    below = npad - (j + 128)
-    rng = numpy.random.default_rng(3)
-    full = numpy.full((npad, npad), numpy.nan)
-    full[j + 128:, j:j + 128] = int_matrix(rng, (below, 128))
-    Lj = int_matrix(rng, (128, 128))
-    want = full[j + 128:, j:j + 128] @ Lj.T
-    Ad, Ld = to_dev(full), to_dev(Lj)
-    assert cu.lib.gp_gemm_set_impl(impl) == 0
-    try:
-        A21 = dptr(Ad, (j + 128) * npad + j)
-        assert cu.lib.gp_dgemm_f64(0, 0, A21, npad, A21, npad, dptr(Ld), 128, below, 128, 128, 1.0, 0.0, KR_FULL, TM_ALL,
-                                   cu.stream_ptr()) == 0
-        got = to_host(Ad)
-    finally:
-        cu.lib.gp_gemm_set_impl(1)
-    assert_equal(got[j + 128:, j:j + 128], want, 'in-place panel solve')
+@pytest.mark.parametrize('tiles', [9, 17])
+@pytest.mark.parametrize('K', [32, 128, 512])
+@pytest.mark.parametrize('alpha,beta', [(1.0, 0.0), (-0.5, 0.25)])
+@pytest.mark.parametrize('pad', [0, 6])
+def test_gemm_in_place_panel_solve(cu, tiles, K, alpha, beta, pad):
+    """The one aliased form, C == A with a single 128-wide column tile (BN = 128: a CTA owns the row block it overwrites),
+    as factor_panel's panel solve L21 = A21 inv(L_jj)^T uses it: C is the first 128 of A's K columns. tiles: tile rows,
+    not a multiple of RASTER_GROUP; pad: extra columns of the leading dimension. Everything outside C (NaN around the
+    block, A's columns past 128) must be left as it was; with beta = 0 the columns of C past K hold NaN, never read."""
+    M, W = 128 * tiles, max(K, 128)
+    r0, c0 = 3, 2                                       # the block starts inside the matrix, 16 bytes into a row
+    ld = c0 + W + pad
+    rng = numpy.random.default_rng(tiles + K)
+    blk = int_matrix(rng, (M, W))
+    if beta == 0.0:
+        blk[:, K:] = numpy.nan
+    full = numpy.full((r0 + M + 2, ld), numpy.nan)
+    full[r0:r0 + M, c0:c0 + W] = blk
+    B = numpy.full((128, K + 2), numpy.nan)             # inv(L_jj) stored [n][k], two NaN padding columns
+    B[:, :K] = int_matrix(rng, (128, K))
+    want = alpha * (blk[:, :K] @ B[:, :K].T)
+    if beta != 0.0:
+        want += beta * blk[:, :128]
+    Ad = to_dev(full)
+    C = dptr(Ad, r0 * ld + c0)
+    assert cu.lib.gp_dgemm_f64(0, 0, C, ld, C, ld, dptr(to_dev(B)), K + 2, M, 128, K, alpha, beta, KR_FULL, TM_ALL,
+                               cu.stream_ptr()) == 0
+    got = to_host(Ad)
+    assert_equal(got[r0:r0 + M, c0:c0 + 128], want, 'in-place panel solve')
     rest = numpy.ones(got.shape, dtype=bool)
-    rest[j + 128:, j:j + 128] = False
-    assert numpy.isnan(got[rest]).all()
-
-
-@gpu
-@pytest.mark.parametrize('env', [{'GP_GEMM_BN': '128'}, {'GP_GEMM_WM': '32'}])
-def test_gemm_environment_variants(cu, env):
-    """GP_GEMM_BN / GP_GEMM_WM are read once per process: the whole suite runs in a child process with the variable set"""
-    here = os.path.dirname(os.path.abspath(__file__))
-    root = os.path.dirname(here)
-    code = ('import sys\n'
-            'sys.path[:0] = [%r, %r, %r]\n'
-            'import test_gpu_dense_kernels as t\n'
-            'from gaussian_proc import _device as dev\n'
-            'dev.require_cuda()\n'
-            't.gemm_suite(dev)\n'
-            'print("suite ok")\n' % (here, root, os.path.join(root, 'gaussian-process-param-estimation_b200')))
-    res = subprocess.run([sys.executable, '-c', code], env=dict(os.environ, **env), capture_output=True, text=True,
-                         timeout=1200)
-    assert res.returncode == 0 and 'suite ok' in res.stdout, (res.stdout[-2000:], res.stderr[-4000:])
+    rest[r0:r0 + M, c0:c0 + 128] = False
+    assert_untouched(got[rest], full[rest], 'in-place panel solve: outside C')
 
 
 @gpu
