@@ -151,6 +151,26 @@ __device__ __forceinline__ void matern_value_drho(double x, const MaternParams& 
         *dval = p.coef * ynu * y * km1 * p.inv_rho;
     }
 }
+
+// h(x) = -K'(x) / x, the radial factor of the gradient with respect to a point: with t_k = (p_k - q_k) / scale_k and
+// x = ||t||, dK/dq_k = h(x) t_k / scale_k. Each branch is written without the division by x (x^2 for the closed forms).
+// x == 0 returns exactly 0: there t = 0, so a coincident pair contributes 0 (nu > 1/2: the true derivative; nu = 1/2, where
+// K has a kink: the symmetric one) and h = inf (nu = 1/2, general nu <= 1) is never multiplied by 0.
+template <int MODE>
+__device__ __forceinline__ double matern_h(double x, const MaternParams& p) {
+    if (x == 0.0) return 0.0;
+    if (MODE == MAT_05) return exp(-x) / x;
+    if (MODE == MAT_15) return 3.0 * exp(-1.7320508075688772 * x);
+    if (MODE == MAT_25) {
+        const double s5 = 2.23606797749979;
+        return (5.0 / 3.0) * (1.0 + s5 * x) * exp(-s5 * x);
+    }
+    if (MODE == MAT_GAUSS) return exp(-0.5 * (x * x));
+    // h = coef 2 nu y^(nu-1) K_{nu-1}(y), y = sqrt(2 nu) x; K_{nu-1} = K_{nu+1} - (2 nu / y) K_nu
+    double y = p.sq2nu * x, k, k1;
+    bessel_k_pair(p.nu, y, &k, &k1);
+    return p.coef * (2.0 * p.nu) * pow(y, p.nu - 1.0) * (k1 - (2.0 * p.nu / y) * k);
+}
 #endif  // __CUDACC__
 
 }  // namespace gp

@@ -48,6 +48,8 @@ SIGNATURES = {
     'gp_matern_cross_points': (_int, [_vp, _i64, _vp, _i64, _i64, _vp, _f64, _vp, _i64, _vp]),
     'gp_predict_workspace_bytes': (_i64, [_i64, _i64, _i64]),
     'gp_predict_dense': (_int, [_vp, _i64, _i64, _vp, _i64, _vp, _i64, _i64, _vp, _i64, _vp, _vp, _vp]),
+    'gp_predict_grad_workspace_bytes': (_i64, [_i64, _i64, _i64, _i64]),
+    'gp_predict_grad_dense': (_int, [_vp, _i64, _vp, _i64, _i64, _vp, _f64, _vp, _i64, _vp, _i64, _vp, _vp, _vp]),
     'gp_kernel_threshold': (_int, [_i64, _i64, _f64, _vp, _f64, _vp]),
     'gp_sparse_workspace_bytes': (_i64, [_i64, _i64]),
     'gp_matern_sparse_count': (_int, [_vp, _vp, _i64, _i64, _vp, _f64, _f64, _vp, _vp, _vp, _vp]),

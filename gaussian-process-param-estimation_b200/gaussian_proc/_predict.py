@@ -11,6 +11,10 @@ For a test point with correlation vector k* (against the training points) and ba
 Device work per chunk of test points (csrc/gp_matern.cu, csrc/gp_predict.cu): the cross block P is generated, V = W P with
 W = inv(L) (cached by the DenseEngine), and one pass reduces P^T S (S = Kn^-1 [X z]) and the column norms of V. The m x m
 algebra runs on the host from that small result. The covariance adds two GEMMs over the whole test set.
+
+Gradients with respect to the test-point coordinates (``predict_gradient``) add, per chunk, U = W^T V = Kn^-1 P (one more
+GEMM into P's buffer, only for the variance) and one pass that regenerates dP/dq from the points and reduces it against S
+and U (gp_predict_grad_dense); the host then combines that with the basis Jacobian.
 """
 
 import ctypes
@@ -79,15 +83,9 @@ class Predictor(object):
         zMz = float(G[m, m] - G[:m, m] @ self.beta)
         self.sigma = math.sqrt(zMz / (n - m)) if sigma is None else float(sigma)
 
-    def predict(self, test_points, X_test, return_var=True, return_cov=False, noise=False, chunk_size=8192):
-        """Mean at the test points (rows of ``test_points``, basis rows ``X_test``), plus the variance and the covariance
-        when asked: returns ``mean``, ``(mean, var)``, ``(mean, cov)`` or ``(mean, var, cov)``. ``noise=True`` adds the
-        nugget sigma0^2 = sigma^2 eta (the variance of a new observation rather than of the latent value). Test points
-        are processed ``chunk_size`` at a time; the results do not depend on it. The covariance is formed over the whole
-        test set in one pass. A variance that cancellation pushed below zero is returned as 0."""
-        torch = dev.torch
-        K, eng = self.K, self.engine
-        n, npad, m, p, d = self.n, self.npad, self.m, self.p, self.d
+    def _test_set(self, test_points, X_test, chunk_size):
+        """test points (m*, d) and basis rows (m*, m) as float64 host arrays, after the checks of predict()"""
+        m, d = self.m, self.d
         tp = numpy.ascontiguousarray(test_points, dtype=numpy.float64)
         Xs = numpy.asarray(X_test, dtype=numpy.float64)
         if tp.ndim != 2 or tp.shape[1] != d:
@@ -100,7 +98,18 @@ class Predictor(object):
             raise ValueError('no test points.')
         if int(chunk_size) < 1:
             raise ValueError('chunk_size must be positive.')
-        chunk = ms if return_cov else min(int(chunk_size), ms)
+        return tp, Xs, ms
+
+    def _sweep(self, tp, chunk, grad=None):
+        """The device pass over the test points, ``chunk`` at a time: P, V = W P and out = [P^T S, ||V[:, j]||^2]
+        (gp_predict_dense), copied to the host as o (m*, p + 1). With ``grad`` not None the same chunk then also gives
+        out_grad[j][k] = [G_k[:, j]^T S, G_k[:, j]^T U[:, j]] (gp_predict_grad_dense, G_k = dP/dq_k), where U = W^T V =
+        Kn^-1 P is formed in P's buffer when ``grad`` is true (the last entry is 0 otherwise); both land in one
+        device-to-host copy. Returns (o, g, qd, V, mcpad) with g (m*, d, p + 1) or None."""
+        torch = dev.torch
+        K, eng = self.K, self.engine
+        n, npad, p, d = self.n, self.npad, self.p, self.d
+        ms = tp.shape[0]
         mcpad = dev.padded_size(chunk)
         s = dev.stream_ptr()
         eng._trtri(self.eta)              # factor of K + eta I and W = inv(L), cached per eta
@@ -109,27 +118,69 @@ class Predictor(object):
         P = torch.empty((npad, mcpad), dtype=f64, device='cuda')
         V = torch.empty((npad, mcpad), dtype=f64, device='cuda')
         ws = torch.empty(lib.gp_predict_workspace_bytes(npad, chunk, p) // 8, dtype=f64, device='cuda')
-        out = torch.empty(chunk * (p + 1), dtype=f64, device='cuda')
         scale, nu = K.correlation_scale, float(K.nu)
         o = numpy.empty((ms, p + 1))
+        if grad is None:
+            out = torch.empty(chunk * (p + 1), dtype=f64, device='cuda')
+            g = None
+        else:
+            out = torch.empty(chunk * (p + 1) * (1 + d), dtype=f64, device='cuda')
+            gws = torch.empty(lib.gp_predict_grad_workspace_bytes(n, chunk, d, p) // 8, dtype=f64, device='cuda')
+            kbeg = torch.arange(0, npad, 128, dtype=torch.int32, device='cuda')   # W^T is upper: row tile t needs k >= 128 t
+            g = numpy.empty((ms, d, p + 1))
         for c0 in range(0, ms, chunk):
             mc = min(chunk, ms - c0)
             check(lib.gp_matern_cross_points(_p(K.points), n, _p(qd, c0 * d), mc, d, dev.host_ptr(scale), nu, _p(P), mcpad,
                                              s), 'gp_matern_cross_points')
             check(lib.gp_predict_dense(_p(eng.W), n, npad, _p(self.S), p, _p(P), mc, mcpad, _p(V), mcpad, _p(out), _p(ws),
                                        s), 'gp_predict_dense')
-            o[c0:c0 + mc] = out[:mc * (p + 1)].cpu().numpy().reshape(mc, p + 1)
+            w = mc * (p + 1)
+            if grad is None:
+                o[c0:c0 + mc] = out[:w].cpu().numpy().reshape(mc, p + 1)
+                continue
+            if grad:
+                check(lib.gp_dgemm_ktab_f64(1, 1, _p(P), mcpad, _p(eng.W), npad, _p(V), mcpad, npad, dev.padded_size(mc),
+                                            npad, 1.0, 0.0, _p(kbeg), None, s), 'gp_dgemm_ktab_f64')
+            check(lib.gp_predict_grad_dense(_p(K.points), n, _p(qd, c0 * d), mc, d, dev.host_ptr(scale), nu, _p(self.S), p,
+                                            _p(P) if grad else None, mcpad, _p(out, w), _p(gws), s),
+                  'gp_predict_grad_dense')
+            h = out[:w * (1 + d)].cpu().numpy()
+            o[c0:c0 + mc] = h[:w].reshape(mc, p + 1)
+            g[c0:c0 + mc] = h[w:].reshape(mc, d, p + 1)
+        return o, g, qd, V, mcpad
 
+    def _moments(self, o, Xs, noise):
+        """mean, variance (clamped at 0), r = x* - X^T Kn^-1 k* (rows) and B^-1 r (columns) from the device result o"""
+        m, p = self.m, self.p
         kS = o[:, :m]                                 # (X^T Kn^-1 k*)^T
         mean = Xs @ self.beta + (o[:, m] - kS @ self.beta)
         r = Xs - kS                                   # rows r^T
         Br = numpy.linalg.solve(self.B, r.T)          # B^-1 r, one column per test point
         sigma2 = self.sigma ** 2
         nugget = sigma2 * self.eta if noise else 0.0
+        var = sigma2 * (1.0 - o[:, p] + numpy.einsum('ij,ji->i', r, Br)) + nugget
+        return mean, numpy.maximum(var, 0.0), r, Br
+
+    def predict(self, test_points, X_test, return_var=True, return_cov=False, noise=False, chunk_size=8192):
+        """Mean at the test points (rows of ``test_points``, basis rows ``X_test``), plus the variance and the covariance
+        when asked: returns ``mean``, ``(mean, var)``, ``(mean, cov)`` or ``(mean, var, cov)``. ``noise=True`` adds the
+        nugget sigma0^2 = sigma^2 eta (the variance of a new observation rather than of the latent value). Test points
+        are processed ``chunk_size`` at a time; the results do not depend on it. The covariance is formed over the whole
+        test set in one pass. A variance that cancellation pushed below zero is returned as 0."""
+        torch = dev.torch
+        npad, m, d = self.npad, self.m, self.d
+        tp, Xs, ms = self._test_set(test_points, X_test, chunk_size)
+        chunk = ms if return_cov else min(int(chunk_size), ms)
+        o, _, qd, V, mcpad = self._sweep(tp, chunk)
+        mean, var, r, Br = self._moments(o, Xs, noise)
+        s = dev.stream_ptr()
+        f64 = torch.float64
+        scale, nu = self.K.correlation_scale, float(self.K.nu)
+        sigma2 = self.sigma ** 2
+        nugget = sigma2 * self.eta if noise else 0.0
         res = [mean]
         if return_var:
-            var = sigma2 * (1.0 - o[:, p] + numpy.einsum('ij,ji->i', r, Br)) + nugget
-            res.append(numpy.maximum(var, 0.0))
+            res.append(var)
         if return_cov:
             C = torch.empty((mcpad, mcpad), dtype=f64, device='cuda')
             check(lib.gp_matern_dense(_p(qd), ms, d, dev.host_ptr(scale), nu, _p(C), mcpad, None, s), 'gp_matern_dense')
@@ -147,3 +198,29 @@ class Predictor(object):
                 cov.diagonal().add_(nugget)
             res.append(cov.cpu().numpy())
         return res[0] if len(res) == 1 else tuple(res)
+
+    def predict_gradient(self, test_points, X_test, X_test_grad, return_var=True, noise=False, chunk_size=8192):
+        """Gradients of the kriging mean (and variance) with respect to the test-point coordinates. ``X_test_grad``
+        (m*, d, m) holds the basis Jacobian dx*_j / dq_jk. Returns ``(mean, mean_grad)`` or ``(mean, var, mean_grad,
+        var_grad)``; the gradients are (m*, d). ``mean`` and ``var`` are those of ``predict()`` bit for bit, and
+        ``noise`` changes only ``var`` (the nugget is constant). With G_k = dk*/dq_k, u = Kn^-1 k* and D_k = S^T G_k:
+            d mean / dq_k = (dx*/dq_k)^T beta^ + D_k[z] - D_k[X] beta^
+            d var / dq_k  = sigma^2 (-2 u^T G_k + 2 (B^-1 r)^T (dx*/dq_k - D_k[X]))
+        A training point at distance exactly 0 from a test point contributes 0 to G_k: the derivative for nu > 1/2 and the
+        symmetric derivative for nu = 1/2, where the correlation has a kink. Where the variance was clamped at 0, its
+        gradient is still that of the unclamped expression. Each chunk adds Kn^-1 P (one more GEMM, only with
+        ``return_var``) and one pass over the training points to the work of ``predict()``."""
+        m, p, d = self.m, self.p, self.d
+        tp, Xs, ms = self._test_set(test_points, X_test, chunk_size)
+        Xg = numpy.asarray(X_test_grad, dtype=numpy.float64)
+        if Xg.shape != (ms, d, m):
+            raise ValueError('X_test_grad must be (%d, %d, %d): d X_test[j] / d test_points[j, k] for each test point j and '
+                             'dimension k; got %s.' % (ms, d, m, Xg.shape))
+        o, g, _, _, _ = self._sweep(tp, min(int(chunk_size), ms), grad=bool(return_var))
+        mean, var, r, Br = self._moments(o, Xs, noise)
+        DX = g[:, :, :m]                              # (S_x^T G_k)[j]
+        mean_grad = Xg @ self.beta + g[:, :, m] - DX @ self.beta
+        if not return_var:
+            return mean, mean_grad
+        var_grad = self.sigma ** 2 * (-2.0 * g[:, :, p] + 2.0 * numpy.einsum('jkc,cj->jk', Xg - DX, Br))
+        return mean, var, mean_grad, var_grad

@@ -33,9 +33,19 @@ class GaussianProcess(object):
         the variance (``return_var``) and the covariance (``return_cov``) of the latent values, or of new observations with
         ``noise=True``. Returns ``mean``, ``(mean, var)``, ``(mean, cov)`` or ``(mean, var, cov)``. Needs a dense K that
         knows its points, correlation_scale and nu (see ``Predictor``)."""
+        return self._predictor('predict').predict(test_points, X_test, return_var=return_var, return_cov=return_cov,
+                                                  noise=noise, chunk_size=chunk_size)
+
+    def predict_gradient(self, test_points, X_test, X_test_grad, return_var=True, noise=False, chunk_size=8192):
+        """Kriging mean at ``test_points`` and its gradient with respect to the test-point coordinates, at the trained
+        sigma and eta; ``X_test_grad`` (m* x d x m) is the Jacobian of the basis rows, d X_test[j] / d test_points[j, k].
+        Returns ``(mean, mean_grad)`` or, with ``return_var``, ``(mean, var, mean_grad, var_grad)``; the gradients are
+        m* x d, and mean and var equal those of ``predict`` (see ``Predictor.predict_gradient``)."""
+        return self._predictor('predict_gradient').predict_gradient(test_points, X_test, X_test_grad, return_var=return_var,
+                                                                    noise=noise, chunk_size=chunk_size)
+
+    def _predictor(self, what):
         if self.results is None:
-            raise RuntimeError('train(z) must be called before predict().')
+            raise RuntimeError('train(z) must be called before %s().' % what)
         from .._predict import Predictor
-        pred = Predictor(self.likelihood.K_mixed, self.X, self.z, self.results['eta'], sigma=self.results['sigma'])
-        return pred.predict(test_points, X_test, return_var=return_var, return_cov=return_cov, noise=noise,
-                            chunk_size=chunk_size)
+        return Predictor(self.likelihood.K_mixed, self.X, self.z, self.results['eta'], sigma=self.results['sigma'])

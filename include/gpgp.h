@@ -385,6 +385,20 @@ int gp_loglik_dense_dscale(const double* Ainv, int64_t n, int64_t npad, int64_t 
 int64_t gp_predict_workspace_bytes(int64_t npad, int64_t mc, int64_t p);
 int gp_predict_dense(const double* W, int64_t n, int64_t npad, const double* S, int64_t p, const double* P, int64_t mc,
                      int64_t ldp, double* V, int64_t ldv, double* out, void* ws, void* stream);
+/* Gradients of the kriging mean and variance with respect to the test-point coordinates. With
+ * G_k[i][j] = dP[i][j]/dq_jk = h(x) (p_ik - q_jk) / scale_k^2, x = ||(p_i - q_j) / scale||, h(x) = -matern'(x) / x,
+ * regenerated from the n training points (n, d) and the mc test points q (mc, d) and never stored:
+ *   out[(j*d + k)*(p+1) + c] = G_k[:, j]^T S[:, c]  for c < p,    out[(j*d + k)*(p+1) + p] = G_k[:, j]^T U[:, j]
+ * (0 when U == NULL: mean gradients only). S as for gp_predict_dense (ld = p); U: n x mc (ld ldu >= mc), normally
+ * Kn^-1 P = W^T V, one gp_dgemm_ktab_f64(1, 1, ...) with kbeg_tab[t] = 128 t. Rows i >= n of S and U and columns j >= mc of
+ * U are never read. A pair at distance exactly 0 contributes exactly 0: the true derivative for nu > 1/2, the symmetric
+ * derivative for nu = 1/2, where the correlation has a kink. scale_host, nu and d <= 8 as gp_matern_cross_points,
+ * p <= 16. A column's results do not depend on mc (fixed-order reduction over 2048-row chunks).
+ * ws: gp_predict_grad_workspace_bytes(n, mc, d, p) bytes (-1 for invalid sizes). No host synchronisation. */
+int64_t gp_predict_grad_workspace_bytes(int64_t n, int64_t mc, int64_t d, int64_t p);
+int gp_predict_grad_dense(const double* points, int64_t n, const double* q, int64_t mc, int64_t d, const double* scale_host,
+                          double nu, const double* S, int64_t p, const double* U, int64_t ldu, double* out, void* ws,
+                          void* stream);
 
 #ifdef __cplusplus
 }
