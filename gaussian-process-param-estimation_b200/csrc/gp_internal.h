@@ -36,6 +36,16 @@ int launch_dgemm_ktab(int at, int bt, double* C, int64_t ldc, const double* A, i
 int profile_enable(int on);
 int profile_read(double* ms_sum, double* ms_union, double* flops, long long* launches);
 
+// ---- row-blocked sparse operator (the SpMM in gp_sparse_la.cu; built by bcsr_build_kernel there and by
+// sparse_blocks_kernel in gp_sparse.cu) ---------------------------------------------------------------------------------
+// BCSR_ROWS consecutive rows of the ordered matrix share one list of block-columns. Groups of four block-columns are
+// stored in DMMA A-fragment order [8-row fragment][row in fragment][block-column in group], so that lane (g, t) of the SpMM
+// warp reads 32 consecutive doubles. 16 rows (two fragments per gathered row of X) measured faster than 8 at every width.
+constexpr int BCSR_ROWS = 16;
+// value (slot, row k) is at bval_pos(bval_group(slot), k)
+__device__ __forceinline__ int64_t bval_group(int64_t slot) { return (slot >> 2) * (4 * BCSR_ROWS) + (slot & 3); }
+__device__ __forceinline__ int64_t bval_pos(int64_t group, int k) { return group + (k >> 3) * 32 + (k & 7) * 4; }
+
 // ---- row-slab (multi-GPU) sparse operator: every rank maps its peers' arenas through CUDA IPC (csrc/gp_peer.cu) ------------
 constexpr int PEER_MAX = 8;         // ranks of one NVSwitch domain
 constexpr int PEER_SLOTS = 8;       // mailbox ring (a peer is never more than one exchange ahead; see peer_block_sum)

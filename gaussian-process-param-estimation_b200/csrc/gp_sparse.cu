@@ -10,6 +10,7 @@
 // are appended to their rows (in that rare case the row pointer is rebuilt on the host).
 #include "../../include/gpgp.h"
 #include "gp_common.cuh"
+#include "gp_internal.h"
 #include "gp_matern.cuh"
 #include <math.h>
 #include <vector>
@@ -678,17 +679,20 @@ static int sparse_prepare(const double* points, int64_t n, int64_t d, const doub
     return 0;
 }
 
-static int sparse_count_impl(const double* points, const double* points_host, int64_t n, int64_t d, const double* scale_host,
-                             double nu, double tau, void* ws, int* indptr_dev, int64_t* nnz_host, void* stream,
-                             const int* row_pos, int64_t row_first, int64_t row_last) {
+extern "C" {
+
+int gp_matern_sparse_count(const double* points, const double* points_host, int64_t n, int64_t d, const double* scale_host,
+                           double nu, double tau, void* ws, int* indptr_dev, int64_t* nnz_host, const int* row_pos_dev,
+                           int64_t row_first, int64_t row_last, void* stream) {
     if (!points || !points_host || !scale_host || !ws || !indptr_dev || !nnz_host || n <= 0 || d <= 0 || d > 8 || n > INT32_MAX)
         return -1;
+    if (row_pos_dev && (row_first < 0 || row_last < row_first || row_last > n)) return -1;
     cudaStream_t s = (cudaStream_t)stream;
     SparseWs w = carve_sparse(ws, n, d);
     SparseParams sp;
     CellGrid g;
     if (int rc = sparse_prepare(points, n, d, scale_host, nu, tau, w, s, &sp, &g)) return rc;
-    sp.row_pos = row_pos;
+    sp.row_pos = row_pos_dev;
     sp.row_first = (int)row_first;
     sp.row_last = (int)row_last;
     const int N = (int)n;
@@ -755,13 +759,6 @@ static int sparse_count_impl(const double* points, const double* points_host, in
     return 0;
 }
 
-extern "C" {
-
-int gp_matern_sparse_count(const double* points, const double* points_host, int64_t n, int64_t d, const double* scale_host,
-                           double nu, double tau, void* ws, int* indptr_dev, int64_t* nnz_host, void* stream) {
-    return sparse_count_impl(points, points_host, n, d, scale_host, nu, tau, ws, indptr_dev, nnz_host, stream, nullptr, 0, 0);
-}
-
 // Space-filling-curve keys of the points over their bounding box (2-D: Hilbert index, 31 bits per coordinate; otherwise
 // Z-order / Morton over the first min(d, 3) coordinates, 63 / min(d, 3) bits each): a stable sort by this key gives a deterministic, spatially local ordering of the points. The sparse operator
 // uses it internally (row-blocked form, gp_bcsr_*): consecutive rows then have nearly identical patterns.
@@ -813,14 +810,13 @@ int gp_csr_sort_rows(int64_t n, const int* indptr_dev, int* indices_dev, double*
     return sort_rows_run(n, indptr_dev, indices_dev, data_dev, ddata_dev, flags_dev, (cudaStream_t)stream);
 }
 
-}  // extern "C"
-
-static int sparse_fill_impl(const double* points, const double* points_host, int64_t n, int64_t d, const double* scale_host,
-                            double nu, double tau, void* ws, const int* indptr_dev, int* indices_dev, double* data_dev,
-                            double* ddata_dev, int sort_rows, void* stream, const int* row_pos, int64_t row_first,
-                            int64_t row_last) {
+int gp_matern_sparse_fill(const double* points, const double* points_host, int64_t n, int64_t d, const double* scale_host,
+                          double nu, double tau, void* ws, const int* indptr_dev, int* indices_dev, double* data_dev,
+                          double* ddata_dev, int sort_rows, const int* row_pos_dev, int64_t row_first, int64_t row_last,
+                          void* stream) {
     if (!points || !points_host || !scale_host || !ws || !indptr_dev || !indices_dev || !data_dev || n <= 0 || d <= 0 || d > 8)
         return -1;
+    if (row_pos_dev && (row_first < 0 || row_last < row_first || row_last > n)) return -1;
     if (ddata_dev)
         for (int k = 0; k < d; ++k)
             if (scale_host[k] != scale_host[0]) return -4;
@@ -834,7 +830,7 @@ static int sparse_fill_impl(const double* points, const double* points_host, int
     SparseParams sp;
     CellGrid g;
     make_params(n, d, scale_host, nu, tau, bb, bb + 8, &sp, &g);
-    sp.row_pos = row_pos;
+    sp.row_pos = row_pos_dev;
     sp.row_first = (int)row_first;
     sp.row_last = (int)row_last;
     int ne = meta[0];
@@ -870,35 +866,6 @@ static int sparse_fill_impl(const double* points, const double* points_host, int
     return 0;
 }
 
-extern "C" {
-
-int gp_matern_sparse_fill(const double* points, const double* points_host, int64_t n, int64_t d, const double* scale_host,
-                          double nu, double tau, void* ws, const int* indptr_dev, int* indices_dev, double* data_dev,
-                          double* ddata_dev, int sort_rows, void* stream) {
-    return sparse_fill_impl(points, points_host, n, d, scale_host, nu, tau, ws, indptr_dev, indices_dev, data_dev, ddata_dev,
-                            sort_rows, stream, nullptr, 0, 0);
-}
-
-// The same two passes restricted to the rows i with row_first <= row_pos_dev[i] < row_last (row_pos: position of row i in
-// the operator's spatial order): the slab of one GPU of the row-slab engine. The other rows stay empty (indptr is still
-// n + 1 long, column ids are global), so counts, memory and time are those of the slab.
-int gp_matern_sparse_count_rows(const double* points, const double* points_host, int64_t n, int64_t d,
-                                const double* scale_host, double nu, double tau, void* ws, int* indptr_dev, int64_t* nnz_host,
-                                const int* row_pos_dev, int64_t row_first, int64_t row_last, void* stream) {
-    if (!row_pos_dev || row_first < 0 || row_last < row_first || row_last > n) return -1;
-    return sparse_count_impl(points, points_host, n, d, scale_host, nu, tau, ws, indptr_dev, nnz_host, stream, row_pos_dev,
-                             row_first, row_last);
-}
-
-int gp_matern_sparse_fill_rows(const double* points, const double* points_host, int64_t n, int64_t d, const double* scale_host,
-                               double nu, double tau, void* ws, const int* indptr_dev, int* indices_dev, double* data_dev,
-                               double* ddata_dev, int sort_rows, const int* row_pos_dev, int64_t row_first, int64_t row_last,
-                               void* stream) {
-    if (!row_pos_dev || row_first < 0 || row_last < row_first || row_last > n) return -1;
-    return sparse_fill_impl(points, points_host, n, d, scale_host, nu, tau, ws, indptr_dev, indices_dev, data_dev, ddata_dev,
-                            sort_rows, stream, row_pos_dev, row_first, row_last);
-}
-
 }  // extern "C"
 
 
@@ -912,7 +879,6 @@ int gp_matern_sparse_fill_rows(const double* points, const double* points_host, 
 // SpMM's fragment order - no memset, no hash build, no second read of a CSR.
 // A pair inside the borderline band (|K - tau| <= 8 ulp: the host decides those in the CSR path) makes PASS 0 report it; the
 // caller then takes the CSR path for this matrix.
-constexpr int BR = 16;
 
 // DIM > 0: the dimension is a compile-time constant (coordinates stay in registers, loops unrolled); DIM = 0: sp.d at run time
 template <int DIM>
@@ -943,19 +909,19 @@ sparse_blocks_kernel(SparseParams sp, CellGrid g, const int* __restrict__ cell_s
                      const int* __restrict__ inv_order, int row_first, int nrows, int* __restrict__ nblk,
                      unsigned long long* stats, const int64_t* __restrict__ bptr, int* __restrict__ bidx,
                      double* __restrict__ bvals, double* __restrict__ bdvals) {
-    __shared__ double rowp_s[4][BR][8];
-    __shared__ int rowid_s[4][BR];
+    __shared__ double rowp_s[4][BCSR_ROWS][8];
+    __shared__ int rowid_s[4][BCSR_ROWS];
     __shared__ int queue_s[4][64];
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     const int rb = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    if (rb * BR >= nrows) return;
+    if (rb * BCSR_ROWS >= nrows) return;
     double (*rowp)[8] = rowp_s[w];
     int* rowid = rowid_s[w];
     int* queue = queue_s[w];
     // the block's rows: original point ids and coordinates
     int cmin[SMAXD] = {1 << 30, 1 << 30, 1 << 30}, cmax[SMAXD] = {-1, -1, -1};
-    if (lane < BR) {
-        const int r = rb * BR + lane;
+    if (lane < BCSR_ROWS) {
+        const int r = rb * BCSR_ROWS + lane;
         const int id = (r < nrows) ? order[row_first + r] : -1;
         rowid[lane] = id;
         double p[8] = {0, 0, 0, 0, 0, 0, 0, 0};
@@ -975,8 +941,8 @@ sparse_blocks_kernel(SparseParams sp, CellGrid g, const int* __restrict__ cell_s
             cmax[k] = max(cmax[k], __shfl_xor_sync(0xffffffffu, cmax[k], o));
         }
     __syncwarp();
-    int nvalid = nrows - rb * BR;
-    if (nvalid > BR) nvalid = BR;
+    int nvalid = nrows - rb * BCSR_ROWS;
+    if (nvalid > BCSR_ROWS) nvalid = BCSR_ROWS;
     // cell box of the block: the cells of its rows, one cell of margin (cell edge >= support radius)
     int blo[SMAXD] = {0, 0, 0}, bsz[SMAXD] = {1, 1, 1};
     int ncell_box = 1;
@@ -1036,9 +1002,9 @@ sparse_blocks_kernel(SparseParams sp, CellGrid g, const int* __restrict__ cell_s
         if (kept) {
             const int64_t slot = base + ncols + __popc(m & ((1u << lane) - 1u));
             bidx[slot] = inv_order[j];
-            const int64_t o = (slot >> 2) * (4 * BR) + (slot & 3);
+            const int64_t o = bval_group(slot);
 #pragma unroll 1
-            for (int r = 0; r < BR; ++r) {
+            for (int r = 0; r < BCSR_ROWS; ++r) {
                 double val = 0.0, dval = 0.0;
                 if (r < nvalid) {
                     const double s2 = sq_dist(rowp[r], pj);
@@ -1047,8 +1013,8 @@ sparse_blocks_kernel(SparseParams sp, CellGrid g, const int* __restrict__ cell_s
                         if (!(val > sp.tau)) { val = 0.0; dval = 0.0; }
                     }
                 }
-                bvals[o + (r >> 3) * 32 + (r & 7) * 4] = val;
-                if (WITH_DK) bdvals[o + (r >> 3) * 32 + (r & 7) * 4] = dval;
+                bvals[bval_pos(o, r)] = val;
+                if (WITH_DK) bdvals[bval_pos(o, r)] = dval;
             }
         }
         ncols += __popc(m);
@@ -1123,11 +1089,11 @@ sparse_blocks_kernel(SparseParams sp, CellGrid g, const int* __restrict__ cell_s
     } else if (lane < padded - ncols) {          // pad the block to a multiple of 4 block-columns (zero values, a valid index)
         const int64_t slot = base + ncols + lane;
         bidx[slot] = inv_order[rowid[0]];
-        const int64_t o = (slot >> 2) * (4 * BR) + (slot & 3);
+        const int64_t o = bval_group(slot);
 #pragma unroll
-        for (int r = 0; r < BR; ++r) {
-            bvals[o + (r >> 3) * 32 + (r & 7) * 4] = 0.0;
-            if (WITH_DK) bdvals[o + (r >> 3) * 32 + (r & 7) * 4] = 0.0;
+        for (int r = 0; r < BCSR_ROWS; ++r) {
+            bvals[bval_pos(o, r)] = 0.0;
+            if (WITH_DK) bdvals[bval_pos(o, r)] = 0.0;
         }
     }
 }
@@ -1136,7 +1102,7 @@ template <int MODE>
 static void launch_blocks(int pass, bool with_dk, const SparseParams& sp, const CellGrid& g, const SparseWs& w, const double* pts,
                           const int* order, const int* inv_order, int row_first, int nrows, int* nblk, unsigned long long* stats,
                           const int64_t* bptr, int* bidx, double* bvals, double* bdvals, cudaStream_t s) {
-    const int nrb = (nrows + BR - 1) / BR;
+    const int nrb = (nrows + BCSR_ROWS - 1) / BCSR_ROWS;
     const unsigned blocks = (unsigned)((nrb + 3) / 4);
 #define GP_BLOCKS_LAUNCH(PASS, DK, DIM)                                                                                         \
     sparse_blocks_kernel<MODE, PASS, DK, DIM><<<blocks, 128, 0, s>>>(sp, g, w.cell_start, w.sorted_idx, w.sorted_pts, pts, order, \
@@ -1180,7 +1146,7 @@ int gp_matern_blocks_count(const double* points, int64_t n, int64_t d, const dou
                            const int* order_dev, const int* inv_order_dev, int64_t row_first, int64_t row_last, int* nblk_dev,
                            int64_t* stats_host, void* stream) {
     if (!points || !scale_host || !ws || !order_dev || !inv_order_dev || !nblk_dev || !stats_host || n <= 0 || d <= 0 || d > 8 ||
-        n > INT32_MAX || row_first < 0 || row_last <= row_first || row_last > n || (row_first % BR))
+        n > INT32_MAX || row_first < 0 || row_last <= row_first || row_last > n || (row_first % BCSR_ROWS))
         return -1;
     cudaStream_t s = (cudaStream_t)stream;
     SparseWs w = carve_sparse(ws, n, d);
@@ -1207,7 +1173,7 @@ int gp_matern_blocks_fill(const double* points, int64_t n, int64_t d, const doub
                           const int* order_dev, const int* inv_order_dev, int64_t row_first, int64_t row_last,
                           const int64_t* bptr_dev, int* bidx_dev, double* bvals_dev, double* bdvals_dev, void* stream) {
     if (!points || !scale_host || !ws || !order_dev || !inv_order_dev || !bptr_dev || !bidx_dev || !bvals_dev || n <= 0 ||
-        d <= 0 || d > 8 || row_first < 0 || row_last <= row_first || row_last > n || (row_first % BR))
+        d <= 0 || d > 8 || row_first < 0 || row_last <= row_first || row_last > n || (row_first % BCSR_ROWS))
         return -1;
     if (bdvals_dev)
         for (int k = 0; k < d; ++k)

@@ -11,15 +11,6 @@
 
 namespace gp {
 
-#ifndef GP_SPMM_MINB
-#define GP_SPMM_MINB 4
-#endif
-#ifndef GP_SPMM_U
-#define GP_SPMM_U 4
-#endif
-#ifndef GP_SPMM_ROWLOAD
-#define GP_SPMM_ROWLOAD 0
-#endif
 constexpr int RED_PARTS = 592;  // CTAs of the column reductions (4 per SM)
 
 // ---- Y = (K + eta I) X, one warp per row; lane = (q, c): q-th nonzero of the current group, column c ---------
@@ -165,10 +156,10 @@ __global__ void rademacher_kernel(int64_t n, int B, uint64_t seed, int64_t probe
     V[idx] = (z & 1ull) ? 1.0 : -1.0;
 }
 
-// ---- row-blocked operator: R = 8 or 16 consecutive rows share one column list (R x 1 blocks, zero filled) ---------
+// ---- row-blocked operator: BCSR_ROWS = 16 consecutive rows share one column list (16 x 1 blocks, zero filled) ----------
 // Rows that are neighbours in a spatially sorted order have almost the same pattern, so one gathered row of X serves
-// R rows of K: gather traffic (the L1/L2-bound part of a multi-column SpMM) drops ~R-fold and the column index is
-// amortised over R values. Block-columns of a row block: [all columns of row 0][columns of row 1 not in row 0]...
+// 16 rows of K: gather traffic (the L1/L2-bound part of a multi-column SpMM) drops ~16-fold and the column index is
+// amortised over 16 values. Block-columns of a row block: [all columns of row 0][columns of row 1 not in row 0]...
 // (each segment in the source row's order); any order is valid for the product.
 __device__ __forceinline__ int find_col(const int* __restrict__ row, int len, int c) {
     int lo = 0, hi = len;
@@ -189,22 +180,14 @@ __device__ __forceinline__ int find_col(const int* __restrict__ row, int len, in
 // the same layout, so both paths write identical output.
 constexpr int HCAP = 2048, HMAX = 1536;
 
-// Position of (block-column slot, row k) in the value stream: groups of four block-columns are stored in DMMA A-fragment
-// order [row][block-column in group] so that lane (g, t) of the SpMM warp reads 32 consecutive doubles (bptr entries are
-// multiples of 4; R = 8 or 16 rows = one or two 8-row fragments).
-template <int R>
-__device__ __forceinline__ int64_t bval_pos(int64_t slot, int k) {
-    return (slot >> 2) * (4 * R) + (k >> 3) * 32 + (k & 7) * 4 + (slot & 3);      // R = 16: two 8-row fragments per group
-}
-
-template <int R, int PASS>
+template <int PASS>
 __device__ __forceinline__ int bcsr_block_search(int lane, int rb, const int* s, const int* len, const int* __restrict__ inv_order,
                                                  const int* __restrict__ indices, const double* __restrict__ data,
                                                  const double* __restrict__ ddata, int64_t base, int* bidx, double* bvals,
                                                  double* bdvals) {
     int running = 0;
 #pragma unroll
-    for (int k = 0; k < R; ++k) {
+    for (int k = 0; k < BCSR_ROWS; ++k) {
         for (int t0 = 0; t0 < len[k]; t0 += 32) {
             const int t = t0 + lane;
             const bool valid = t < len[k];
@@ -217,13 +200,13 @@ __device__ __forceinline__ int bcsr_block_search(int lane, int rb, const int* s,
             if (PASS == 1 && owned) {
                 const int64_t slot = base + running + __popc(m & ((1u << lane) - 1u));
                 bidx[slot] = inv_order ? inv_order[c] : c;
-                double v[R], dv[R];
+                double v[BCSR_ROWS], dv[BCSR_ROWS];
 #pragma unroll
-                for (int kk = 0; kk < R; ++kk) { v[kk] = 0.0; dv[kk] = 0.0; }
+                for (int kk = 0; kk < BCSR_ROWS; ++kk) { v[kk] = 0.0; dv[kk] = 0.0; }
                 v[k] = data[s[k] + t];
                 if (ddata) dv[k] = ddata[s[k] + t];
 #pragma unroll
-                for (int kk = k + 1; kk < R; ++kk) {
+                for (int kk = k + 1; kk < BCSR_ROWS; ++kk) {
                     int pos = find_col(indices + s[kk], len[kk], c);
                     if (pos >= 0) {
                         v[kk] = data[s[kk] + pos];
@@ -231,10 +214,10 @@ __device__ __forceinline__ int bcsr_block_search(int lane, int rb, const int* s,
                     }
                 }
 #pragma unroll
-                for (int kk = 0; kk < R; ++kk) bvals[bval_pos<R>(slot, kk)] = v[kk];
+                for (int kk = 0; kk < BCSR_ROWS; ++kk) bvals[bval_pos(bval_group(slot), kk)] = v[kk];
                 if (ddata) {
 #pragma unroll
-                    for (int kk = 0; kk < R; ++kk) bdvals[bval_pos<R>(slot, kk)] = dv[kk];
+                    for (int kk = 0; kk < BCSR_ROWS; ++kk) bdvals[bval_pos(bval_group(slot), kk)] = dv[kk];
                 }
             }
             running += __popc(m);
@@ -243,7 +226,7 @@ __device__ __forceinline__ int bcsr_block_search(int lane, int rb, const int* s,
     return running;
 }
 
-template <int R, int PASS>
+template <int PASS>
 __global__ void __launch_bounds__(128)
 bcsr_build_kernel(int n, const int* __restrict__ order, const int* __restrict__ inv_order, const int* __restrict__ indptr,
                   const int* __restrict__ indices, const double* __restrict__ data, const double* __restrict__ ddata,
@@ -252,14 +235,14 @@ bcsr_build_kernel(int n, const int* __restrict__ order, const int* __restrict__ 
     __shared__ unsigned short hslot[4][HCAP];      // slots < HMAX + 32
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     const int rb = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    if (rb * R >= n) return;
+    if (rb * BCSR_ROWS >= n) return;
     int* hk = hkey[w];
     unsigned short* hs = hslot[w];
     for (int i = lane; i < HCAP; i += 32) hk[i] = -1;
-    int s[R], len[R];
+    int s[BCSR_ROWS], len[BCSR_ROWS];
 #pragma unroll
-    for (int k = 0; k < R; ++k) {
-        int r = rb * R + k;
+    for (int k = 0; k < BCSR_ROWS; ++k) {
+        int r = rb * BCSR_ROWS + k;
         if (r < n) {
             int o = order ? order[r] : r;
             s[k] = indptr[o];
@@ -274,7 +257,7 @@ bcsr_build_kernel(int n, const int* __restrict__ order, const int* __restrict__ 
     int running = 0;
     bool overflow = false;
 #pragma unroll
-    for (int k = 0; k < R; ++k) {
+    for (int k = 0; k < BCSR_ROWS; ++k) {
         for (int t0 = 0; t0 < len[k] && !overflow; t0 += 32) {
             const int t = t0 + lane;
             const bool valid = t < len[k];
@@ -303,7 +286,7 @@ bcsr_build_kernel(int n, const int* __restrict__ order, const int* __restrict__ 
             __syncwarp();
             if (running > HMAX) overflow = true;
             if (PASS == 1 && valid && !overflow) {
-                const int64_t o = bval_pos<R>(base + slot, k);
+                const int64_t o = bval_pos(bval_group(base + slot), k);
                 bvals[o] = data[s[k] + t];
                 if (ddata) bdvals[o] = ddata[s[k] + t];
                 if (isnew) bidx[base + slot] = inv_order ? inv_order[c] : c;
@@ -313,30 +296,30 @@ bcsr_build_kernel(int n, const int* __restrict__ order, const int* __restrict__ 
     if (overflow) {
         if (searched && lane == 0) atomicExch(searched, 1);
         if (PASS == 1) {      // clear what the hash path wrote, then redo the block by searching
-            const int64_t cnt = (bptr[rb + 1] - base) * R;
+            const int64_t cnt = (bptr[rb + 1] - base) * BCSR_ROWS;
             for (int64_t i = lane; i < cnt; i += 32) {
-                bvals[base * R + i] = 0.0;
-                if (ddata) bdvals[base * R + i] = 0.0;
+                bvals[base * BCSR_ROWS + i] = 0.0;
+                if (ddata) bdvals[base * BCSR_ROWS + i] = 0.0;
             }
             __syncwarp();
         }
-        running = bcsr_block_search<R, PASS>(lane, rb, s, len, inv_order, indices, data, ddata, base, bidx, bvals, bdvals);
+        running = bcsr_block_search<PASS>(lane, rb, s, len, inv_order, indices, data, ddata, base, bidx, bvals, bdvals);
     }
     const int padded = (running + 3) & ~3;
     if (PASS == 0 && lane == 0) nblk[rb] = padded;
     if (PASS == 1 && lane < padded - running) {
         const int64_t slot = base + running + lane;
-        const int c0 = (len[0] > 0) ? indices[s[0]] : (order ? order[rb * R] : rb * R);
+        const int c0 = (len[0] > 0) ? indices[s[0]] : (order ? order[rb * BCSR_ROWS] : rb * BCSR_ROWS);
         bidx[slot] = inv_order ? inv_order[c0] : c0;
 #pragma unroll
-        for (int kk = 0; kk < R; ++kk) {
-            bvals[bval_pos<R>(slot, kk)] = 0.0;
-            if (ddata) bdvals[bval_pos<R>(slot, kk)] = 0.0;
+        for (int kk = 0; kk < BCSR_ROWS; ++kk) {
+            bvals[bval_pos(bval_group(slot), kk)] = 0.0;
+            if (ddata) bdvals[bval_pos(bval_group(slot), kk)] = 0.0;
         }
     }
 }
 
-// Y = (K + eta I) X on the row-blocked operator (R = 8 H rows per block, H = 1 or 2) with FP64 tensor-core MMAs. One warp per row block. Four
+// Y = (K + eta I) X on the row-blocked operator with FP64 tensor-core MMAs. One warp per row block. Four
 // block-columns form one DMMA.8x8x4: A (8 rows x 4 block-columns) is exactly 256 contiguous bytes of the value stream
 // (one 8-byte load per lane, no broadcast), B (4 x 8) holds the four gathered rows of X restricted to 8 columns, and the
 // 8 x 8 accumulator stays in two registers per lane for the whole row block - no cross-lane reduction. For B = 16 / 32
@@ -345,16 +328,19 @@ bcsr_build_kernel(int n, const int* __restrict__ order, const int* __restrict__ 
 // consecutive columns of one Y row. Index and values are streamed past L1 (ld.global.cs): L1 is kept for X.
 // Epilogue: Y = scale[c] (A X + eta X) (scale optional) and, with DOT, partial[cta][c] = sum over the CTA's 64 rows
 // of X[i][c] Y[i][c] (fixed order) - the Lanczos alpha / CG p^T A p reduction without another pass over the vectors.
-// H = 1: 8 x 1 row blocks; H = 2: 16 x 1 row blocks (two A fragments and two MMAs per gathered B fragment).
+// A 16-row block is H = 2 fragments: two A fragments and two MMAs per gathered B fragment.
 // PEER (row-slab operator on several GPUs): the rows of this rank's slab; a block-column index carries the owner rank in its
 // top 4 bits and the row within the owner's slab below (gp_slab_encode_columns), and the gather goes to the owner's copy of
 // the exchange vector - local HBM for the own slab, a load over NVLink from the mapped arena of a peer for the halo.
 constexpr int PEER_SHIFT = 28;
-template <int B, bool DOT, int H, bool PEER = false>
-__global__ void __launch_bounds__(256, GP_SPMM_MINB)
+constexpr int SPMM_MINB = 4;      // CTAs per SM (launch bounds)
+constexpr int SPMM_U = 4;         // steps in flight per warp for B <= 16
+template <int B, bool DOT, bool PEER = false>
+__global__ void __launch_bounds__(256, SPMM_MINB)
 bcsr8_spmm_dmma_kernel(const int64_t* __restrict__ bptr, const int* __restrict__ bidx, const double* __restrict__ bvals, int n,
                        double eta, const double* __restrict__ X, const double* __restrict__ scale, double* __restrict__ Y,
                        double* __restrict__ partial, const __grid_constant__ PeerVec pv) {
+    constexpr int H = BCSR_ROWS / 8;           // 8-row A fragments per row block
     constexpr int NT = (B >= 8) ? B / 8 : 1;   // 8-column MMA tiles per step
     const int lane = threadIdx.x & 31;
     const int g = lane >> 2, t = lane & 3;     // DMMA.8x8x4 fragments: A[g][t], B[t][g], D[g][2t .. 2t+1]
@@ -362,7 +348,7 @@ bcsr8_spmm_dmma_kernel(const int64_t* __restrict__ bptr, const int* __restrict__
     // blocks start first and the interior ones fill the tail
     const int bx = PEER ? ((blockIdx.x & 1) ? (int)gridDim.x - 1 - (int)(blockIdx.x >> 1) : (int)(blockIdx.x >> 1)) : (int)blockIdx.x;
     const int rb = (bx * blockDim.x + threadIdx.x) >> 5;
-    const bool live = rb * (8 * H) < n;
+    const bool live = rb * BCSR_ROWS < n;
     if (!DOT && !live) return;
     const int64_t p0 = live ? bptr[rb] : 0, p1 = live ? bptr[rb + 1] : 0;   // p1 - p0 is a multiple of 4
     double acc[H][NT][2];
@@ -375,15 +361,7 @@ bcsr8_spmm_dmma_kernel(const int64_t* __restrict__ bptr, const int* __restrict__
     const double* aptr = bvals + lane;          // A fragment order: element (row g, block-column t) at 4 g + t = lane
     // B = 16: a gathered X row is 128 bytes = one L1 line. In the fragment layout (lane 4 g + t holds row t, columns 2 g,
     // 2 g + 1) a quarter-warp - the unit a 16-byte load is served in - touches FOUR rows: 16 line accesses (wavefronts) per
-    // load instruction, and the L1 data pipe, not HBM, bounds the kernel (ncu, profiles/r01_spmm_ncu_summary.md). ROWLOAD
-    // (compile-time experiment, OFF): lane 8 t' + g' loads chunk g' of row t' - every quarter-warp reads one whole line -
-    // and two 64-bit warp shuffles bring the chunk to the lane that owns it in the fragment layout. Measured at n = 2^20:
-    // 1.043 ms against 0.910 ms for the direct fragment gather - the shuffles go through the same LSU data path and cost
-    // more than the saved line accesses (like the shared-memory staging of round 1: the bytes pass the pipe twice).
-    constexpr bool ROWLOAD = (B == 16) && (GP_SPMM_ROWLOAD != 0);
-    const int tsel = ROWLOAD ? (lane >> 3) : t;                    // which of the step's 4 block-columns this lane loads
-    const int xoff = ROWLOAD ? 2 * (lane & 7) : coff;
-    const int xsrc = 8 * t + g;                                    // ROWLOAD: the lane that loaded this lane's fragment
+    // load instruction, and the L1 data pipe, not HBM, bounds the kernel (ncu, profiles/r01_spmm_ncu_summary.md).
     auto load_x = [&](int col, double* x) {
         const double* xr;
         if (PEER) {
@@ -392,16 +370,12 @@ bcsr8_spmm_dmma_kernel(const int64_t* __restrict__ bptr, const int* __restrict__
             // a dependent constant-bank load in front of every gather - is taken only by steps that touch a peer.
             const unsigned owner = (unsigned)col >> PEER_SHIFT;
             const int64_t local = (int64_t)(col & ((1 << PEER_SHIFT) - 1));
-            if (__any_sync(0xffffffffu, owner != (unsigned)pv.rank)) xr = pv.base[owner] + local * B + xoff;
-            else xr = X + local * B + xoff;
+            if (__any_sync(0xffffffffu, owner != (unsigned)pv.rank)) xr = pv.base[owner] + local * B + coff;
+            else xr = X + local * B + coff;
         } else {
-            xr = X + (int64_t)col * B + xoff;
+            xr = X + (int64_t)col * B + coff;
         }
-        if (ROWLOAD) {
-            const double2 v = *reinterpret_cast<const double2*>(xr);
-            x[0] = __shfl_sync(0xffffffffu, v.x, xsrc);
-            x[NT > 1 ? 1 : 0] = __shfl_sync(0xffffffffu, v.y, xsrc);
-        } else if (NT == 1) {
+        if (NT == 1) {
             x[0] = colok ? *xr : 0.0;
         } else {
 #pragma unroll
@@ -412,17 +386,17 @@ bcsr8_spmm_dmma_kernel(const int64_t* __restrict__ bptr, const int* __restrict__
             }
         }
     };
-    constexpr int U = (NT <= 2) ? GP_SPMM_U : 2;       // steps in flight per warp: all loads of U steps are issued before their MMAs
+    constexpr int U = (NT <= 2) ? SPMM_U : 2;          // steps in flight per warp: all loads of U steps are issued before their MMAs
     int64_t p = p0;
     for (; p + 4 * U <= p1; p += 4 * U) {
         int col[U];
         double a[U][H], x[U][NT];
 #pragma unroll
-        for (int u = 0; u < U; ++u) col[u] = __ldcs(bidx + p + 4 * u + tsel);
+        for (int u = 0; u < U; ++u) col[u] = __ldcs(bidx + p + 4 * u + t);
 #pragma unroll
         for (int u = 0; u < U; ++u)
 #pragma unroll
-            for (int h = 0; h < H; ++h) a[u][h] = __ldcs(aptr + (p + 4 * u) * (8 * H) + 32 * h);
+            for (int h = 0; h < H; ++h) a[u][h] = __ldcs(aptr + (p + 4 * u) * BCSR_ROWS + 32 * h);
 #pragma unroll
         for (int u = 0; u < U; ++u) load_x(col[u], x[u]);
 #pragma unroll
@@ -433,10 +407,10 @@ bcsr8_spmm_dmma_kernel(const int64_t* __restrict__ bptr, const int* __restrict__
                 for (int j = 0; j < NT; ++j) dmma884(acc[h][j][0], acc[h][j][1], a[u][h], x[u][j]);
     }
     for (; p < p1; p += 4) {
-        const int col = __ldcs(bidx + p + tsel);
+        const int col = __ldcs(bidx + p + t);
         double a[H], x[NT];
 #pragma unroll
-        for (int h = 0; h < H; ++h) a[h] = __ldcs(aptr + p * (8 * H) + 32 * h);
+        for (int h = 0; h < H; ++h) a[h] = __ldcs(aptr + p * BCSR_ROWS + 32 * h);
         load_x(col, x);
 #pragma unroll
         for (int h = 0; h < H; ++h)
@@ -450,7 +424,7 @@ bcsr8_spmm_dmma_kernel(const int64_t* __restrict__ bptr, const int* __restrict__
     for (int k = 0; k < NC; ++k) dsum[k] = 0.0;
 #pragma unroll
     for (int h = 0; h < H; ++h) {
-        const int row = rb * (8 * H) + h * 8 + g;
+        const int row = rb * BCSR_ROWS + h * 8 + g;
         if (live && row < n) {
 #pragma unroll
             for (int k = 0; k < NC; ++k) {
@@ -487,9 +461,9 @@ bcsr8_spmm_dmma_kernel(const int64_t* __restrict__ bptr, const int* __restrict__
     }
 }
 
-// the operator a Krylov routine works on: plain CSR (R = 1) or the row-blocked form (R = 8 or 16)
+// the operator a Krylov routine works on: plain CSR or the row-blocked form
 struct SparseOp {
-    int R;                 // 1: CSR (ptr32, idx, val); > 1: row-blocked (ptr64, idx, val)
+    bool blocked;          // false: CSR (ptr32, idx, val); true: row-blocked (ptr64, idx, val)
     const int* ptr32;
     const int64_t* ptr64;
     const int* idx;
@@ -497,25 +471,23 @@ struct SparseOp {
     int n;
 };
 
-static int bcsr_parts(int n, int R) { return (((n + R - 1) / R) + 7) / 8; }   // CTAs of the row-blocked SpMM = dot partials
-static int bcsr8_parts(int n) { return bcsr_parts(n, 8); }
+// CTAs of the row-blocked SpMM (8 warps = 8 row blocks each) = rows of its dot partials
+static int bcsr_parts(int n) { return ((n + BCSR_ROWS - 1) / BCSR_ROWS + 7) / 8; }
 
 template <int B>
 static void bcsr8_spmm_launch_b(const SparseOp& A, double eta, const double* X, const double* scale, double* Y,
                                 double* partial, cudaStream_t s, const PeerVec* pvp) {
-    const int blocks = bcsr_parts(A.n, A.R);
+    const int blocks = bcsr_parts(A.n);
     PeerVec pv = {};
     if (pvp) pv = *pvp;
-#define GP_SPMM_LAUNCH(DOT, H, PEER) \
-    bcsr8_spmm_dmma_kernel<B, DOT, H, PEER><<<blocks, 256, 0, s>>>(A.ptr64, A.idx, A.val, A.n, eta, X, scale, Y, partial, pv)
-    if (pvp) {       // row-slab operator (16-row blocks only)
-        if (partial) GP_SPMM_LAUNCH(true, 2, true); else GP_SPMM_LAUNCH(false, 2, true);
-    } else if (A.R == 16) {
-        if (partial) GP_SPMM_LAUNCH(true, 2, false); else GP_SPMM_LAUNCH(false, 2, false);
+#define SPMM_LAUNCH(DOT, PEER) \
+    bcsr8_spmm_dmma_kernel<B, DOT, PEER><<<blocks, 256, 0, s>>>(A.ptr64, A.idx, A.val, A.n, eta, X, scale, Y, partial, pv)
+    if (pvp) {       // row-slab operator
+        if (partial) SPMM_LAUNCH(true, true); else SPMM_LAUNCH(false, true);
     } else {
-        if (partial) GP_SPMM_LAUNCH(true, 1, false); else GP_SPMM_LAUNCH(false, 1, false);
+        if (partial) SPMM_LAUNCH(true, false); else SPMM_LAUNCH(false, false);
     }
-#undef GP_SPMM_LAUNCH
+#undef SPMM_LAUNCH
 }
 
 // Y = scale (.) ((A + eta I) X); with `partial` also the per-column partial sums of X (.) Y: *nparts rows of B doubles
@@ -523,8 +495,7 @@ static void bcsr8_spmm_launch_b(const SparseOp& A, double eta, const double* X, 
 static int spmm(const SparseOp& A, double eta, const double* X, int B, double* Y, cudaStream_t s,
                 const double* scale = nullptr, double* partial = nullptr, int* nparts = nullptr, const PeerVec* pv = nullptr) {
     const int n = A.n;
-    if (pv && A.R != 16) return -3;
-    if (A.R == 1) {
+    if (!A.blocked) {
         int blocks = (int)(((int64_t)n * 32 + 255) / 256);
         switch (B) {
             case 1: csr_spmm_kernel<1><<<blocks, 256, 0, s>>>(A.ptr32, A.idx, A.val, n, eta, X, scale, Y); break;
@@ -541,7 +512,7 @@ static int spmm(const SparseOp& A, double eta, const double* X, int B, double* Y
             *nparts = RED_PARTS;
             GP_COUNT(1);
         }
-    } else if (A.R == 8 || A.R == 16) {
+    } else {
         switch (B) {
             case 1: bcsr8_spmm_launch_b<1>(A, eta, X, scale, Y, partial, s, pv); break;
             case 2: bcsr8_spmm_launch_b<2>(A, eta, X, scale, Y, partial, s, pv); break;
@@ -551,10 +522,8 @@ static int spmm(const SparseOp& A, double eta, const double* X, int B, double* Y
             case 32: bcsr8_spmm_launch_b<32>(A, eta, X, scale, Y, partial, s, pv); break;
             default: return -2;
         }
-        if (partial) *nparts = bcsr_parts(n, A.R);
+        if (partial) *nparts = bcsr_parts(n);
         GP_COUNT(1);
-    } else {
-        return -3;
     }
     GP_LAUNCH_CHECK();
     return 0;
@@ -576,11 +545,11 @@ static void col_final(const double* partial, int nparts, int B, int op, double* 
 }
 
 static SparseOp csr_op(const int* indptr, const int* indices, const double* data, int64_t n) {
-    SparseOp A = {1, indptr, nullptr, indices, data, (int)n};
+    SparseOp A = {false, indptr, nullptr, indices, data, (int)n};
     return A;
 }
-static SparseOp bcsr_op(int64_t R, const int64_t* bptr, const int* bidx, const double* bvals, int64_t n) {
-    SparseOp A = {(int)R, nullptr, bptr, bidx, bvals, (int)n};
+static SparseOp bcsr_op(const int64_t* bptr, const int* bidx, const double* bvals, int64_t n) {
+    SparseOp A = {true, nullptr, bptr, bidx, bvals, (int)n};
     return A;
 }
 
@@ -677,59 +646,58 @@ int gp_csr_spmm(const int* indptr, const int* indices, const double* data, int64
     return spmm(csr_op(indptr, indices, data, n), eta, X, (int)B, Y, (cudaStream_t)stream);
 }
 
-int gp_bcsr_spmm(int64_t R, const int64_t* bptr, const int* bidx, const double* bvals, int64_t n, double eta, const double* X,
+// Y = (K + eta I) X restricted to the rows of the operator. Row-slab operator (`peer`): X (this rank's rows) is first copied
+// into exchange vector 2; a barrier before (every rank's copy is in place) and after (nobody overwrites it while a peer
+// still gathers) the SpMM.
+int gp_bcsr_spmm(void* peer, const int64_t* bptr, const int* bidx, const double* bvals, int64_t n, double eta, const double* X,
                  int64_t B, double* Y, void* stream) {
     if (!bptr || !bidx || !bvals || !X || !Y || n <= 0 || n > INT32_MAX) return -1;
-    return spmm(bcsr_op(R, bptr, bidx, bvals, n), eta, X, (int)B, Y, (cudaStream_t)stream);
+    cudaStream_t s = (cudaStream_t)stream;
+    PeerCtx* px = (PeerCtx*)peer;
+    if (!px) return spmm(bcsr_op(bptr, bidx, bvals, n), eta, X, (int)B, Y, s);
+    double* E = peer_local_vec(px, 2);
+    PeerVec pv = peer_vec(px, 2);
+    GP_CUDA_CHECK(cudaMemcpyAsync(E, X, sizeof(double) * n * B, cudaMemcpyDeviceToDevice, s));
+    if (int rc = peer_barrier_launch(px, s)) return rc;
+    if (int rc = spmm(bcsr_op(bptr, bidx, bvals, n), eta, E, (int)B, Y, s, nullptr, nullptr, nullptr, &pv)) return rc;
+    return peer_barrier_launch(px, s);
 }
 
 }  // extern "C"
 
-template <int R>
-static int bcsr_build(int pass, int n, const int* order, const int* inv_order, const int* indptr, const int* indices,
+static int bcsr_build(int pass, int64_t n, const int* order, const int* inv_order, const int* indptr, const int* indices,
                       const double* data, const double* ddata, int* nblk, const int64_t* bptr, int* bidx, double* bvals,
-                      double* bdvals, int* searched, cudaStream_t s) {
-    const int nrb = (n + R - 1) / R;
+                      double* bdvals, int* searched, void* stream) {
+    cudaStream_t s = (cudaStream_t)stream;
+    if (!indptr || !indices || n <= 0 || n > INT32_MAX || ((order == nullptr) != (inv_order == nullptr))) return -1;
+    const int nrb = (int)((n + BCSR_ROWS - 1) / BCSR_ROWS);
     const unsigned blocks = (unsigned)(((int64_t)nrb * 32 + 127) / 128);
     if (pass == 0)
-        bcsr_build_kernel<R, 0><<<blocks, 128, 0, s>>>(n, order, inv_order, indptr, indices, data, ddata, nblk, bptr, bidx, bvals, bdvals, searched);
+        bcsr_build_kernel<0><<<blocks, 128, 0, s>>>((int)n, order, inv_order, indptr, indices, data, ddata, nblk, bptr, bidx, bvals, bdvals, searched);
     else
-        bcsr_build_kernel<R, 1><<<blocks, 128, 0, s>>>(n, order, inv_order, indptr, indices, data, ddata, nblk, bptr, bidx, bvals, bdvals, searched);
+        bcsr_build_kernel<1><<<blocks, 128, 0, s>>>((int)n, order, inv_order, indptr, indices, data, ddata, nblk, bptr, bidx, bvals, bdvals, searched);
     GP_COUNT(1);
     GP_LAUNCH_CHECK();
     return 0;
 }
 
-static int bcsr_build_any(int64_t R, int pass, int64_t n, const int* order, const int* inv_order, const int* indptr,
-                          const int* indices, const double* data, const double* ddata, int* nblk, const int64_t* bptr,
-                          int* bidx, double* bvals, double* bdvals, int* searched, void* stream) {
-    cudaStream_t s = (cudaStream_t)stream;
-    if (!indptr || !indices || n <= 0 || n > INT32_MAX || ((order == nullptr) != (inv_order == nullptr))) return -1;
-    switch (R) {
-        case 8: return bcsr_build<8>(pass, (int)n, order, inv_order, indptr, indices, data, ddata, nblk, bptr, bidx, bvals, bdvals, searched, s);
-        case 16: return bcsr_build<16>(pass, (int)n, order, inv_order, indptr, indices, data, ddata, nblk, bptr, bidx, bvals, bdvals, searched, s);
-        default: return -3;
-    }
-}
-
 extern "C" {
 
-int gp_bcsr_count(int64_t R, int64_t n, const int* order, const int* inv_order, const int* indptr, const int* indices,
-                  int* nblk, int* needs_sorted_dev, void* stream) {
+int gp_bcsr_count(int64_t n, const int* order, const int* inv_order, const int* indptr, const int* indices, int* nblk,
+                  int* needs_sorted_dev, void* stream) {
     if (!nblk) return -1;
     if (needs_sorted_dev) GP_CUDA_CHECK(cudaMemsetAsync(needs_sorted_dev, 0, sizeof(int), (cudaStream_t)stream));
-    return bcsr_build_any(R, 0, n, order, inv_order, indptr, indices, nullptr, nullptr, nblk, nullptr, nullptr, nullptr, nullptr,
-                          needs_sorted_dev, stream);
+    return bcsr_build(0, n, order, inv_order, indptr, indices, nullptr, nullptr, nblk, nullptr, nullptr, nullptr, nullptr,
+                      needs_sorted_dev, stream);
 }
 
-int gp_bcsr_fill(int64_t R, int64_t n, const int* order, const int* inv_order, const int* indptr, const int* indices,
-                 const double* data, const double* ddata, const int64_t* bptr, int64_t nblocks, int* bidx, double* bvals,
-                 double* bdvals, void* stream) {
+int gp_bcsr_fill(int64_t n, const int* order, const int* inv_order, const int* indptr, const int* indices, const double* data,
+                 const double* ddata, const int64_t* bptr, int64_t nblocks, int* bidx, double* bvals, double* bdvals,
+                 void* stream) {
     if (!data || !bptr || !bidx || !bvals || (ddata && !bdvals) || nblocks < 0) return -1;
-    GP_CUDA_CHECK(cudaMemsetAsync(bvals, 0, sizeof(double) * nblocks * R, (cudaStream_t)stream));
-    if (ddata) GP_CUDA_CHECK(cudaMemsetAsync(bdvals, 0, sizeof(double) * nblocks * R, (cudaStream_t)stream));
-    return bcsr_build_any(R, 1, n, order, inv_order, indptr, indices, data, ddata, nullptr, bptr, bidx, bvals, bdvals, nullptr,
-                          stream);
+    GP_CUDA_CHECK(cudaMemsetAsync(bvals, 0, sizeof(double) * nblocks * BCSR_ROWS, (cudaStream_t)stream));
+    if (ddata) GP_CUDA_CHECK(cudaMemsetAsync(bdvals, 0, sizeof(double) * nblocks * BCSR_ROWS, (cudaStream_t)stream));
+    return bcsr_build(1, n, order, inv_order, indptr, indices, data, ddata, nullptr, bptr, bidx, bvals, bdvals, nullptr, stream);
 }
 
 int gp_rademacher(double* V, int64_t n, int64_t B, uint64_t seed, int64_t probe_offset, const int* row_map, void* stream) {
@@ -741,7 +709,7 @@ int gp_rademacher(double* V, int64_t n, int64_t B, uint64_t seed, int64_t probe_
 }
 
 static size_t partial_rows(int64_t n) {
-    int64_t parts = bcsr8_parts((int)n);
+    int64_t parts = bcsr_parts((int)n);
     return (size_t)(parts < RED_PARTS ? RED_PARTS : parts);
 }
 // reduction partials: the main list followed by the first-stage scratch (1/256 of it)
@@ -754,28 +722,18 @@ int64_t gp_krylov_workspace_bytes(int64_t n, int64_t B) {
     return (int64_t)(4 * al256(sizeof(double) * n * B) + partial_bytes(n) + 16 * al256(sizeof(double) * 32));
 }
 
-// out[c] = sum_i X[i][c] * Y[i][c]
-static int col_dot_run(PeerCtx* px, const double* X, const double* Y, int64_t n, int64_t B, double* out_dev, void* ws,
-                       void* stream) {
+// out[c] = sum_i X[i][c] * Y[i][c]; row-slab operator (`peer`): X, Y are this rank's rows and out holds the dot products
+// over ALL rows (identical on every rank)
+int gp_col_dot(void* peer, const double* X, const double* Y, int64_t n, int64_t B, double* out_dev, void* ws, void* stream) {
     if (!X || !Y || !out_dev || !ws || B <= 0 || B > 32 || (32 % B)) return -1;
     cudaStream_t s = (cudaStream_t)stream;
     double* partial = (double*)ws;
     col_fused_kernel<0><<<RED_PARTS, 256, 0, s>>>(n * B, (int)B, X, Y, nullptr, nullptr, nullptr, nullptr, partial);
-    col_final_kernel<<<1, 256, 0, s>>>(partial, RED_PARTS, (int)B, 0, out_dev, nullptr, nullptr, nullptr, 0.0, peer_next(px));
+    col_final_kernel<<<1, 256, 0, s>>>(partial, RED_PARTS, (int)B, 0, out_dev, nullptr, nullptr, nullptr, 0.0,
+                                       peer_next((PeerCtx*)peer));
     GP_COUNT(2);
     GP_LAUNCH_CHECK();
     return 0;
-}
-
-int gp_col_dot(const double* X, const double* Y, int64_t n, int64_t B, double* out_dev, void* ws, void* stream) {
-    return col_dot_run(nullptr, X, Y, n, B, out_dev, ws, stream);
-}
-
-// row-slab operator: X, Y are this rank's rows; out = the dot products over ALL rows (identical on every rank)
-int gp_slab_col_dot(void* peer, const double* X, const double* Y, int64_t nloc, int64_t B, double* out_dev, void* ws,
-                    void* stream) {
-    if (!peer) return -1;
-    return col_dot_run((PeerCtx*)peer, X, Y, nloc, B, out_dev, ws, stream);
 }
 
 }  // extern "C"
@@ -925,11 +883,12 @@ int gp_lanczos(const int* indptr, const int* indices, const double* data, int64_
     return lanczos_run(csr_op(indptr, indices, data, n), eta, V, B, m, alpha_dev, beta_dev, basis_dev, ws, stream);
 }
 
-int gp_bcsr_lanczos(int64_t R, const int64_t* bptr, const int* bidx, const double* bvals, int64_t n, double eta,
+int gp_bcsr_lanczos(void* peer, const int64_t* bptr, const int* bidx, const double* bvals, int64_t n, double eta,
                     const double* V, int64_t B, int64_t m, double* alpha_dev, double* beta_dev, double* basis_dev, void* ws,
                     void* stream) {
-    if (!bptr || n <= 0 || n > INT32_MAX || (R != 8 && R != 16)) return -1;
-    return lanczos_run(bcsr_op(R, bptr, bidx, bvals, n), eta, V, B, m, alpha_dev, beta_dev, basis_dev, ws, stream);
+    if (!bptr || n <= 0 || n > INT32_MAX) return -1;
+    return lanczos_run(bcsr_op(bptr, bidx, bvals, n), eta, V, B, m, alpha_dev, beta_dev, basis_dev, ws, stream,
+                       (PeerCtx*)peer);
 }
 
 // X[i][c] = sum_j coef[j][c] basis[j][i][c]: the Lanczos solution ||v|| Q T^-1 e_1 from the kept vectors
@@ -953,10 +912,10 @@ int gp_cg_solve(const int* indptr, const int* indices, const double* data, int64
     return cg_run(csr_op(indptr, indices, data, n), eta, R0, X, B, tol, maxiter, iters_host, ws, stream);
 }
 
-int gp_bcsr_cg_solve(int64_t R, const int64_t* bptr, const int* bidx, const double* bvals, int64_t n, double eta, double* R0,
+int gp_bcsr_cg_solve(void* peer, const int64_t* bptr, const int* bidx, const double* bvals, int64_t n, double eta, double* R0,
                      double* X, int64_t B, double tol, int64_t maxiter, int64_t* iters_host, void* ws, void* stream) {
-    if (!bptr || n <= 0 || n > INT32_MAX || (R != 8 && R != 16)) return -1;
-    return cg_run(bcsr_op(R, bptr, bidx, bvals, n), eta, R0, X, B, tol, maxiter, iters_host, ws, stream);
+    if (!bptr || n <= 0 || n > INT32_MAX) return -1;
+    return cg_run(bcsr_op(bptr, bidx, bvals, n), eta, R0, X, B, tol, maxiter, iters_host, ws, stream, (PeerCtx*)peer);
 }
 
 // ---- row-slab operator on several GPUs (one process per GPU, peers' arenas mapped: gp_peer_*) ---------------------------------
@@ -1019,36 +978,6 @@ int gp_slab_encode_columns(int* bidx, int64_t total, int64_t slab, int64_t rank,
         halo_host[1] = (int64_t)h[1];
     }
     return 0;
-}
-
-// Y = (K + eta I) X restricted to this rank's rows. X (nloc x B, this rank's rows) is first copied into exchange vector 2;
-// a barrier before (every rank's copy is in place) and after (nobody overwrites it while a peer still gathers) the SpMM.
-int gp_slab_spmm(void* peer, const int64_t* bptr, const int* bidx, const double* bvals, int64_t nloc, double eta,
-                 const double* X, int64_t B, double* Y, void* stream) {
-    PeerCtx* px = (PeerCtx*)peer;
-    if (!px || !bptr || !bidx || !bvals || !X || !Y || nloc <= 0 || nloc > INT32_MAX) return -1;
-    cudaStream_t s = (cudaStream_t)stream;
-    double* E = peer_local_vec(px, 2);
-    PeerVec pv = peer_vec(px, 2);
-    GP_CUDA_CHECK(cudaMemcpyAsync(E, X, sizeof(double) * nloc * B, cudaMemcpyDeviceToDevice, s));
-    if (int rc = peer_barrier_launch(px, s)) return rc;
-    if (int rc = spmm(bcsr_op(16, bptr, bidx, bvals, nloc), eta, E, (int)B, Y, s, nullptr, nullptr, nullptr, &pv)) return rc;
-    return peer_barrier_launch(px, s);
-}
-
-int gp_slab_lanczos(void* peer, const int64_t* bptr, const int* bidx, const double* bvals, int64_t nloc, double eta,
-                    const double* V, int64_t B, int64_t m, double* alpha_dev, double* beta_dev, double* basis_dev, void* ws,
-                    void* stream) {
-    if (!peer || !bptr || nloc <= 0 || nloc > INT32_MAX) return -1;
-    return lanczos_run(bcsr_op(16, bptr, bidx, bvals, nloc), eta, V, B, m, alpha_dev, beta_dev, basis_dev, ws, stream,
-                       (PeerCtx*)peer);
-}
-
-int gp_slab_cg_solve(void* peer, const int64_t* bptr, const int* bidx, const double* bvals, int64_t nloc, double eta,
-                     double* R0, double* X, int64_t B, double tol, int64_t maxiter, int64_t* iters_host, void* ws,
-                     void* stream) {
-    if (!peer || !bptr || nloc <= 0 || nloc > INT32_MAX) return -1;
-    return cg_run(bcsr_op(16, bptr, bidx, bvals, nloc), eta, R0, X, B, tol, maxiter, iters_host, ws, stream, (PeerCtx*)peer);
 }
 
 }  // extern "C"

@@ -52,24 +52,21 @@ SIGNATURES = {
     'gp_predict_grad_dense': (_int, [_vp, _i64, _vp, _i64, _i64, _vp, _f64, _vp, _i64, _vp, _i64, _vp, _vp, _vp]),
     'gp_kernel_threshold': (_int, [_i64, _i64, _f64, _vp, _f64, _vp]),
     'gp_sparse_workspace_bytes': (_i64, [_i64, _i64]),
-    'gp_matern_sparse_count': (_int, [_vp, _vp, _i64, _i64, _vp, _f64, _f64, _vp, _vp, _vp, _vp]),
-    'gp_matern_sparse_fill': (_int, [_vp, _vp, _i64, _i64, _vp, _f64, _f64, _vp, _vp, _vp, _vp, _vp, _int, _vp]),
-    'gp_matern_sparse_count_rows': (_int, [_vp, _vp, _i64, _i64, _vp, _f64, _f64, _vp, _vp, _vp, _vp, _i64, _i64, _vp]),
-    'gp_matern_sparse_fill_rows': (_int, [_vp, _vp, _i64, _i64, _vp, _f64, _f64, _vp, _vp, _vp, _vp, _vp, _int, _vp, _i64, _i64,
-                                          _vp]),
+    'gp_matern_sparse_count': (_int, [_vp, _vp, _i64, _i64, _vp, _f64, _f64, _vp, _vp, _vp, _vp, _i64, _i64, _vp]),
+    'gp_matern_sparse_fill': (_int, [_vp, _vp, _i64, _i64, _vp, _f64, _f64, _vp, _vp, _vp, _vp, _vp, _int, _vp, _i64, _i64, _vp]),
     'gp_csr_sort_rows': (_int, [_i64, _vp, _vp, _vp, _vp, _vp, _vp]),
     'gp_csr_spmm': (_int, [_vp, _vp, _vp, _i64, _f64, _vp, _i64, _vp, _vp]),
     'gp_rademacher': (_int, [_vp, _i64, _i64, ctypes.c_uint64, _i64, _vp, _vp]),
     'gp_spatial_keys': (_int, [_vp, _i64, _i64, _vp, _vp, _vp, _vp]),
-    'gp_bcsr_count': (_int, [_i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
-    'gp_bcsr_fill': (_int, [_i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp]),
-    'gp_bcsr_spmm': (_int, [_i64, _vp, _vp, _vp, _i64, _f64, _vp, _i64, _vp, _vp]),
+    'gp_bcsr_count': (_int, [_i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    'gp_bcsr_fill': (_int, [_i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp]),
+    'gp_bcsr_spmm': (_int, [_vp, _vp, _vp, _vp, _i64, _f64, _vp, _i64, _vp, _vp]),
     'gp_gram_workspace_bytes': (_i64, [_i64]),
     'gp_gram_skinny': (_int, [_vp, _vp, _i64, _i64, _vp, _vp, _vp]),
-    'gp_bcsr_lanczos': (_int, [_i64, _vp, _vp, _vp, _i64, _f64, _vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
-    'gp_bcsr_cg_solve': (_int, [_i64, _vp, _vp, _vp, _i64, _f64, _vp, _vp, _i64, _f64, _i64, _vp, _vp, _vp]),
+    'gp_bcsr_lanczos': (_int, [_vp, _vp, _vp, _vp, _i64, _f64, _vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
+    'gp_bcsr_cg_solve': (_int, [_vp, _vp, _vp, _vp, _i64, _f64, _vp, _vp, _i64, _f64, _i64, _vp, _vp, _vp]),
     'gp_krylov_workspace_bytes': (_i64, [_i64, _i64]),
-    'gp_col_dot': (_int, [_vp, _vp, _i64, _i64, _vp, _vp, _vp]),
+    'gp_col_dot': (_int, [_vp, _vp, _vp, _i64, _i64, _vp, _vp, _vp]),
     'gp_lanczos': (_int, [_vp, _vp, _vp, _i64, _f64, _vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
     'gp_block_combine': (_int, [_vp, _i64, _i64, _i64, _vp, _vp, _vp]),
     'gp_cg_solve': (_int, [_vp, _vp, _vp, _i64, _f64, _vp, _vp, _i64, _f64, _i64, _vp, _vp, _vp]),
@@ -101,10 +98,6 @@ SIGNATURES = {
     'gp_peer_allreduce': (_int, [_vp, _vp, _i64, _vp]),
     'gp_peer_error': (_int, [_vp, _vp]),
     'gp_slab_encode_columns': (_int, [_vp, _i64, _i64, _i64, _i64, _vp, _vp, _vp]),
-    'gp_slab_spmm': (_int, [_vp, _vp, _vp, _vp, _i64, _f64, _vp, _i64, _vp, _vp]),
-    'gp_slab_col_dot': (_int, [_vp, _vp, _vp, _i64, _i64, _vp, _vp, _vp]),
-    'gp_slab_lanczos': (_int, [_vp, _vp, _vp, _vp, _i64, _f64, _vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
-    'gp_slab_cg_solve': (_int, [_vp, _vp, _vp, _vp, _i64, _f64, _vp, _vp, _i64, _f64, _i64, _vp, _vp, _vp]),
     'gp_sytrd_workspace_bytes': (_i64, [_i64]),
     'gp_sytrd_f64': (_int, [_vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
     'gp_stebz_f64': (_int, [_vp, _vp, _i64, _vp, _vp, _vp]),

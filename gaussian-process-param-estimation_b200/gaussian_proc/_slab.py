@@ -30,11 +30,11 @@ lib = dev.lib
 __all__ = ['SlabSparseEngine', 'slab_geometry', 'PeerArena']
 
 
-def slab_geometry(n, world, rank, block_rows=16):
-    """(slab, first, last): uniform slabs of `slab` rows (a multiple of the row-block height), this rank's rows are
+def slab_geometry(n, world, rank):
+    """(slab, first, last): uniform slabs of `slab` rows (a multiple of the 16-row block height), this rank's rows are
     [first, last) of the ordered operator. The last slab may be short."""
     per = (n + world - 1) // world
-    slab = (per + block_rows - 1) // block_rows * block_rows
+    slab = (per + 15) // 16 * 16
     first = min(n, rank * slab)
     return slab, first, min(n, first + slab)
 
@@ -105,8 +105,9 @@ class PeerArena(object):
 
 
 class SlabSparseEngine(SparseEngine):
-    """SparseEngine on this rank's slab of rows. Same interface and - to rounding of the reordered sums - the same numbers
-    as SparseEngine on one GPU; every rank of the group must make the same calls in the same order."""
+    """SparseEngine on this rank's slab of rows, with the peer arenas that carry the halo rows and the reductions. Same
+    interface and - to rounding of the reordered sums - the same numbers as SparseEngine on one GPU; every rank of the
+    group must make the same calls in the same order."""
 
     def __init__(self, K, imate_method='slq', imate_options=None, rank=None, world=None):
         from ._distributed import rank_world
@@ -117,9 +118,6 @@ class SlabSparseEngine(SparseEngine):
             raise ValueError('the row-slab engine needs a device handle from generate_sparse_operator / '
                              'generate_sparse_correlation(..., device=True).')
         opts = dict(imate_options or {})
-        if int(opts.get('block_rows', 16)) != 16:
-            raise ValueError('the row-slab engine works on 16-row blocks.')
-        opts['block_rows'] = 16
         self.slab, self.first_row, self.last_row = slab_geometry(K.n, self.world, self.rank)
         if self.last_row <= self.first_row:
             raise ValueError('n = %d is too small for %d slabs of 16-row blocks.' % (K.n, self.world))
@@ -137,85 +135,6 @@ class SlabSparseEngine(SparseEngine):
         SparseEngine.__init__(self, K, imate_method, opts, probe_range=None)
 
     # ---- operator -------------------------------------------------------------------------------------------------
-    def _halo_ws(self):
-        """scratch of the halo statistics: two counters + one bit per row of the operator"""
-        return dev.torch.empty(2 + (self.n + 63) // 64 + 1, dtype=dev.torch.int64, device='cuda')
-
-    def _build_blocked(self, K, R):
-        torch = dev.torch
-        n, r0, r1 = self.n, self.first_row, self.last_row
-        nloc = r1 - r0
-        s = dev.stream_ptr()
-        if isinstance(K, DeviceRowBlocks):         # generated as the row blocks of this slab: only the column encoding is left
-            total = K.bidx.numel()
-            if K.encoded is None:
-                halo = (ctypes.c_int64 * 2)()
-                check(lib.gp_slab_encode_columns(_p(K.bidx), total, self.slab, self.rank, n, halo, _p(self._halo_ws()), s),
-                      'gp_slab_encode_columns')
-                K.encoded = (self.slab, self.rank, int(halo[0]), int(halo[1]))
-            elif K.encoded[:2] != (self.slab, self.rank):
-                raise ValueError('this operator was encoded for another slab geometry')
-            self.halo_blocks, self.halo_rows, self.total_blocks = K.encoded[2], K.encoded[3], total
-            self.halo_fraction = self.halo_blocks / float(max(total, 1))
-            self.R, self.rows = R, nloc
-            self.blocked = (K.bptr, K.bidx, K.bvals, K.bdvals)
-            self.fill_ratio = total * R / float(max(K.nnz, 1))
-            self.order, self.inv_order = K.order, K.inv_order
-            self._my_rows = K.order[r0:r1]
-            return
-        inv = getattr(K, 'inv_order', None)
-        if inv is None:
-            inv = torch.empty(n, dtype=torch.int32, device='cuda')
-            check(lib.gp_inverse_permutation(_p(K.order), n, _p(inv), s), 'gp_inverse_permutation')
-        my_rows = K.order[r0:r1]                              # original ids of this rank's rows (contiguous int32 view)
-        nrb = (nloc + R - 1) // R
-        nblk = torch.empty(nrb, dtype=torch.int32, device='cuda')
-        flag = torch.zeros(1, dtype=torch.int32, device='cuda')
-        check(lib.gp_bcsr_count(R, nloc, _p(my_rows), _p(inv), _p(K.indptr), _p(K.indices), _p(nblk), _p(flag), s),
-              'gp_bcsr_count')
-        if not K.sorted_rows and int(flag.item()) != 0:
-            K.canonicalize()
-            check(lib.gp_bcsr_count(R, nloc, _p(my_rows), _p(inv), _p(K.indptr), _p(K.indices), _p(nblk), _p(flag), s),
-                  'gp_bcsr_count')
-        bptr = torch.empty(nrb + 1, dtype=torch.int64, device='cuda')
-        check(lib.gp_scan_counts(_p(nblk), nrb, _p(bptr), s), 'gp_scan_counts')
-        total = int(bptr[-1].item())
-        bidx = torch.empty(total, dtype=torch.int32, device='cuda')
-        bvals = torch.empty(total * R, dtype=torch.float64, device='cuda')
-        bdvals = torch.empty(total * R, dtype=torch.float64, device='cuda') if K.ddata is not None else None
-        check(lib.gp_bcsr_fill(R, nloc, _p(my_rows), _p(inv), _p(K.indptr), _p(K.indices), _p(K.data),
-                               _p(K.ddata) if K.ddata is not None else None, _p(bptr), total, _p(bidx), _p(bvals),
-                               _p(bdvals) if bdvals is not None else None, s), 'gp_bcsr_fill')
-        halo = (ctypes.c_int64 * 2)()   # block-columns whose row of X lives on another rank, and the distinct rows among them
-        check(lib.gp_slab_encode_columns(_p(bidx), total, self.slab, self.rank, n, halo, _p(self._halo_ws()), s),
-              'gp_slab_encode_columns')
-        self.halo_blocks, self.halo_rows, self.total_blocks = int(halo[0]), int(halo[1]), total
-        self.halo_fraction = halo[0] / float(max(total, 1))
-        self.R = R
-        self.rows = nloc
-        self.blocked = (bptr, bidx, bvals, bdvals)
-        self.fill_ratio = total * R / float(max(K.nnz, 1)) * (1 if getattr(K, 'row_slab', None) else self.world)
-        self.order, self.inv_order = K.order, inv
-        self._my_rows = my_rows
-
-    def spmm(self, eta, X_dev, derivative=False):
-        torch = dev.torch
-        B = X_dev.shape[1]
-        X_dev = X_dev.contiguous()
-        Y = torch.empty_like(X_dev)
-        bptr, bidx, bvals, bdvals = self.blocked
-        check(lib.gp_slab_spmm(self.peer.ctx, _p(bptr), _p(bidx), _p(bdvals if derivative else bvals), self.rows, float(eta),
-                               _p(X_dev), B, _p(Y), dev.stream_ptr()), 'gp_slab_spmm')
-        return Y
-
-    def to_op(self, X_dev):
-        """this rank's rows (operator order) of a FULL (n x B) block given in the caller's row order"""
-        X_dev = X_dev.contiguous()
-        B = X_dev.numel() // self.n
-        Y = dev.torch.empty((self.rows, B), dtype=dev.torch.float64, device='cuda')
-        check(lib.gp_gather_rows(_p(X_dev), _p(self._my_rows), self.rows, B, _p(Y), dev.stream_ptr()), 'gp_gather_rows')
-        return Y
-
     def from_op(self, X_dev):
         """the FULL (n x B) block in the caller's row order from the ranks' slabs (host API only: all-gather)"""
         torch = dev.torch
@@ -231,64 +150,6 @@ class SlabSparseEngine(SparseEngine):
         Y = torch.empty((self.n, B), dtype=torch.float64, device='cuda')
         check(lib.gp_gather_rows(_p(full), _p(self.inv_order), self.n, B, _p(Y), dev.stream_ptr()), 'gp_gather_rows')
         return Y
-
-    def probes(self, first, B, out=None):
-        torch = dev.torch
-        V = torch.empty((self.rows, B), dtype=torch.float64, device='cuda') if out is None else out
-        check(lib.gp_rademacher(_p(V), self.rows, B, int(self.opt['seed']), int(first), _p(self._my_rows),
-                                dev.stream_ptr()), 'gp_rademacher')
-        return V
-
-    # ---- Krylov drivers ---------------------------------------------------------------------------------------------
-    def _lanczos_launch(self, eta, V, m, basis=None, alpha=None, beta=None, side=False):
-        torch = dev.torch
-        B = V.shape[1]
-        alpha = torch.empty((m, B), dtype=torch.float64, device='cuda') if alpha is None else alpha
-        beta = torch.empty((m, B), dtype=torch.float64, device='cuda') if beta is None else beta
-        bptr, bidx, bvals, _ = self.blocked
-        peer = self.peer_side if side else self.peer
-        check(lib.gp_slab_lanczos(peer.ctx, _p(bptr), _p(bidx), _p(bvals), self.rows, float(eta), _p(V), B, m, _p(alpha),
-                                  _p(beta), _p(basis) if basis is not None else None, _p(self._workspace(B, side)),
-                                  dev.stream_ptr()), 'gp_slab_lanczos')
-        return alpha, beta
-
-    def col_dot(self, X, Y):
-        torch = dev.torch
-        B = X.shape[1]
-        out = torch.empty(32, dtype=torch.float64, device='cuda')
-        check(lib.gp_slab_col_dot(self.peer.ctx, _p(X), _p(Y), self.rows, B, _p(out), _p(self._workspace(B)),
-                                  dev.stream_ptr()), 'gp_slab_col_dot')
-        return out[:B].cpu().numpy()
-
-    def solve_dev(self, eta, R_dev):
-        torch = dev.torch
-        B = R_dev.shape[1]
-        X = torch.empty_like(R_dev)
-        it = ctypes.c_int64()
-        bptr, bidx, bvals, _ = self.blocked
-        rc = lib.gp_slab_cg_solve(self.peer.ctx, _p(bptr), _p(bidx), _p(bvals), self.rows, float(eta), _p(R_dev), _p(X), B,
-                                  float(self.opt['cg_tol']), int(self.opt['cg_maxiter']), ctypes.byref(it),
-                                  _p(self._workspace(B)), dev.stream_ptr())
-        check(rc, 'gp_slab_cg_solve')
-        self.last_cg_iterations = it.value
-        if rc == 2:
-            raise numpy.linalg.LinAlgError(
-                'K + eta*I (eta=%g) is not positive definite (CG met p^T A p <= 0). The thresholded Matern matrix is '
-                'indefinite; use a larger eta (reference: _generate_sparse_correlation.pyx:516-523).' % eta)
-        if rc == 1:
-            raise numpy.linalg.LinAlgError('CG did not converge in %d iterations (eta=%g)' % (it.value, eta))
-        return X
-
-    def gram(self, X_dev, Y_dev):
-        torch = dev.torch
-        B = X_dev.shape[1]
-        if '_gram' not in self._ws:
-            self._ws['_gram'] = torch.empty(lib.gp_gram_workspace_bytes(16) // 8, dtype=torch.float64, device='cuda')
-        out = torch.empty(B * B, dtype=torch.float64, device='cuda')
-        s = dev.stream_ptr()
-        check(lib.gp_gram_skinny(_p(X_dev), _p(Y_dev), self.rows, B, _p(out), _p(self._ws['_gram']), s), 'gp_gram_skinny')
-        check(lib.gp_peer_allreduce(self.peer.ctx, _p(out), B * B, s), 'gp_peer_allreduce')
-        return out.cpu().numpy().reshape(B, B)
 
     def fused(self, eta, X, z, traceinv=True, drho=True, cubic=False):
         out = SparseEngine.fused(self, eta, X, z, traceinv=traceinv, drho=drho, cubic=cubic)

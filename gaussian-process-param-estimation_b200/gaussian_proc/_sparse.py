@@ -28,7 +28,7 @@ __all__ = ['DeviceCSR', 'DeviceRowBlocks', 'SparseEngine', 'generate_sparse_corr
 
 # imate's documented defaults for the stochastic estimators (SURVEY 8c)
 DEFAULTS = dict(min_num_samples=10, max_num_samples=50, error_rtol=1e-2, error_atol=None, confidence_level=0.95,
-                lanczos_degree=20, seed=0, batch=16, cg_tol=1e-6, cg_maxiter=2000, block_rows=16, reuse_lanczos=True, overlap=True,
+                lanczos_degree=20, seed=0, batch=16, cg_tol=1e-6, cg_maxiter=2000, reuse_lanczos=True, overlap=True,
                 shift_reuse=True, solve_degree=None, eager_rhs_basis=False)
 
 
@@ -199,38 +199,27 @@ def generate_sparse_correlation(points, correlation_scale, nu, density, verbose=
         raise ValueError('row_slab needs device=True (a slab is not a complete matrix).')
     s = dev.stream_ptr()
     dpts, order, pos = _device_points(points)
-    rows = None
+    rows = (None, 0, 0)              # (row filter, first, last): every row
     if row_slab is not None:
         from ._slab import slab_geometry
         rank, world = int(row_slab[0]), int(row_slab[1])
         _, first, last = slab_geometry(n, world, rank)
-        rows = (pos, first, last)
+        rows = (_p(pos), first, last)
     ws = torch.empty(lib.gp_sparse_workspace_bytes(n, d) // 8 + 8, dtype=torch.float64, device='cuda')
     indptr = torch.empty(n + 1, dtype=torch.int32, device='cuda')
     nnz = ctypes.c_int64()
-    if rows is None:
-        rc = lib.gp_matern_sparse_count(_p(dpts), dev.host_ptr(points), n, d, dev.host_ptr(scale), float(nu), tau, _p(ws),
-                                        _p(indptr), ctypes.byref(nnz), s)
-    else:
-        rc = lib.gp_matern_sparse_count_rows(_p(dpts), dev.host_ptr(points), n, d, dev.host_ptr(scale), float(nu), tau, _p(ws),
-                                             _p(indptr), ctypes.byref(nnz), _p(rows[0]), rows[1], rows[2], s)
-    check(rc, 'gp_matern_sparse_count')
+    check(lib.gp_matern_sparse_count(_p(dpts), dev.host_ptr(points), n, d, dev.host_ptr(scale), float(nu), tau, _p(ws),
+                                     _p(indptr), ctypes.byref(nnz), *rows, s), 'gp_matern_sparse_count')
     indices = torch.empty(nnz.value, dtype=torch.int32, device='cuda')
     data = torch.empty(nnz.value, dtype=torch.float64, device='cuda')
     ddata = torch.empty(nnz.value, dtype=torch.float64, device='cuda') if with_derivative else None
-    if rows is None:
-        rc = lib.gp_matern_sparse_fill(_p(dpts), dev.host_ptr(points), n, d, dev.host_ptr(scale), float(nu), tau, _p(ws),
-                                       _p(indptr), _p(indices), _p(data), _p(ddata) if ddata is not None else None,
-                                       1 if sort_rows else 0, s)
-    else:
-        rc = lib.gp_matern_sparse_fill_rows(_p(dpts), dev.host_ptr(points), n, d, dev.host_ptr(scale), float(nu), tau, _p(ws),
-                                            _p(indptr), _p(indices), _p(data), _p(ddata) if ddata is not None else None,
-                                            1 if sort_rows else 0, _p(rows[0]), rows[1], rows[2], s)
-    check(rc, 'gp_matern_sparse_fill')
+    check(lib.gp_matern_sparse_fill(_p(dpts), dev.host_ptr(points), n, d, dev.host_ptr(scale), float(nu), tau, _p(ws),
+                                    _p(indptr), _p(indices), _p(data), _p(ddata) if ddata is not None else None,
+                                    1 if sort_rows else 0, *rows, s), 'gp_matern_sparse_fill')
     K = DeviceCSR(n, indptr, indices, data, ddata, kernel_threshold=tau, order=order, sorted_rows=sort_rows)
     K.inv_order = pos
-    if rows is not None:
-        K.row_slab = (rank, world, rows[1], rows[2])       # only these rows of the ordered operator are present
+    if row_slab is not None:
+        K.row_slab = (rank, world, first, last)       # only these rows of the ordered operator are present
     if verbose:
         print('Generated sparse correlation matrix using kernel threshold: %0.4f and sparse density: %0.2e.'
               % (tau, K.nnz / float(n) ** 2))
@@ -345,7 +334,10 @@ def lanczos_block_quadrature(alpha, beta, vnorm=None):
 
 
 class SparseEngine(object):
-    """Stochastic logdet / traceinv and CG solves for K + eta I with K in device CSR."""
+    """Stochastic logdet / traceinv and CG solves for K + eta I with K in device CSR or row blocks. On one GPU the engine
+    works on every row; the row-slab engine (gaussian_proc/_slab.py) is this engine on one slab of rows with a peer."""
+
+    peer = peer_side = None        # row-slab engine: this rank's PeerArena and the one of the prefetch stream
 
     def __init__(self, K, imate_method='slq', imate_options=None, probe_range=None):
         dev.require_cuda()
@@ -353,7 +345,9 @@ class SparseEngine(object):
             K = DeviceCSR.from_scipy(K)
         self.K = K
         self.n = K.n
-        self.rows = K.n            # rows of the vectors this engine works on (a slab of n on the row-slab engine, _slab.py)
+        if self.peer is None:      # one GPU: the rows [first_row, last_row) of the operator are all of them
+            self.first_row, self.last_row = 0, K.n
+        self.rows = self.last_row - self.first_row      # rows of the vectors this engine works on
         self.method = imate_method
         self.opt = dict(DEFAULTS)
         self.opt.update(imate_options or {})
@@ -364,62 +358,76 @@ class SparseEngine(object):
         self.last_info = {}
         # multi-GPU: (rank, world) -> this engine evaluates its slice of every round of probes; see _run_estimator
         self.probe_range = probe_range
-        # Internally the operator works on the ROW-BLOCKED form of the symmetrically permuted matrix P K P^T (rows in
-        # the generator's Z-order): 8 consecutive rows share one column list, so one gathered row of the probe block
-        # serves 8 rows of K and four such block-columns are one DMMA.8x8x4 (csrc/gp_sparse_la.cu). Results do not depend
-        # on the permutation: probes are hashed with ORIGINAL row ids. block_rows = 1 (or a K without an order, e.g. from
-        # SciPy) keeps plain CSR in the original order.
+        # A K with a spatial order (from the device generators) is worked on as the ROW-BLOCKED form of the symmetrically
+        # permuted matrix P K P^T (rows in that order): 16 consecutive rows share one column list, so one gathered row of
+        # the probe block serves 16 rows of K and four such block-columns are one DMMA.8x8x4 (csrc/gp_sparse_la.cu).
+        # Results do not depend on the permutation: probes are hashed with ORIGINAL row ids. A K without an order (e.g.
+        # from SciPy) stays plain CSR in the original order.
         self.order = self.inv_order = None
-        self.R = 1
+        self.R = 1                 # rows per block of the operator in use: 16 row-blocked, 1 plain CSR
         self.blocked = None
-        R = int(self.opt.get('block_rows', 16))
-        if R not in (1, 8, 16):
-            raise ValueError('block_rows should be 8 or 16 (row-blocked, FP64 tensor-core SpMM) or 1 (plain CSR).')
-        if isinstance(K, DeviceRowBlocks) and R != 16:
-            raise ValueError('a directly generated operator (DeviceRowBlocks) has 16-row blocks.')
-        if K.order is not None and R > 1:
-            self._build_blocked(K, R)
+        if K.order is not None:
+            self._build_blocked(K)
 
-    def _build_blocked(self, K, R):
+    def _build_blocked(self, K):
+        """The 16-row blocks of the rows [first_row, last_row) of the ordered operator: those of a DeviceRowBlocks as
+        they are, else built from the CSR. With a peer the block-columns are encoded as (owner rank, row in its slab)."""
         torch = dev.torch
-        n = self.n
+        n, r0, r1, R = self.n, self.first_row, self.last_row, 16
+        s = dev.stream_ptr()
+        my_rows = K.order[r0:r1]   # original ids of this engine's rows (contiguous int32 view)
+        share = 1                  # 1 / the share of K's entries that lie in the rows built
         if isinstance(K, DeviceRowBlocks):         # generated as row blocks: nothing to build
-            if (K.first_row, K.last_row) != (0, n) or K.encoded is not None:
+            if self.peer is None and ((K.first_row, K.last_row) != (0, n) or K.encoded is not None):
                 raise ValueError('this operator holds one slab of rows (or its columns were encoded for the row-slab engine): '
                                  'use the row-slab engine (row_slabs=True).')
-            self.R = R
-            self.blocked = (K.bptr, K.bidx, K.bvals, K.bdvals)
-            self.fill_ratio = K.bidx.numel() * R / float(max(K.nnz, 1))
-            self.order, self.inv_order = K.order, K.inv_order
-            return
-        s = dev.stream_ptr()
-        inv = getattr(K, 'inv_order', None)
-        if inv is None:
-            inv = torch.empty(n, dtype=torch.int32, device='cuda')
-            check(lib.gp_inverse_permutation(_p(K.order), n, _p(inv), s), 'gp_inverse_permutation')
-        nrb = (n + R - 1) // R
-        nblk = torch.empty(nrb, dtype=torch.int32, device='cuda')
-        flag = torch.zeros(1, dtype=torch.int32, device='cuda')
-        check(lib.gp_bcsr_count(R, n, _p(K.order), _p(inv), _p(K.indptr), _p(K.indices), _p(nblk), _p(flag), s),
-              'gp_bcsr_count')
-        if not K.sorted_rows and int(flag.item()) != 0:
-            # some row block is too wide for the hash path: its binary-search fallback needs canonical rows
-            K.canonicalize()
-            check(lib.gp_bcsr_count(R, n, _p(K.order), _p(inv), _p(K.indptr), _p(K.indices), _p(nblk), _p(flag), s),
+            bptr, bidx, bvals, bdvals, inv, encoded = K.bptr, K.bidx, K.bvals, K.bdvals, K.inv_order, K.encoded
+        else:
+            inv = getattr(K, 'inv_order', None)
+            if inv is None:
+                inv = torch.empty(n, dtype=torch.int32, device='cuda')
+                check(lib.gp_inverse_permutation(_p(K.order), n, _p(inv), s), 'gp_inverse_permutation')
+            nrb = (self.rows + R - 1) // R
+            nblk = torch.empty(nrb, dtype=torch.int32, device='cuda')
+            flag = torch.zeros(1, dtype=torch.int32, device='cuda')
+            check(lib.gp_bcsr_count(self.rows, _p(my_rows), _p(inv), _p(K.indptr), _p(K.indices), _p(nblk), _p(flag), s),
                   'gp_bcsr_count')
-        bptr = torch.empty(nrb + 1, dtype=torch.int64, device='cuda')
-        check(lib.gp_scan_counts(_p(nblk), nrb, _p(bptr), s), 'gp_scan_counts')
-        total = int(bptr[-1].item())
-        bidx = torch.empty(total, dtype=torch.int32, device='cuda')
-        bvals = torch.empty(total * R, dtype=torch.float64, device='cuda')
-        bdvals = torch.empty(total * R, dtype=torch.float64, device='cuda') if K.ddata is not None else None
-        check(lib.gp_bcsr_fill(R, n, _p(K.order), _p(inv), _p(K.indptr), _p(K.indices), _p(K.data),
-                               _p(K.ddata) if K.ddata is not None else None, _p(bptr), total, _p(bidx), _p(bvals),
-                               _p(bdvals) if bdvals is not None else None, s), 'gp_bcsr_fill')
+            if not K.sorted_rows and int(flag.item()) != 0:
+                # some row block is too wide for the hash path: its binary-search fallback needs canonical rows
+                K.canonicalize()
+                check(lib.gp_bcsr_count(self.rows, _p(my_rows), _p(inv), _p(K.indptr), _p(K.indices), _p(nblk), _p(flag), s),
+                      'gp_bcsr_count')
+            bptr = torch.empty(nrb + 1, dtype=torch.int64, device='cuda')
+            check(lib.gp_scan_counts(_p(nblk), nrb, _p(bptr), s), 'gp_scan_counts')
+            total = int(bptr[-1].item())
+            bidx = torch.empty(total, dtype=torch.int32, device='cuda')
+            bvals = torch.empty(total * R, dtype=torch.float64, device='cuda')
+            bdvals = torch.empty(total * R, dtype=torch.float64, device='cuda') if K.ddata is not None else None
+            check(lib.gp_bcsr_fill(self.rows, _p(my_rows), _p(inv), _p(K.indptr), _p(K.indices), _p(K.data),
+                                   _p(K.ddata) if K.ddata is not None else None, _p(bptr), total, _p(bidx), _p(bvals),
+                                   _p(bdvals) if bdvals is not None else None, s), 'gp_bcsr_fill')
+            encoded = None
+            if self.peer is not None and getattr(K, 'row_slab', None) is None:
+                share = self.world     # a handle with every row, of which this slab is built
+        total = bidx.numel()
+        if self.peer is not None:
+            if encoded is None:
+                halo = (ctypes.c_int64 * 2)()   # block-columns whose row of X lives on another rank, and the distinct rows among them
+                ws = torch.empty(2 + (n + 63) // 64 + 1, dtype=torch.int64, device='cuda')
+                check(lib.gp_slab_encode_columns(_p(bidx), total, self.slab, self.rank, n, halo, _p(ws), s),
+                      'gp_slab_encode_columns')
+                encoded = (self.slab, self.rank, int(halo[0]), int(halo[1]))
+                if isinstance(K, DeviceRowBlocks):
+                    K.encoded = encoded        # its bidx now carries the encoding
+            elif encoded[:2] != (self.slab, self.rank):
+                raise ValueError('this operator was encoded for another slab geometry')
+            self.halo_blocks, self.halo_rows, self.total_blocks = encoded[2], encoded[3], total
+            self.halo_fraction = self.halo_blocks / float(max(total, 1))
         self.R = R
         self.blocked = (bptr, bidx, bvals, bdvals)
-        self.fill_ratio = total * R / float(max(K.nnz, 1))     # stored values per original nonzero (>= 1)
+        self.fill_ratio = total * R / float(max(K.nnz, 1)) * share     # stored values per original nonzero (>= 1)
         self.order, self.inv_order = K.order, inv            # device int32 row maps of to_op / from_op
+        self._my_rows = my_rows
 
     # ---- plumbing ----------------------------------------------------------------------------------------------
     def _workspace(self, B, side=False):
@@ -431,40 +439,52 @@ class SparseEngine(object):
             self._ws[key] = torch.empty(lib.gp_krylov_workspace_bytes(self.rows, B) // 8 + 8, dtype=torch.float64, device='cuda')
         return self._ws[key]
 
+    def _peer_ctx(self, side=False):
+        """the peer argument of the row-blocked drivers: NULL on one GPU"""
+        arena = self.peer_side if side else self.peer
+        return arena.ctx if arena is not None else None
+
     def spmm(self, eta, X_dev, derivative=False):
         """(K + eta I) X, or (dK/drho + eta I) X with ``derivative``, in OPERATOR space (rows in self.order when the
         operator is permuted)"""
         torch = dev.torch
         B = X_dev.shape[1]
+        X_dev = X_dev.contiguous()
         Y = torch.empty_like(X_dev)
         if self.blocked is not None:
             bptr, bidx, bvals, bdvals = self.blocked
-            check(lib.gp_bcsr_spmm(self.R, _p(bptr), _p(bidx), _p(bdvals if derivative else bvals), self.n, float(eta),
-                                   _p(X_dev), B, _p(Y), dev.stream_ptr()), 'gp_bcsr_spmm')
+            check(lib.gp_bcsr_spmm(self._peer_ctx(), _p(bptr), _p(bidx), _p(bdvals if derivative else bvals), self.rows,
+                                   float(eta), _p(X_dev), B, _p(Y), dev.stream_ptr()), 'gp_bcsr_spmm')
         else:
             K = self.K
             check(lib.gp_csr_spmm(_p(K.indptr), _p(K.indices), _p(K.ddata if derivative else K.data), self.n, float(eta),
                                   _p(X_dev), B, _p(Y), dev.stream_ptr()), 'gp_csr_spmm')
         return Y
 
-    def _gather(self, X_dev, rmap):
+    def to_op(self, X_dev):
+        """this engine's rows, in operator order, of an (n x B) block given in the caller's row order"""
+        if self.order is None:
+            return X_dev
         X_dev = X_dev.contiguous()
-        Y = dev.torch.empty_like(X_dev)
         B = X_dev.numel() // self.n
-        check(lib.gp_gather_rows(_p(X_dev), _p(rmap), self.n, B, _p(Y), dev.stream_ptr()), 'gp_gather_rows')
+        Y = dev.torch.empty((self.rows, B), dtype=dev.torch.float64, device='cuda')
+        check(lib.gp_gather_rows(_p(X_dev), _p(self._my_rows), self.rows, B, _p(Y), dev.stream_ptr()), 'gp_gather_rows')
         return Y
 
-    def to_op(self, X_dev):
-        """rows of an (n x B) block from the caller's order into operator order"""
-        return X_dev if self.order is None else self._gather(X_dev, self.order)
-
     def from_op(self, X_dev):
-        return X_dev if self.order is None else self._gather(X_dev, self.inv_order)
+        """the (n x B) block in the caller's row order from operator order"""
+        if self.order is None:
+            return X_dev
+        X_dev = X_dev.contiguous()
+        Y = dev.torch.empty_like(X_dev)
+        check(lib.gp_gather_rows(_p(X_dev), _p(self.inv_order), self.n, X_dev.numel() // self.n, _p(Y), dev.stream_ptr()),
+              'gp_gather_rows')
+        return Y
 
     def probes(self, first, B, out=None):
         torch = dev.torch
         V = torch.empty((self.rows, B), dtype=torch.float64, device='cuda') if out is None else out
-        rmap = self.K.order if self.order is not None else None
+        rmap = self._my_rows if self.order is not None else None
         check(lib.gp_rademacher(_p(V), self.rows, B, int(self.opt['seed']), int(first), _p(rmap) if rmap is not None else None,
                                 dev.stream_ptr()), 'gp_rademacher')
         return V
@@ -483,8 +503,9 @@ class SparseEngine(object):
         bp = _p(basis) if basis is not None else None
         if self.blocked is not None:
             bptr, bidx, bvals, _ = self.blocked
-            check(lib.gp_bcsr_lanczos(self.R, _p(bptr), _p(bidx), _p(bvals), self.n, float(eta), _p(V), B, m, _p(alpha),
-                                      _p(beta), bp, _p(self._workspace(B, side)), dev.stream_ptr()), 'gp_bcsr_lanczos')
+            check(lib.gp_bcsr_lanczos(self._peer_ctx(side), _p(bptr), _p(bidx), _p(bvals), self.rows, float(eta), _p(V), B, m,
+                                      _p(alpha), _p(beta), bp, _p(self._workspace(B, side)), dev.stream_ptr()),
+                  'gp_bcsr_lanczos')
         else:
             K = self.K
             check(lib.gp_lanczos(_p(K.indptr), _p(K.indices), _p(K.data), self.n, float(eta), _p(V), B, m, _p(alpha),
@@ -790,7 +811,8 @@ class SparseEngine(object):
         torch = dev.torch
         B = X.shape[1]
         out = torch.empty(32, dtype=torch.float64, device='cuda')
-        check(lib.gp_col_dot(_p(X), _p(Y), self.n, B, _p(out), _p(self._workspace(B)), dev.stream_ptr()), 'gp_col_dot')
+        check(lib.gp_col_dot(self._peer_ctx(), _p(X), _p(Y), self.rows, B, _p(out), _p(self._workspace(B)), dev.stream_ptr()),
+              'gp_col_dot')
         return out[:B].cpu().numpy()
 
     def solve_dev(self, eta, R_dev):
@@ -801,7 +823,7 @@ class SparseEngine(object):
         it = ctypes.c_int64()
         if self.blocked is not None:
             bptr, bidx, bvals, _ = self.blocked
-            rc = lib.gp_bcsr_cg_solve(self.R, _p(bptr), _p(bidx), _p(bvals), self.n, float(eta), _p(R_dev), _p(X), B,
+            rc = lib.gp_bcsr_cg_solve(self._peer_ctx(), _p(bptr), _p(bidx), _p(bvals), self.rows, float(eta), _p(R_dev), _p(X), B,
                                       float(self.opt['cg_tol']), int(self.opt['cg_maxiter']), ctypes.byref(it),
                                       _p(self._workspace(B)), dev.stream_ptr())
         else:
@@ -821,7 +843,7 @@ class SparseEngine(object):
 
     def _max_block(self):
         """widest column block handed to the SpMM: the 16 x 1 row-blocked kernel is tuned for B <= 16"""
-        return 16 if self.blocked is not None and self.R == 16 else 32
+        return 16 if self.blocked is not None else 32
 
     def solve(self, eta, Y):
         """mixed_correlation.py:280-299 for sparse K: CG per column with rtol 1e-6 (batched on the device)."""
@@ -862,14 +884,16 @@ class SparseEngine(object):
 
     # ---- fused likelihood ingredients -------------------------------------------------------------------------
     def gram(self, X_dev, Y_dev):
-        """X^T Y (B x B, host) of two n x B device blocks."""
+        """X^T Y (B x B, host) of two n x B device blocks (with a peer: summed over the ranks' slabs)."""
         torch = dev.torch
         B = X_dev.shape[1]
         if '_gram' not in self._ws:
             self._ws['_gram'] = torch.empty(lib.gp_gram_workspace_bytes(16) // 8, dtype=torch.float64, device='cuda')
         out = torch.empty(B * B, dtype=torch.float64, device='cuda')
-        check(lib.gp_gram_skinny(_p(X_dev), _p(Y_dev), self.n, B, _p(out), _p(self._ws['_gram']), dev.stream_ptr()),
-              'gp_gram_skinny')
+        s = dev.stream_ptr()
+        check(lib.gp_gram_skinny(_p(X_dev), _p(Y_dev), self.rows, B, _p(out), _p(self._ws['_gram']), s), 'gp_gram_skinny')
+        if self.peer is not None:
+            check(lib.gp_peer_allreduce(self.peer.ctx, _p(out), B * B, s), 'gp_peer_allreduce')
         return out.cpu().numpy().reshape(B, B)
 
     def _rhs_block(self, X, z, key=None):

@@ -98,11 +98,15 @@ int gp_kernel_threshold(int64_t n, int64_t d, double density, const double* scal
  * retries with doubled buffers, :548-577): count -> indptr (device int32, n + 1) and nnz (host); fill -> indices
  * (int32, sorted within each row), data and optionally ddata = d/d(rho) values on the same pattern.
  * points: device (n, d); points_host: the same array on the host (bounding box + host re-decision of the pairs with
- * |K - tau| <= 8 ulp, which makes the pattern bit-exact). ws: gp_sparse_workspace_bytes(n, d), shared by both calls. */
+ * |K - tau| <= 8 ulp, which makes the pattern bit-exact). ws: gp_sparse_workspace_bytes(n, d), shared by both calls.
+ * row_pos_dev: NULL for every row. Otherwise (device int32, n) only the rows i with row_first <= row_pos_dev[i] < row_last
+ * are generated - one slab of the spatially ordered operator on the row-slab engine, with row_pos = the position of a row
+ * in that order - and the other rows stay empty; indptr keeps n + 1 entries and the column ids stay global. Work, memory
+ * and time are then those of the slab. Both calls must get the same rows. */
 int64_t gp_sparse_workspace_bytes(int64_t n, int64_t d);
 int gp_matern_sparse_count(const double* points, const double* points_host, int64_t n, int64_t d,
                            const double* scale_host, double nu, double tau, void* ws, int* indptr_dev,
-                           int64_t* nnz_host, void* stream);
+                           int64_t* nnz_host, const int* row_pos_dev, int64_t row_first, int64_t row_last, void* stream);
 /* Space-filling-curve keys of the points over the bounding box [lo_host, hi_host] (d = 2: Hilbert index; otherwise
  * Z-order over the first min(d,3) coordinates): a stable sort by key is the deterministic, spatially local row order the
  * row-blocked sparse operator (gp_bcsr_*) uses. */
@@ -112,17 +116,8 @@ int gp_spatial_keys(const double* points, int64_t n, int64_t d, const double* lo
  * the device operators (gp_csr_spmm, the hash path of gp_bcsr_*); gp_csr_sort_rows canonicalises later, on demand. */
 int gp_matern_sparse_fill(const double* points, const double* points_host, int64_t n, int64_t d,
                           const double* scale_host, double nu, double tau, void* ws, const int* indptr_dev,
-                          int* indices_dev, double* data_dev, double* ddata_dev, int sort_rows, void* stream);
-/* The same two passes for ONE slab of rows (row-slab engine, one slab of the spatially ordered operator per GPU): only rows i
- * with row_first <= row_pos_dev[i] < row_last are generated, the others stay empty; indptr keeps n + 1 entries and the
- * column ids stay global. Work, memory and time are those of the slab. */
-int gp_matern_sparse_count_rows(const double* points, const double* points_host, int64_t n, int64_t d,
-                                const double* scale_host, double nu, double tau, void* ws, int* indptr_dev, int64_t* nnz_host,
-                                const int* row_pos_dev, int64_t row_first, int64_t row_last, void* stream);
-int gp_matern_sparse_fill_rows(const double* points, const double* points_host, int64_t n, int64_t d, const double* scale_host,
-                               double nu, double tau, void* ws, const int* indptr_dev, int* indices_dev, double* data_dev,
-                               double* ddata_dev, int sort_rows, const int* row_pos_dev, int64_t row_first, int64_t row_last,
-                               void* stream);
+                          int* indices_dev, double* data_dev, double* ddata_dev, int sort_rows, const int* row_pos_dev,
+                          int64_t row_first, int64_t row_last, void* stream);
 /* Sorts every row of a CSR matrix by column (data / ddata follow); flags_dev: 2 device ints of scratch. */
 int gp_csr_sort_rows(int64_t n, const int* indptr_dev, int* indices_dev, double* data_dev, double* ddata_dev,
                      int* flags_dev, void* stream);
@@ -201,30 +196,37 @@ int gp_csr_spmm(const int* indptr, const int* indices, const double* data, int64
  * row = row_map[i] when row_map (device int32, n) is given (internally permuted operators), else i. */
 int gp_rademacher(double* V, int64_t n, int64_t B, uint64_t seed, int64_t probe_offset, const int* row_map,
                   void* stream);
-/* Row-blocked form of a (symmetrically permuted) CSR matrix: R = 8 or 16 consecutive rows share one list of block-columns
- * (R x 1 blocks, zero filled; the list is padded with zero blocks to a multiple of 4 = one DMMA.8x8x4 k-step). New row r = old row order[r], new column = inv_order[old column] (both
- * NULL: no permutation); the source rows must be sorted. With a spatially local order (gp_spatial_keys) neighbouring
- * rows have nearly the same pattern: one gathered row of X then serves R rows of K and the index is amortised.
- *   gp_bcsr_count: nblk[rb] = number of block-columns of row block rb (ceil(n/R) entries); the caller's exclusive
- *                  prefix sum gives bptr (int64, ceil(n/R)+1). needs_sorted_dev (device int, may be NULL) is set to 1
+/* Row-blocked form of a (symmetrically permuted) CSR matrix: 16 consecutive rows share one list of block-columns
+ * (16 x 1 blocks, zero filled; the list is padded with zero blocks to a multiple of 4 = one DMMA.8x8x4 k-step). New row r =
+ * old row order[r], new column = inv_order[old column] (both NULL: no permutation); the source rows must be sorted. With a
+ * spatially local order
+ * (gp_spatial_keys) neighbouring rows have nearly the same pattern: one gathered row of X then serves 16 rows of K and the
+ * index is amortised. n rows are built; order may point into a longer order (one slab: order + first row).
+ *   gp_bcsr_count: nblk[rb] = number of block-columns of row block rb (ceil(n/16) entries); the caller's exclusive
+ *                  prefix sum gives bptr (int64, ceil(n/16)+1). needs_sorted_dev (device int, may be NULL) is set to 1
  *                  when some row block exceeded the shared-memory hash table and used the binary-search path, which
  *                  requires SORTED source rows (the hash path does not).
- *   gp_bcsr_fill : nblocks = bptr[last]; bidx (int32, nblocks), bvals / bdvals (f64, R * nblocks): every group of four
+ *   gp_bcsr_fill : nblocks = bptr[last]; bidx (int32, nblocks), bvals / bdvals (f64, 16 * nblocks): every group of four
  *                  block-columns is stored in DMMA A-fragment order (one 8-row fragment after the other), value
- *                  (slot s, row k) at 4 R (s/4) + 32 (k/8) + 4 (k%8) + s%4. */
-int gp_bcsr_count(int64_t R, int64_t n, const int* order, const int* inv_order, const int* indptr, const int* indices,
-                  int* nblk, int* needs_sorted_dev, void* stream);
-int gp_bcsr_fill(int64_t R, int64_t n, const int* order, const int* inv_order, const int* indptr, const int* indices,
-                 const double* data, const double* ddata, const int64_t* bptr, int64_t nblocks, int* bidx, double* bvals,
-                 double* bdvals, void* stream);
-/* Y = (K + eta I) X on the row-blocked operator (FP64 tensor-core MMAs: 4 block-columns x 8 rows x 8 columns; with
- * R = 16 two MMAs share each gathered fragment of X). Tuned for B <= 16. */
-int gp_bcsr_spmm(int64_t R, const int64_t* bptr, const int* bidx, const double* bvals, int64_t n, double eta,
+ *                  (slot s, row k) at 64 (s/4) + 32 (k/8) + 4 (k%8) + s%4. */
+int gp_bcsr_count(int64_t n, const int* order, const int* inv_order, const int* indptr, const int* indices, int* nblk,
+                  int* needs_sorted_dev, void* stream);
+int gp_bcsr_fill(int64_t n, const int* order, const int* inv_order, const int* indptr, const int* indices, const double* data,
+                 const double* ddata, const int64_t* bptr, int64_t nblocks, int* bidx, double* bvals, double* bdvals,
+                 void* stream);
+/* The row-blocked drivers (gp_bcsr_spmm, gp_col_dot, gp_bcsr_lanczos, gp_bcsr_cg_solve) take `peer`: NULL on one GPU.
+ * Otherwise it is this rank's arena (gp_peer_create) of the row-slab operator: the row blocks are this rank's rows with
+ * encoded columns (gp_slab_encode_columns), n is the number of those rows, vectors are the rank's rows (n x B), and alpha,
+ * beta and dot products are summed over the ranks - identical on every rank.
+ * Y = (K + eta I) X on the row-blocked operator (FP64 tensor-core MMAs: 4 block-columns x 8 rows x 8 columns; two MMAs
+ * share each gathered fragment of X). Tuned for B <= 16. With a peer, X is copied into exchange vector 2 between two
+ * cross-GPU barriers. */
+int gp_bcsr_spmm(void* peer, const int64_t* bptr, const int* bidx, const double* bvals, int64_t n, double eta,
                  const double* X, int64_t B, double* Y, void* stream);
 /* workspace for gp_col_dot / gp_lanczos / gp_cg_solve */
 int64_t gp_krylov_workspace_bytes(int64_t n, int64_t B);
 /* out_dev[c] = sum_i X[i][c] Y[i][c] (deterministic two-stage reduction) */
-int gp_col_dot(const double* X, const double* Y, int64_t n, int64_t B, double* out_dev, void* ws, void* stream);
+int gp_col_dot(void* peer, const double* X, const double* Y, int64_t n, int64_t B, double* out_dev, void* ws, void* stream);
 /* m Lanczos steps per column started from V (normalised internally); alpha_dev, beta_dev: (m x B) device arrays of
  * the tridiagonal coefficients (beta[j] couples steps j and j+1). The quadrature itself is host-side.
  * basis_dev: NULL, or m x n x B doubles that receive the unnormalised Lanczos vectors u_j = beta_{j-1} q_j. */
@@ -240,14 +242,14 @@ int gp_cg_solve(const int* indptr, const int* indices, const double* data, int64
 int64_t gp_gram_workspace_bytes(int64_t B);
 int gp_gram_skinny(const double* X, const double* Y, int64_t n, int64_t B, double* out_dev, void* ws, void* stream);
 /* the same two Krylov drivers on the row-blocked operator */
-int gp_bcsr_lanczos(int64_t R, const int64_t* bptr, const int* bidx, const double* bvals, int64_t n, double eta,
+int gp_bcsr_lanczos(void* peer, const int64_t* bptr, const int* bidx, const double* bvals, int64_t n, double eta,
                     const double* V, int64_t B, int64_t m, double* alpha_dev, double* beta_dev, double* basis_dev, void* ws,
                     void* stream);
 /* X[i][c] = sum_j coef_dev[j][c] basis[j][i][c] (coef: m x B). With coef[j][c] = ||v_c|| y_jc / beta_{j-1,c} and
  * y = T^-1 e_1 this is the Lanczos solution of (K + eta I) x = v from the vectors kept by gp_*_lanczos: the Hutchinson
  * tr(Kn^-1 dK) estimator reuses the SLQ run instead of a second Krylov solve. */
 int gp_block_combine(const double* basis, int64_t n, int64_t B, int64_t m, const double* coef_dev, double* X, void* stream);
-int gp_bcsr_cg_solve(int64_t R, const int64_t* bptr, const int* bidx, const double* bvals, int64_t n, double eta,
+int gp_bcsr_cg_solve(void* peer, const int64_t* bptr, const int* bidx, const double* bvals, int64_t n, double eta,
                      double* R0, double* X, int64_t B, double tol, int64_t maxiter, int64_t* iters_host, void* ws,
                      void* stream);
 
@@ -289,18 +291,7 @@ int gp_peer_error(void* peer, void* stream);                              /* 1: 
  * gathered over NVLink per SpMM), [1] distinct remote rows among them (what a bulk halo exchange would move) */
 int gp_slab_encode_columns(int* bidx, int64_t total, int64_t slab, int64_t rank, int64_t n, int64_t* halo_host, void* ws,
                            void* stream);
-/* The drivers below take the 16-row blocks of this rank's rows (gp_bcsr_count / gp_bcsr_fill on order + first row) with
- * encoded columns; vectors are the rank's rows (nloc x B); alpha, beta, dots are identical on every rank. */
-int gp_slab_spmm(void* peer, const int64_t* bptr, const int* bidx, const double* bvals, int64_t nloc, double eta,
-                 const double* X, int64_t B, double* Y, void* stream);
-int gp_slab_col_dot(void* peer, const double* X, const double* Y, int64_t nloc, int64_t B, double* out_dev, void* ws,
-                    void* stream);
-int gp_slab_lanczos(void* peer, const int64_t* bptr, const int* bidx, const double* bvals, int64_t nloc, double eta,
-                    const double* V, int64_t B, int64_t m, double* alpha_dev, double* beta_dev, double* basis_dev, void* ws,
-                    void* stream);
-int gp_slab_cg_solve(void* peer, const int64_t* bptr, const int* bidx, const double* bvals, int64_t nloc, double eta,
-                     double* R0, double* X, int64_t B, double tol, int64_t maxiter, int64_t* iters_host, void* ws,
-                     void* stream);
+/* The row-blocked drivers take this rank's arena as `peer` (gp_bcsr_spmm, gp_col_dot, gp_bcsr_lanczos, gp_bcsr_cg_solve). */
 
 /* ---- index plumbing of the sparse operator build (csrc/gp_index.cu): own kernels instead of library sort / scan ------ */
 /* out_host[0..d) = column minima, out_host[d..2d) = column maxima of the device points; ws >= (148 * d * 2 + 2 * d) doubles;

@@ -126,6 +126,13 @@ def sparse_problem(gp):
     return pts, du.generate_data(pts, 0.2), du.generate_basis_functions(pts, 2), Kd
 
 
+def _plain_csr(Kd):
+    """the same matrix without a spatial order (its arrays shared): the engine keeps plain CSR in the original order"""
+    from gaussian_proc._sparse import DeviceCSR
+    return DeviceCSR(Kd.n, Kd.indptr, Kd.indices, Kd.data, Kd.ddata, kernel_threshold=Kd.kernel_threshold,
+                     sorted_rows=Kd.sorted_rows)
+
+
 def test_spmm_dot_solve(sparse_problem):
     from gaussian_proc._mixed_correlation import MixedCorrelation
     pts, z, X, Kd = sparse_problem
@@ -151,13 +158,13 @@ def test_slq_samples_equal_the_cpu_oracle_per_probe(sparse_problem):
     from gaussian_proc._sparse import SparseEngine
     from oracle import slq
     pts, z, X, Kd = sparse_problem
-    eng = SparseEngine(Kd, 'slq', {'seed': 11, 'lanczos_degree': 20, 'block_rows': 1})
+    eng = SparseEngine(_plain_csr(Kd), 'slq', {'seed': 11, 'lanczos_degree': 20})
     assert (eng.probes(4, 4).cpu().numpy() == slq.rademacher(eng.n, 4, 11, 4)).all()
     ref = slq.slq_samples(Kd.to_scipy(), 2.0, 11, 4, 4, 20)
-    for R in (1, 16):
-        e = SparseEngine(Kd, 'slq', {'seed': 11, 'lanczos_degree': 20, 'block_rows': R})
+    for K in (_plain_csr(Kd), Kd):
+        e = SparseEngine(K, 'slq', {'seed': 11, 'lanczos_degree': 20})
         got = e._slq_samples(2.0, 4, 4)
-        assert numpy.max(numpy.abs(got - ref) / numpy.abs(ref)) <= 1e-9, (R, got, ref)
+        assert numpy.max(numpy.abs(got - ref) / numpy.abs(ref)) <= 1e-9, (e.blocked is not None, got, ref)
 
 
 def test_probes_are_batching_invariant(sparse_problem):
@@ -398,10 +405,9 @@ def test_sparse_loglik_wide_basis(sparse_problem):
         assert abs(q.logdet_Kn - exact) <= 2e-2 * abs(exact)          # the estimator stops at a 1 % half width
 
 
-@pytest.mark.parametrize('R', [8, 16])
-def test_row_blocked_operator_equals_csr(gp, R):
-    """The row-blocked operator (8 x 1 or 16 x 1 blocks of the curve-ordered matrix, zero filled, DMMA SpMM) is the same linear map as the
-    canonical CSR: products against the SciPy matrix to rounding, for K and for dK/drho, n not a multiple of R."""
+def test_row_blocked_operator_equals_csr(gp):
+    """The row-blocked operator (16 x 1 blocks of the curve-ordered matrix, zero filled, DMMA SpMM) is the same linear map as
+    the canonical CSR: products against the SciPy matrix to rounding, for K and for dK/drho, n not a multiple of 16."""
     import torch
     from gaussian_proc._sparse import SparseEngine, generate_sparse_correlation
     numpy.random.seed(5)
@@ -410,7 +416,8 @@ def test_row_blocked_operator_equals_csr(gp, R):
     Kd = generate_sparse_correlation(pts, numpy.array([0.03, 0.03]), 1.5, 0.01, device=True, with_derivative=True)
     order = Kd.order.cpu().numpy()
     assert sorted(order.tolist()) == list(range(n))
-    eng = SparseEngine(Kd, 'slq', {'block_rows': R})
+    eng = SparseEngine(Kd, 'slq', {})
+    R = 16
     assert eng.R == R and eng.blocked is not None and 1.0 <= eng.fill_ratio <= R
     Ks = Kd.to_scipy()
     dKs = scipy.sparse.csr_matrix((Kd.ddata.cpu().numpy(), Ks.indices, Ks.indptr), shape=Ks.shape)
@@ -497,11 +504,9 @@ def test_internal_permutation_does_not_change_results(sparse_problem):
     from gaussian_proc._sparse import SparseEngine
     pts, z, X, Kd = sparse_problem
     opts = {'seed': 3, 'lanczos_degree': 25, 'min_num_samples': 16, 'max_num_samples': 16}
-    a = SparseEngine(Kd, 'slq', dict(opts, block_rows=16))
-    b = SparseEngine(Kd, 'slq', dict(opts, block_rows=1))
-    a2 = SparseEngine(Kd, 'slq', dict(opts, block_rows=16))
-    a8 = SparseEngine(Kd, 'slq', dict(opts, block_rows=8))
-    assert abs(a8.logdet(2.0) - b.logdet(2.0)) <= 1e-10 * abs(b.logdet(2.0))
+    a = SparseEngine(Kd, 'slq', dict(opts))
+    b = SparseEngine(_plain_csr(Kd), 'slq', dict(opts))
+    a2 = SparseEngine(Kd, 'slq', dict(opts))
     assert a.order is not None and b.order is None
     assert a.logdet(2.0) == a2.logdet(2.0)
     assert abs(a.logdet(2.0) - b.logdet(2.0)) <= 1e-10 * abs(b.logdet(2.0))

@@ -7,11 +7,10 @@ from gaussian_proc._sparse import generate_sparse_correlation, SparseEngine
 
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 2 ** 20
 B = int(sys.argv[2]) if len(sys.argv) > 2 else 16
-R = int(sys.argv[3]) if len(sys.argv) > 3 else 16
 numpy.random.seed(0)
 pts = numpy.random.rand(n, 2)
 K = generate_sparse_correlation(pts, numpy.array([0.005, 0.005]), 0.5, 1e-3, device=True)
-e = SparseEngine(K, 'slq', {'block_rows': R})
+e = SparseEngine(K, 'slq', {})
 V = e.probes(0, B)
 for _ in range(3):
     Y = e.spmm(1.0, V)
