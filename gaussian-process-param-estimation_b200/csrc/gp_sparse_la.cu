@@ -553,32 +553,40 @@ static SparseOp bcsr_op(const int64_t* bptr, const int* bidx, const double* bval
     return A;
 }
 
-// X = sum_j coef[j][c] U_j (elementwise per column): one pass over the m kept Lanczos vectors
+// X = sum_j coef[j][c] U_j (elementwise per column): one pass over the m kept Lanczos vectors. The coefficients are
+// staged in shared memory mc degrees at a time (mc = min(m, COMBINE_DEGREES)); the accumulators stay in registers across
+// the chunks, so the sum runs over j = 0 .. m - 1 in order whatever m is.
+constexpr int COMBINE_DEGREES = 256;    // 64 KB of coefficients at B = 32
 __global__ void __launch_bounds__(256)
-block_combine_kernel(const double* __restrict__ basis, int64_t total, int B, int m, const double* __restrict__ coef,
+block_combine_kernel(const double* __restrict__ basis, int64_t total, int B, int m, int mc, const double* __restrict__ coef,
                      double* __restrict__ X) {
-    extern __shared__ double cf[];      // m x B
-    for (int i = threadIdx.x; i < m * B; i += blockDim.x) cf[i] = coef[i];
-    __syncthreads();
+    extern __shared__ double cf[];      // mc x B: degrees [j0, j0 + mc)
     const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (B == 1) {
-        if (idx >= total) return;
-        double acc = 0.0;
-        for (int j = 0; j < m; ++j) acc += cf[j] * basis[(int64_t)j * total + idx];
-        X[idx] = acc;
-        return;
-    }
-    const int64_t e = idx * 2;          // two adjacent columns of one row (B is even)
-    if (e >= total) return;
+    const int64_t e = (B == 1) ? idx : idx * 2;     // B > 1: two adjacent columns of one row (B is even)
+    const bool live = e < total;
     const int c = (int)(e % B);
     double a0 = 0.0, a1 = 0.0;
+    for (int j0 = 0; j0 < m; j0 += mc) {
+        const int mj = min(mc, m - j0);
+        if (j0 > 0) __syncthreads();    // every thread is done with the previous chunk
+        for (int i = threadIdx.x; i < mj * B; i += blockDim.x) cf[i] = coef[(int64_t)j0 * B + i];
+        __syncthreads();
+        if (!live) continue;
+        const double* bj = basis + (int64_t)j0 * total + e;
+        if (B == 1) {
+            for (int j = 0; j < mj; ++j) a0 += cf[j] * bj[(int64_t)j * total];
+        } else {
 #pragma unroll 4
-    for (int j = 0; j < m; ++j) {
-        const double2 u = *reinterpret_cast<const double2*>(basis + (int64_t)j * total + e);
-        a0 += cf[j * B + c] * u.x;
-        a1 += cf[j * B + c + 1] * u.y;
+            for (int j = 0; j < mj; ++j) {
+                const double2 u = *reinterpret_cast<const double2*>(bj + (int64_t)j * total);
+                a0 += cf[j * B + c] * u.x;
+                a1 += cf[j * B + c + 1] * u.y;
+            }
+        }
     }
-    *reinterpret_cast<double2*>(X + e) = make_double2(a0, a1);
+    if (!live) return;
+    if (B == 1) X[e] = a0;
+    else *reinterpret_cast<double2*>(X + e) = make_double2(a0, a1);
 }
 
 // ---- skinny Gram matrix: out[a][b] = sum_i X[i][a] Y[i][b] for two n x B blocks (B <= 16) ----------------------
@@ -893,14 +901,15 @@ int gp_bcsr_lanczos(void* peer, const int64_t* bptr, const int* bidx, const doub
 
 // X[i][c] = sum_j coef[j][c] basis[j][i][c]: the Lanczos solution ||v|| Q T^-1 e_1 from the kept vectors
 int gp_block_combine(const double* basis, int64_t n, int64_t B, int64_t m, const double* coef_dev, double* X, void* stream) {
-    if (!basis || !coef_dev || !X || n <= 0 || B <= 0 || B > 32 || m <= 0 || m > 256) return -1;
+    if (!basis || !coef_dev || !X || n <= 0 || B <= 0 || B > 32 || (32 % B) || m <= 0 || m > INT32_MAX) return -1;
     const int64_t total = n * B;
     const int64_t work = (B == 1) ? total : total / 2;
-    // m B coefficients in dynamic shared memory: up to 64 KB (m = 256, B = 32), above the 48 KB default
-    if (m * B * (int64_t)sizeof(double) > 48 * 1024)
+    const int64_t mc = m < COMBINE_DEGREES ? m : COMBINE_DEGREES;
+    // mc B coefficients in dynamic shared memory: up to 64 KB (mc = 256, B = 32), above the 48 KB default
+    if (mc * B * (int64_t)sizeof(double) > 48 * 1024)
         if (int rc = configure_once((const void*)block_combine_kernel, 64 * 1024)) return rc;
-    block_combine_kernel<<<(unsigned)((work + 255) / 256), 256, (size_t)(m * B * sizeof(double)), (cudaStream_t)stream>>>(
-        basis, total, (int)B, (int)m, coef_dev, X);
+    block_combine_kernel<<<(unsigned)((work + 255) / 256), 256, (size_t)(mc * B * sizeof(double)), (cudaStream_t)stream>>>(
+        basis, total, (int)B, (int)m, (int)mc, coef_dev, X);
     GP_COUNT(1);
     GP_LAUNCH_CHECK();
     return 0;

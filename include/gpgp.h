@@ -247,7 +247,8 @@ int gp_bcsr_lanczos(void* peer, const int64_t* bptr, const int* bidx, const doub
                     void* stream);
 /* X[i][c] = sum_j coef_dev[j][c] basis[j][i][c] (coef: m x B). With coef[j][c] = ||v_c|| y_jc / beta_{j-1,c} and
  * y = T^-1 e_1 this is the Lanczos solution of (K + eta I) x = v from the vectors kept by gp_*_lanczos: the Hutchinson
- * tr(Kn^-1 dK) estimator reuses the SLQ run instead of a second Krylov solve. */
+ * tr(Kn^-1 dK) estimator reuses the SLQ run instead of a second Krylov solve. B in {1,2,4,8,16,32} and any degree
+ * m >= 1 (the sum runs over j = 0 .. m - 1 in order); -1 otherwise. */
 int gp_block_combine(const double* basis, int64_t n, int64_t B, int64_t m, const double* coef_dev, double* X, void* stream);
 int gp_bcsr_cg_solve(void* peer, const int64_t* bptr, const int* bidx, const double* bvals, int64_t n, double eta,
                      double* R0, double* X, int64_t B, double tol, int64_t maxiter, int64_t* iters_host, void* ws,
