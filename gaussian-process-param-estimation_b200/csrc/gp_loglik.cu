@@ -486,25 +486,11 @@ int gp_dk_apply(const double* points, int64_t n, int64_t d, const double* scale_
                 int64_t lds, double* V, void* stream) {
     if (!points || !scale_host || !S || !V || n <= 0 || d <= 0 || d > LMAXD || p <= 0 || p > MAXP || lds < p) return -1;
     MaternParams mp;
-    mp.nu = nu; mp.coef = 0.0; mp.sq2nu = 0.0;
-    for (int k = 0; k < d; ++k) {
-        if (!(scale_host[k] > 0.0) || scale_host[k] != scale_host[0]) return -4;
-        mp.inv_scale[k] = 1.0 / scale_host[k];
-    }
-    mp.inv_rho = 1.0 / scale_host[0];
-    int mode = matern_mode_of(nu);
-    if (mode == MAT_GENERAL) {
-        mp.coef = pow(2.0, 1.0 - nu) / tgamma(nu);
-        mp.sq2nu = sqrt(2.0 * nu);
-    }
-    cudaStream_t s = (cudaStream_t)stream;
-    switch (mode) {
-        case MAT_05: launch_dk_apply<MAT_05>(points, (int)n, (int)d, mp, S, (int)p, lds, V, s); break;
-        case MAT_15: launch_dk_apply<MAT_15>(points, (int)n, (int)d, mp, S, (int)p, lds, V, s); break;
-        case MAT_25: launch_dk_apply<MAT_25>(points, (int)n, (int)d, mp, S, (int)p, lds, V, s); break;
-        case MAT_GAUSS: launch_dk_apply<MAT_GAUSS>(points, (int)n, (int)d, mp, S, (int)p, lds, V, s); break;
-        default: launch_dk_apply<MAT_GENERAL>(points, (int)n, (int)d, mp, S, (int)p, lds, V, s); break;
-    }
+    int mode;
+    if (int rc = matern_params(scale_host, d, nu, true, &mp, &mode)) return rc;
+    with_matern_mode(mode, [&](auto tag) {
+        launch_dk_apply<decltype(tag)::value>(points, (int)n, (int)d, mp, S, (int)p, lds, V, (cudaStream_t)stream);
+    });
     GP_COUNT(1);
     GP_LAUNCH_CHECK();
     return 0;
@@ -551,28 +537,17 @@ int gp_loglik_dense_dscale(const double* Ainv, int64_t n, int64_t npad, int64_t 
     if (!Ainv || !points || !scale_host || !ws || !out_dim || n <= 0 || npad != gp_padded_size(n) || p <= 0 || p > MAXP ||
         d <= 0 || d > LMAXD || dim < 0 || dim >= d)
         return -1;
+    MaternParams mp;
+    int mode;
+    if (int rc = matern_params(scale_host, d, nu, false, &mp, &mode)) return rc;
+    mp.inv_rho = 1.0;
+    mp.ddim = (int)dim;
     cudaStream_t s = (cudaStream_t)stream;
     LoglikWs w = carve(ws, npad, (int)p);
-    MaternParams mp;
-    mp.nu = nu; mp.coef = 0.0; mp.sq2nu = 0.0; mp.inv_rho = 1.0; mp.ddim = (int)dim;
-    for (int k = 0; k < d; ++k) {
-        if (!(scale_host[k] > 0.0)) return -4;
-        mp.inv_scale[k] = 1.0 / scale_host[k];
-    }
-    int mode = matern_mode_of(nu);
-    if (mode == MAT_GENERAL) {
-        mp.coef = pow(2.0, 1.0 - nu) / tgamma(nu);
-        mp.sq2nu = sqrt(2.0 * nu);
-    }
-    const int N = (int)n, NP = (int)npad, P = (int)p;
-    int rc;
-    switch (mode) {
-        case MAT_05: rc = grad_reductions<MAT_05>(Ainv, N, NP, points, (int)d, mp, true, w, P, out_dim + 1, s); break;
-        case MAT_15: rc = grad_reductions<MAT_15>(Ainv, N, NP, points, (int)d, mp, true, w, P, out_dim + 1, s); break;
-        case MAT_25: rc = grad_reductions<MAT_25>(Ainv, N, NP, points, (int)d, mp, true, w, P, out_dim + 1, s); break;
-        case MAT_GAUSS: rc = grad_reductions<MAT_GAUSS>(Ainv, N, NP, points, (int)d, mp, true, w, P, out_dim + 1, s); break;
-        default: rc = grad_reductions<MAT_GENERAL>(Ainv, N, NP, points, (int)d, mp, true, w, P, out_dim + 1, s); break;
-    }
+    const int NP = (int)npad;
+    int rc = with_matern_mode(mode, [&](auto tag) {
+        return grad_reductions<decltype(tag)::value>(Ainv, (int)n, NP, points, (int)d, mp, true, w, (int)p, out_dim + 1, s);
+    });
     if (rc) return rc;
     int T = NP / 128;
     sum_trace3_kernel<<<1, 256, 0, s>>>(w.tr, T * (T + 1) / 2, out_dim);
@@ -590,8 +565,13 @@ int gp_loglik_dense(const double* K, int64_t n, int64_t npad, const double* R, i
                     void* potrf_ws, void* ws, double* out, void* stream) {
     if (!K || !R || !A || !potrf_ws || !ws || !out || n <= 0 || npad != gp_padded_size(n) || p <= 0 || p > MAXP) return -1;
     if ((flags & 3) && !W) return -2;
-    if ((flags & 4) && (!(flags & 2) || !points || !scale_host || d <= 0 || d > LMAXD)) return -3;
-    if ((flags & 8) && !(flags & 3)) return -5;
+    if ((flags & 4) && (!(flags & 2) || !points || !scale_host || d <= 0 || d > LMAXD)) return -8;
+    if ((flags & 8) && !(flags & 3)) return -9;
+    const bool with_dk = (flags & 4) != 0;
+    MaternParams mp{};     // without flag 4 the reductions do not read it
+    int mode = MAT_05;
+    if (with_dk)
+        if (int rc = matern_params(scale_host, d, nu, true, &mp, &mode)) return rc;
     cudaStream_t s = (cudaStream_t)stream;
     LoglikWs w = carve(ws, npad, (int)p);
     const int N = (int)n, NP = (int)npad, P = (int)p;
@@ -624,29 +604,9 @@ int gp_loglik_dense(const double* K, int64_t n, int64_t npad, const double* R, i
     }
     if (flags & 2) {
         if ((rc = gp_lauum_f64(W, A, npad, stream))) return rc;
-        bool with_dk = (flags & 4) != 0;
-        MaternParams mp;
-        mp.nu = nu; mp.coef = 0.0; mp.sq2nu = 0.0; mp.inv_rho = 0.0;
-        int mode = MAT_05;
-        if (with_dk) {
-            for (int k = 0; k < d; ++k) {
-                if (!(scale_host[k] > 0.0) || scale_host[k] != scale_host[0]) return -4;
-                mp.inv_scale[k] = 1.0 / scale_host[k];
-            }
-            mp.inv_rho = 1.0 / scale_host[0];
-            mode = matern_mode_of(nu);
-            if (mode == MAT_GENERAL) {
-                mp.coef = pow(2.0, 1.0 - nu) / tgamma(nu);
-                mp.sq2nu = sqrt(2.0 * nu);
-            }
-        }
-        switch (mode) {
-            case MAT_05: rc = grad_reductions<MAT_05>(A, N, NP, points, (int)d, mp, with_dk, w, P, Q, s); break;
-            case MAT_15: rc = grad_reductions<MAT_15>(A, N, NP, points, (int)d, mp, with_dk, w, P, Q, s); break;
-            case MAT_25: rc = grad_reductions<MAT_25>(A, N, NP, points, (int)d, mp, with_dk, w, P, Q, s); break;
-            case MAT_GAUSS: rc = grad_reductions<MAT_GAUSS>(A, N, NP, points, (int)d, mp, with_dk, w, P, Q, s); break;
-            default: rc = grad_reductions<MAT_GENERAL>(A, N, NP, points, (int)d, mp, with_dk, w, P, Q, s); break;
-        }
+        rc = with_matern_mode(mode, [&](auto tag) {
+            return grad_reductions<decltype(tag)::value>(A, N, NP, points, (int)d, mp, with_dk, w, P, Q, s);
+        });
         if (rc) return rc;
     } else if (flags & 1) {
         frob_lower_kernel<<<dim3(T, T), 256, 0, s>>>(W, N, NP, w.frob);

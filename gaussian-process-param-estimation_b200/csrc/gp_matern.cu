@@ -260,30 +260,12 @@ extern "C" int gp_matern_dense(const double* points, int64_t n, int64_t d, const
     if (n <= 0 || d <= 0 || d > MAXD || !points || !K || !scale_host) return -1;
     int64_t npad = gp_padded_size(n);
     if (ldk != npad || npad > INT32_MAX) return -2;
-    cudaStream_t s = (cudaStream_t)stream;
     MaternParams mp;
-    for (int k = 0; k < d; ++k) {
-        if (!(scale_host[k] > 0.0)) return -3;
-        if (dK && scale_host[k] != scale_host[0]) return -4;  // d/drho is defined for an isotropic scale only
-        mp.inv_scale[k] = 1.0 / scale_host[k];
-    }
-    mp.nu = nu;
-    mp.coef = 0.0;
-    mp.sq2nu = 0.0;
-    mp.inv_rho = 1.0 / scale_host[0];
-    int mode = matern_mode_of(nu);
-    if (mode == MAT_GENERAL) {
-        if (!(nu > 0.0)) return -5;
-        mp.coef = pow(2.0, 1.0 - nu) / tgamma(nu);
-        mp.sq2nu = sqrt(2.0 * nu);
-    }
-    switch (mode) {
-        case MAT_05: return launch_mode<MAT_05>(points, (int)n, (int)d, (int)npad, K, dK, mp, s);
-        case MAT_15: return launch_mode<MAT_15>(points, (int)n, (int)d, (int)npad, K, dK, mp, s);
-        case MAT_25: return launch_mode<MAT_25>(points, (int)n, (int)d, (int)npad, K, dK, mp, s);
-        case MAT_GAUSS: return launch_mode<MAT_GAUSS>(points, (int)n, (int)d, (int)npad, K, dK, mp, s);
-        default: return launch_mode<MAT_GENERAL>(points, (int)n, (int)d, (int)npad, K, dK, mp, s);
-    }
+    int mode;
+    if (int rc = matern_params(scale_host, d, nu, dK != nullptr, &mp, &mode)) return rc;
+    return with_matern_mode(mode, [&](auto tag) {
+        return launch_mode<decltype(tag)::value>(points, (int)n, (int)d, (int)npad, K, dK, mp, (cudaStream_t)stream);
+    });
 }
 
 // out[r][c] = K(p_row[r], p_col[c]) (+ eta on the global diagonal) for nr x nc blocks of a larger padded matrix;
@@ -296,26 +278,12 @@ static int matern_cross_impl(const double* prow, const double* pcol, const int* 
         d > MAXD || (ld & 1))
         return -1;
     MaternParams mp;
-    for (int k = 0; k < d; ++k) {
-        if (!(scale_host[k] > 0.0)) return -3;
-        if (dk && scale_host[k] != scale_host[0]) return -4;
-        mp.inv_scale[k] = 1.0 / scale_host[k];
-    }
-    mp.nu = nu; mp.coef = 0.0; mp.sq2nu = 0.0; mp.inv_rho = 1.0 / scale_host[0];
-    int mode = matern_mode_of(nu);
-    if (mode == MAT_GENERAL) {
-        if (!(nu > 0.0)) return -5;
-        mp.coef = pow(2.0, 1.0 - nu) / tgamma(nu);
-        mp.sq2nu = sqrt(2.0 * nu);
-    }
-    cudaStream_t s = (cudaStream_t)stream;
-    switch (mode) {
-        case MAT_05: return launch_cross<MAT_05>(prow, pcol, row_gidx, col_gidx, (int)nr, (int)nc, (int)n, (int)d, ld, out, eta, mp, s, dk);
-        case MAT_15: return launch_cross<MAT_15>(prow, pcol, row_gidx, col_gidx, (int)nr, (int)nc, (int)n, (int)d, ld, out, eta, mp, s, dk);
-        case MAT_25: return launch_cross<MAT_25>(prow, pcol, row_gidx, col_gidx, (int)nr, (int)nc, (int)n, (int)d, ld, out, eta, mp, s, dk);
-        case MAT_GAUSS: return launch_cross<MAT_GAUSS>(prow, pcol, row_gidx, col_gidx, (int)nr, (int)nc, (int)n, (int)d, ld, out, eta, mp, s, dk);
-        default: return launch_cross<MAT_GENERAL>(prow, pcol, row_gidx, col_gidx, (int)nr, (int)nc, (int)n, (int)d, ld, out, eta, mp, s, dk);
-    }
+    int mode;
+    if (int rc = matern_params(scale_host, d, nu, dk, &mp, &mode)) return rc;
+    return with_matern_mode(mode, [&](auto tag) {
+        return launch_cross<decltype(tag)::value>(prow, pcol, row_gidx, col_gidx, (int)nr, (int)nc, (int)n, (int)d, ld, out,
+                                                  eta, mp, (cudaStream_t)stream, dk);
+    });
 }
 
 extern "C" int gp_matern_cross(const double* prow, const double* pcol, const int* row_gidx, const int* col_gidx, int64_t nr,
@@ -338,23 +306,9 @@ extern "C" int gp_matern_cross_points(const double* p, int64_t n, const double* 
     int64_t npad = gp_padded_size(n), mpad = gp_padded_size(m);
     if (ldp < mpad || (ldp & 1) || ((uintptr_t)P & 15) || npad > INT32_MAX || mpad > INT32_MAX) return -2;
     MaternParams mp;
-    for (int k = 0; k < d; ++k) {
-        if (!(scale_host[k] > 0.0)) return -3;
-        mp.inv_scale[k] = 1.0 / scale_host[k];
-    }
-    mp.nu = nu; mp.coef = 0.0; mp.sq2nu = 0.0; mp.inv_rho = 1.0 / scale_host[0];
-    int mode = matern_mode_of(nu);
-    if (mode == MAT_GENERAL) {
-        if (!(nu > 0.0)) return -5;
-        mp.coef = pow(2.0, 1.0 - nu) / tgamma(nu);
-        mp.sq2nu = sqrt(2.0 * nu);
-    }
-    cudaStream_t s = (cudaStream_t)stream;
-    switch (mode) {
-        case MAT_05: return launch_cross_points<MAT_05>(p, (int)n, q, (int)m, (int)d, ldp, P, mp, s);
-        case MAT_15: return launch_cross_points<MAT_15>(p, (int)n, q, (int)m, (int)d, ldp, P, mp, s);
-        case MAT_25: return launch_cross_points<MAT_25>(p, (int)n, q, (int)m, (int)d, ldp, P, mp, s);
-        case MAT_GAUSS: return launch_cross_points<MAT_GAUSS>(p, (int)n, q, (int)m, (int)d, ldp, P, mp, s);
-        default: return launch_cross_points<MAT_GENERAL>(p, (int)n, q, (int)m, (int)d, ldp, P, mp, s);
-    }
+    int mode;
+    if (int rc = matern_params(scale_host, d, nu, false, &mp, &mode)) return rc;
+    return with_matern_mode(mode, [&](auto tag) {
+        return launch_cross_points<decltype(tag)::value>(p, (int)n, q, (int)m, (int)d, ldp, P, mp, (cudaStream_t)stream);
+    });
 }

@@ -2,6 +2,8 @@
 // on-the-fly dK/drho reductions. Follows gaussian_proc/generate_correlation/_kernels.pyx:17-100 branch by branch.
 #pragma once
 #include <math.h>
+#include <stdint.h>
+#include <type_traits>
 
 namespace gp {
 
@@ -19,8 +21,9 @@ static inline int matern_mode_of(double nu) {
 #ifdef __CUDACC__
 // Modified Bessel K_nu(x) and K_{nu+1}(x) for real nu >= 0, x > 0: Temme's series for x <= 2, Steed's
 // continued fraction CF2 for x > 2, then upward recurrence from the fractional order mu in [-1/2, 1/2].
-// (Published algorithm: Temme 1975; Numerical Recipes `bessik`.) Used only for the general-nu Matern branch.
-__device__ inline void bessel_k_pair(double nu, double x, double* knu, double* knu1) {
+// (Published algorithm: Temme 1975; Numerical Recipes `bessik`.) Used only for the general-nu Matern branch, on the device
+// and by the host evaluation that decides the sparse generator's borderline pairs and support radius (gp_sparse.cu).
+__host__ __device__ inline void bessel_k_pair(double nu, double x, double* knu, double* knu1) {
     const double EPS = 1e-16;
     const int MAXIT = 100000;
     int nl = (int)(nu + 0.5);
@@ -102,6 +105,48 @@ struct MaternParams {
     double inv_scale[8]; // 1 / correlation_scale[k]
     int ddim = -1;       // >= 0: derivative with respect to correlation_scale[ddim] alone (anisotropic gradient; inv_rho = 1)
 };
+
+// The parameter checks of every entry point that takes scale_host and nu, made before anything is enqueued: -3 when a scale
+// entry is not > 0 (NaN included), -4 when `isotropic` (a d/drho is requested) and the d entries are not all equal, -5 when
+// nu selects the general branch and is not > 0. NaN nu takes the Gaussian branch, as in the reference. gp_kernel_threshold,
+// host-only and defined for any d, uses these checks alone; every other entry point calls matern_params.
+static inline int matern_check(const double* scale_host, int64_t d, double nu, bool isotropic) {
+    for (int64_t k = 0; k < d; ++k)
+        if (!(scale_host[k] > 0.0)) return -3;
+    if (isotropic)
+        for (int64_t k = 1; k < d; ++k)
+            if (scale_host[k] != scale_host[0]) return -4;
+    if (matern_mode_of(nu) == MAT_GENERAL && !(nu > 0.0)) return -5;
+    return 0;
+}
+
+// matern_check, then the kernel parameters (d <= 8) and the branch: mode is the template argument of the kernels, passed
+// through with_matern_mode. ddim stays -1.
+static inline int matern_params(const double* scale_host, int64_t d, double nu, bool isotropic, MaternParams* mp, int* mode) {
+    if (int rc = matern_check(scale_host, d, nu, isotropic)) return rc;
+    *mp = MaternParams();
+    *mode = matern_mode_of(nu);
+    mp->nu = nu;
+    if (*mode == MAT_GENERAL) {
+        mp->coef = pow(2.0, 1.0 - nu) / tgamma(nu);
+        mp->sq2nu = sqrt(2.0 * nu);
+    }
+    mp->inv_rho = 1.0 / scale_host[0];
+    for (int64_t k = 0; k < d; ++k) mp->inv_scale[k] = 1.0 / scale_host[k];
+    return 0;
+}
+
+// f(std::integral_constant<int, MODE>()) for the run-time branch `mode`: instantiates f for each of the five branches.
+template <class F>
+decltype(auto) with_matern_mode(int mode, F&& f) {
+    switch (mode) {
+        case MAT_05: return f(std::integral_constant<int, MAT_05>());
+        case MAT_15: return f(std::integral_constant<int, MAT_15>());
+        case MAT_25: return f(std::integral_constant<int, MAT_25>());
+        case MAT_GAUSS: return f(std::integral_constant<int, MAT_GAUSS>());
+        default: return f(std::integral_constant<int, MAT_GENERAL>());
+    }
+}
 
 // correlation value only; x is the scaled distance (>= 0). x == 0 -> exactly 1 (_kernels.pyx:73-74).
 template <int MODE>

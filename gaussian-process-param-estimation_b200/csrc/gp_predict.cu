@@ -220,27 +220,13 @@ int gp_predict_grad_dense(const double* points, int64_t n, const double* q, int6
         return -1;
     if (gp_padded_size(n) > INT32_MAX || gp_padded_size(mc) > INT32_MAX || (U && ldu < mc)) return -2;
     MaternParams mp;
-    for (int k = 0; k < d; ++k) {
-        if (!(scale_host[k] > 0.0)) return -3;
-        mp.inv_scale[k] = 1.0 / scale_host[k];
-    }
-    mp.nu = nu; mp.coef = 0.0; mp.sq2nu = 0.0; mp.inv_rho = 1.0 / scale_host[0];
-    const int mode = matern_mode_of(nu);
-    if (mode == MAT_GENERAL) {
-        if (!(nu > 0.0)) return -5;
-        mp.coef = pow(2.0, 1.0 - nu) / tgamma(nu);
-        mp.sq2nu = sqrt(2.0 * nu);
-    }
+    int mode;
+    if (int rc = matern_params(scale_host, d, nu, false, &mp, &mode)) return rc;
     cudaStream_t s = (cudaStream_t)stream;
     double* partial = (double*)ws;
-    const int N = (int)n, M = (int)mc, D = (int)d, PN = (int)p;
-    switch (mode) {
-        case MAT_05: launch_grad_partial<MAT_05>(points, N, q, M, D, mp, S, PN, U, ldu, partial, s); break;
-        case MAT_15: launch_grad_partial<MAT_15>(points, N, q, M, D, mp, S, PN, U, ldu, partial, s); break;
-        case MAT_25: launch_grad_partial<MAT_25>(points, N, q, M, D, mp, S, PN, U, ldu, partial, s); break;
-        case MAT_GAUSS: launch_grad_partial<MAT_GAUSS>(points, N, q, M, D, mp, S, PN, U, ldu, partial, s); break;
-        default: launch_grad_partial<MAT_GENERAL>(points, N, q, M, D, mp, S, PN, U, ldu, partial, s); break;
-    }
+    with_matern_mode(mode, [&](auto tag) {
+        launch_grad_partial<decltype(tag)::value>(points, (int)n, q, (int)mc, (int)d, mp, S, (int)p, U, ldu, partial, s);
+    });
     const int nchunks = (int)((n + PRED_ROWS - 1) / PRED_ROWS);
     const int64_t width = mc * d * (p + 1);
     predict_reduce_kernel<<<(unsigned)((width + 255) / 256), 256, 0, s>>>(partial, nchunks, width, width, out);

@@ -42,8 +42,6 @@ static double gamma_half_int(int dimension) {  // Gamma(d/2 + 1), _generate_spar
     return g;
 }
 
-static void bessel_k_pair_host(double nu, double x, double* knu, double* knu1);
-
 static double matern_host(double x, double nu) {  // _kernels.pyx:17-100, glibc exp/sqrt/pow
     if (x == 0) return 1.0;
     if (nu == 0.5) return exp(-x);
@@ -51,7 +49,7 @@ static double matern_host(double x, double nu) {  // _kernels.pyx:17-100, glibc 
     if (nu == 2.5) return (1.0 + sqrt(5.0) * x + (5.0 / 3.0) * pow(x, 2.0)) * exp(-sqrt(5.0) * x);
     if (nu < 100) {
         double y = sqrt(2.0 * nu) * x, k, k1;
-        bessel_k_pair_host(nu, y, &k, &k1);
+        bessel_k_pair(nu, y, &k, &k1);
         return (pow(2.0, 1.0 - nu) / tgamma(nu)) * pow(y, nu) * k;
     }
     return exp(-0.5 * pow(x, 2.0));
@@ -61,47 +59,6 @@ static double distance_host(const double* a, const double* b, const double* scal
     double s = 0;
     for (int k = 0; k < d; ++k) s += pow((a[k] - b[k]) / scale[k], 2.0);
     return sqrt(s);
-}
-
-// Temme / Steed evaluation of K_nu, K_{nu+1} (same algorithm as the device version in gp_matern.cuh)
-static void bessel_k_pair_host(double nu, double x, double* knu, double* knu1) {
-    const double EPS = 1e-16;
-    int nl = (int)(nu + 0.5);
-    double xmu = nu - nl, xmu2 = xmu * xmu, xi = 1.0 / x, xi2 = 2.0 * xi, rkmu, rk1;
-    if (x < 2.0) {
-        double b = 0.5 * x, d = -log(b), e = xmu * d;
-        double fact2 = (fabs(e) < EPS) ? 1.0 : sinh(e) / e;
-        double pimu = M_PI * xmu;
-        double fact = (fabs(pimu) < EPS) ? 1.0 : pimu / sin(pimu);
-        double gampl = 1.0 / tgamma(1.0 + xmu), gammi = 1.0 / tgamma(1.0 - xmu);
-        double gam2 = 0.5 * (gammi + gampl);
-        double gam1 = (fabs(xmu) < 1e-4) ? -0.5772156649015329 + xmu2 * 0.04200263503409524 : (gammi - gampl) / (2.0 * xmu);
-        double ff = fact * (gam1 * cosh(e) + gam2 * fact2 * d), sum = ff;
-        e = exp(e);
-        double p = 0.5 * e / gampl, q = 0.5 / (e * gammi), c = 1.0, d2 = b * b, sum1 = p;
-        for (int i = 1; i <= 100000; ++i) {
-            ff = (i * ff + p + q) / (i * i - xmu2);
-            c *= (d2 / i); p /= (i - xmu); q /= (i + xmu);
-            double del = c * ff; sum += del; sum1 += c * (p - i * ff);
-            if (fabs(del) < fabs(sum) * EPS) break;
-        }
-        rkmu = sum; rk1 = sum1 * xi2;
-    } else {
-        double b = 2.0 * (1.0 + x), d = 1.0 / b, h = d, delh = d, q1 = 0.0, q2 = 1.0, a1 = 0.25 - xmu2;
-        double q = a1, c = a1, a = -a1, s = 1.0 + q * delh;
-        for (int i = 2; i <= 100000; ++i) {
-            a -= 2 * (i - 1); c = -a * c / i;
-            double qnew = (q1 - b * q2) / a; q1 = q2; q2 = qnew; q += c * qnew;
-            b += 2.0; d = 1.0 / (b + a * d); delh = (b * d - 1.0) * delh; h += delh;
-            double dels = q * delh; s += dels;
-            if (fabs(dels / s) < EPS) break;
-        }
-        h = a1 * h;
-        rkmu = sqrt(M_PI / (2.0 * x)) * exp(-x) / s;
-        rk1 = rkmu * (xmu + x + 0.5 - h) * xi;
-    }
-    for (int i = 1; i <= nl; ++i) { double t = (xmu + i) * xi2 * rk1 + rkmu; rkmu = rk1; rk1 = t; }
-    *knu = rkmu; *knu1 = rk1;
 }
 
 // scaled taper radius x_tau: K(x) > tau only if x < x_tau (K is decreasing); bisection, returned with a safety margin
@@ -486,8 +443,8 @@ static SparseWs carve_sparse(void* ws, int64_t n, int64_t d) {
     return w;
 }
 
-static int make_params(int64_t n, int64_t d, const double* scale_host, double nu, double tau, const double* bbox_lo,
-                       const double* bbox_hi, SparseParams* sp, CellGrid* g) {
+static int make_params(int64_t n, int64_t d, const double* scale_host, double nu, double tau, const MaternParams& mp,
+                       const double* bbox_lo, const double* bbox_hi, SparseParams* sp, CellGrid* g) {
     sp->tau = tau;
     sp->band = 8.0 * 2.220446049250313e-16 * fabs(tau);
     sp->d = (int)d;
@@ -495,14 +452,7 @@ static int make_params(int64_t n, int64_t d, const double* scale_host, double nu
     sp->row_pos = nullptr;
     sp->row_first = sp->row_last = 0;
     for (int k = 0; k < d; ++k) sp->scale[k] = scale_host[k];
-    sp->mp.nu = nu;
-    sp->mp.coef = 0.0; sp->mp.sq2nu = 0.0;
-    sp->mp.inv_rho = 1.0 / scale_host[0];
-    for (int k = 0; k < d; ++k) sp->mp.inv_scale[k] = 1.0 / scale_host[k];
-    if (matern_mode_of(nu) == MAT_GENERAL) {
-        sp->mp.coef = pow(2.0, 1.0 - nu) / tgamma(nu);
-        sp->mp.sq2nu = sqrt(2.0 * nu);
-    }
+    sp->mp = mp;
     double xr = support_radius(tau, nu);
     sp->quick = (tau > 0.0 && tau < 1.0 && xr > 0.0 && xr < 1e100) ? 1 : 0;
     sp->r2_lo = xr * xr * (1.0 - 4e-7);
@@ -554,17 +504,6 @@ static void launch_rows(int pass, bool with_dk, const SparseParams& sp, const Ce
     GP_COUNT(1);
 }
 
-static void launch_rows_mode(int mode, int pass, bool with_dk, const SparseParams& sp, const CellGrid& g, const SparseWs& w,
-                             const int* indptr, int* indices, double* data, double* ddata, cudaStream_t s) {
-    switch (mode) {
-        case MAT_05: launch_rows<MAT_05>(pass, with_dk, sp, g, w, indptr, indices, data, ddata, s); break;
-        case MAT_15: launch_rows<MAT_15>(pass, with_dk, sp, g, w, indptr, indices, data, ddata, s); break;
-        case MAT_25: launch_rows<MAT_25>(pass, with_dk, sp, g, w, indptr, indices, data, ddata, s); break;
-        case MAT_GAUSS: launch_rows<MAT_GAUSS>(pass, with_dk, sp, g, w, indptr, indices, data, ddata, s); break;
-        default: launch_rows<MAT_GENERAL>(pass, with_dk, sp, g, w, indptr, indices, data, ddata, s); break;
-    }
-}
-
 struct MortonParams {
     double lo[3], mul[3];
     int nd, d, bits;
@@ -611,6 +550,7 @@ extern "C" {
 int gp_kernel_threshold(int64_t n, int64_t d, double density, const double* scale_host, double nu, double* tau_host) {
     // _estimate_kernel_threshold, _generate_sparse_correlation.pyx:294-413 (with _ball_volume given its dimension)
     if (!scale_host || !tau_host || n <= 0 || d <= 0) return -1;
+    if (int rc = matern_check(scale_host, d, nu, false)) return rc;
     double adjacency_volume = density * (double)n;
     if (adjacency_volume < 1.0) return -10;  // -> ValueError in the Python layer (:378-383)
     double prod = 1.0;
@@ -633,7 +573,7 @@ int64_t gp_sparse_workspace_bytes(int64_t n, int64_t d) { return (int64_t)carve_
 // Bounding box, cell grid (cell edge >= support radius), cell-sorted point list: everything the row / row-block kernels
 // enumerate candidates from. Leaves the bounding box in w.bbox for the fill call.
 static int sparse_prepare(const double* points, int64_t n, int64_t d, const double* scale_host, double nu, double tau,
-                          const SparseWs& w, cudaStream_t s, SparseParams* sp_out, CellGrid* g_out) {
+                          const MaternParams& mp, const SparseWs& w, cudaStream_t s, SparseParams* sp_out, CellGrid* g_out) {
     const int N = (int)n, D = (int)d;
     double lo[8], hi[8], bb[16];
     {
@@ -654,7 +594,7 @@ static int sparse_prepare(const double* points, int64_t n, int64_t d, const doub
     }
     SparseParams& sp = *sp_out;
     CellGrid& g = *g_out;
-    make_params(n, d, scale_host, nu, tau, lo, hi, &sp, &g);
+    make_params(n, d, scale_host, nu, tau, mp, lo, hi, &sp, &g);
     GP_CUDA_CHECK(cudaMemsetAsync(w.cell_start, 0, sizeof(int) * (g.ncells + 1), s));
     GP_CUDA_CHECK(cudaMemsetAsync(w.border_cnt, 0, sizeof(int) * 4, s));
     GP_CUDA_CHECK(cudaMemsetAsync(w.overflow, 0, sizeof(int) * 4, s));
@@ -687,16 +627,21 @@ int gp_matern_sparse_count(const double* points, const double* points_host, int6
     if (!points || !points_host || !scale_host || !ws || !indptr_dev || !nnz_host || n <= 0 || d <= 0 || d > 8 || n > INT32_MAX)
         return -1;
     if (row_pos_dev && (row_first < 0 || row_last < row_first || row_last > n)) return -1;
+    MaternParams mp;
+    int mode;
+    if (int rc = matern_params(scale_host, d, nu, false, &mp, &mode)) return rc;
     cudaStream_t s = (cudaStream_t)stream;
     SparseWs w = carve_sparse(ws, n, d);
     SparseParams sp;
     CellGrid g;
-    if (int rc = sparse_prepare(points, n, d, scale_host, nu, tau, w, s, &sp, &g)) return rc;
+    if (int rc = sparse_prepare(points, n, d, scale_host, nu, tau, mp, w, s, &sp, &g)) return rc;
     sp.row_pos = row_pos_dev;
     sp.row_first = (int)row_first;
     sp.row_last = (int)row_last;
     const int N = (int)n;
-    launch_rows_mode(matern_mode_of(nu), 0, false, sp, g, w, nullptr, nullptr, nullptr, nullptr, s);
+    with_matern_mode(mode, [&](auto tag) {
+        launch_rows<decltype(tag)::value>(0, false, sp, g, w, nullptr, nullptr, nullptr, nullptr, s);
+    });
     GP_LAUNCH_CHECK();
     int nb = 0;
     unsigned long long total = 0;
@@ -817,9 +762,9 @@ int gp_matern_sparse_fill(const double* points, const double* points_host, int64
     if (!points || !points_host || !scale_host || !ws || !indptr_dev || !indices_dev || !data_dev || n <= 0 || d <= 0 || d > 8)
         return -1;
     if (row_pos_dev && (row_first < 0 || row_last < row_first || row_last > n)) return -1;
-    if (ddata_dev)
-        for (int k = 0; k < d; ++k)
-            if (scale_host[k] != scale_host[0]) return -4;
+    MaternParams mp;
+    int mode;
+    if (int rc = matern_params(scale_host, d, nu, ddata_dev != nullptr, &mp, &mode)) return rc;
     cudaStream_t s = (cudaStream_t)stream;
     SparseWs w = carve_sparse(ws, n, d);
     double bb[16];
@@ -829,12 +774,14 @@ int gp_matern_sparse_fill(const double* points, const double* points_host, int64
     GP_CUDA_CHECK(cudaStreamSynchronize(s));
     SparseParams sp;
     CellGrid g;
-    make_params(n, d, scale_host, nu, tau, bb, bb + 8, &sp, &g);
+    make_params(n, d, scale_host, nu, tau, mp, bb, bb + 8, &sp, &g);
     sp.row_pos = row_pos_dev;
     sp.row_first = (int)row_first;
     sp.row_last = (int)row_last;
     int ne = meta[0];
-    launch_rows_mode(matern_mode_of(nu), 1, ddata_dev != nullptr, sp, g, w, indptr_dev, indices_dev, data_dev, ddata_dev, s);
+    with_matern_mode(mode, [&](auto tag) {
+        launch_rows<decltype(tag)::value>(1, ddata_dev != nullptr, sp, g, w, indptr_dev, indices_dev, data_dev, ddata_dev, s);
+    });
     if (ne > 0) {
         if (ddata_dev) {
             // derivative values of the host-decided entries (any ulp-level value is fine here: only the pattern and
@@ -1120,21 +1067,6 @@ static void launch_blocks(int pass, bool with_dk, const SparseParams& sp, const 
     GP_COUNT(1);
 }
 
-static void launch_blocks_mode(int mode, int pass, bool with_dk, const SparseParams& sp, const CellGrid& g, const SparseWs& w,
-                               const double* pts, const int* order, const int* inv_order, int row_first, int nrows, int* nblk,
-                               unsigned long long* stats, const int64_t* bptr, int* bidx, double* bvals, double* bdvals,
-                               cudaStream_t s) {
-#define GP_BM(M) launch_blocks<M>(pass, with_dk, sp, g, w, pts, order, inv_order, row_first, nrows, nblk, stats, bptr, bidx, bvals, bdvals, s)
-    switch (mode) {
-        case MAT_05: GP_BM(MAT_05); break;
-        case MAT_15: GP_BM(MAT_15); break;
-        case MAT_25: GP_BM(MAT_25); break;
-        case MAT_GAUSS: GP_BM(MAT_GAUSS); break;
-        default: GP_BM(MAT_GENERAL); break;
-    }
-#undef GP_BM
-}
-
 extern "C" {
 
 // Pass 0 of the direct row-blocked generation for the operator rows [row_first, row_last) (row_first a multiple of 16;
@@ -1148,17 +1080,22 @@ int gp_matern_blocks_count(const double* points, int64_t n, int64_t d, const dou
     if (!points || !scale_host || !ws || !order_dev || !inv_order_dev || !nblk_dev || !stats_host || n <= 0 || d <= 0 || d > 8 ||
         n > INT32_MAX || row_first < 0 || row_last <= row_first || row_last > n || (row_first % BCSR_ROWS))
         return -1;
+    MaternParams mp;
+    int mode;
+    if (int rc = matern_params(scale_host, d, nu, false, &mp, &mode)) return rc;
     cudaStream_t s = (cudaStream_t)stream;
     SparseWs w = carve_sparse(ws, n, d);
     SparseParams sp;
     CellGrid g;
-    if (int rc = sparse_prepare(points, n, d, scale_host, nu, tau, w, s, &sp, &g)) return rc;
+    if (int rc = sparse_prepare(points, n, d, scale_host, nu, tau, mp, w, s, &sp, &g)) return rc;
     stats_host[0] = stats_host[1] = 0;
     if (!sp.quick) return 3;
     unsigned long long* stats = w.bbox_keys + 16;
     GP_CUDA_CHECK(cudaMemsetAsync(stats, 0, 2 * sizeof(unsigned long long), s));
-    launch_blocks_mode(matern_mode_of(nu), 0, false, sp, g, w, points, order_dev, inv_order_dev, (int)row_first,
-                       (int)(row_last - row_first), nblk_dev, stats, nullptr, nullptr, nullptr, nullptr, s);
+    with_matern_mode(mode, [&](auto tag) {
+        launch_blocks<decltype(tag)::value>(0, false, sp, g, w, points, order_dev, inv_order_dev, (int)row_first,
+                                            (int)(row_last - row_first), nblk_dev, stats, nullptr, nullptr, nullptr, nullptr, s);
+    });
     GP_LAUNCH_CHECK();
     unsigned long long h[2] = {0, 0};
     GP_CUDA_CHECK(cudaMemcpyAsync(h, stats, sizeof(h), cudaMemcpyDeviceToHost, s));
@@ -1175,9 +1112,9 @@ int gp_matern_blocks_fill(const double* points, int64_t n, int64_t d, const doub
     if (!points || !scale_host || !ws || !order_dev || !inv_order_dev || !bptr_dev || !bidx_dev || !bvals_dev || n <= 0 ||
         d <= 0 || d > 8 || row_first < 0 || row_last <= row_first || row_last > n || (row_first % BCSR_ROWS))
         return -1;
-    if (bdvals_dev)
-        for (int k = 0; k < d; ++k)
-            if (scale_host[k] != scale_host[0]) return -4;
+    MaternParams mp;
+    int mode;
+    if (int rc = matern_params(scale_host, d, nu, bdvals_dev != nullptr, &mp, &mode)) return rc;
     cudaStream_t s = (cudaStream_t)stream;
     SparseWs w = carve_sparse(ws, n, d);
     double bb[16];
@@ -1185,9 +1122,12 @@ int gp_matern_blocks_fill(const double* points, int64_t n, int64_t d, const doub
     GP_CUDA_CHECK(cudaStreamSynchronize(s));
     SparseParams sp;
     CellGrid g;
-    make_params(n, d, scale_host, nu, tau, bb, bb + 8, &sp, &g);
-    launch_blocks_mode(matern_mode_of(nu), 1, bdvals_dev != nullptr, sp, g, w, points, order_dev, inv_order_dev, (int)row_first,
-                       (int)(row_last - row_first), nullptr, nullptr, bptr_dev, bidx_dev, bvals_dev, bdvals_dev, s);
+    make_params(n, d, scale_host, nu, tau, mp, bb, bb + 8, &sp, &g);
+    with_matern_mode(mode, [&](auto tag) {
+        launch_blocks<decltype(tag)::value>(1, bdvals_dev != nullptr, sp, g, w, points, order_dev, inv_order_dev, (int)row_first,
+                                            (int)(row_last - row_first), nullptr, nullptr, bptr_dev, bidx_dev, bvals_dev,
+                                            bdvals_dev, s);
+    });
     GP_LAUNCH_CHECK();
     return 0;
 }

@@ -15,6 +15,9 @@
  *    log-determinant of the padded matrix restrict exactly to those of the n x n matrix.
  *  - return value: 0 ok; > 0 LAPACK-style info (1-based index of the first non-positive pivot, or the Lanczos /
  *    CG breakdown step); < 0 bad argument (-1..-99) or CUDA error (-1000 - cudaError).
+ *  - every entry point that takes a correlation scale (scale_host, d entries) and nu checks them before anything is
+ *    enqueued: -3 when a scale entry is not > 0 (NaN included); -4 when a d/d(rho) is requested, which needs an isotropic
+ *    scale, and the entries differ; -5 when nu takes the general (Bessel) branch and is not > 0.
  *  - nothing here allocates persistent device memory; the caller passes workspaces sized by the matching
  *    *_workspace_bytes query. Calls are stream-ordered and re-entrant per (device, stream).
  */
@@ -48,8 +51,8 @@ int gp_gemm_profile_read(double* ms_sum_host, double* ms_union_host, double* flo
  * ------------------------------------------------------------------------------------------------------- */
 
 /* K[i][j] = matern(||(p_i - p_j) / scale||, nu) into a padded buffer (ldk = npad; padding = identity).
- * dK (optional, may be NULL) receives dK/d(rho) for an isotropic scale rho = scale_host[0] (all entries of
- * scale_host must then be equal); its padding is zero. points: (n, d) row-major. */
+ * dK (optional, may be NULL) receives dK/d(rho) for an isotropic scale rho = scale_host[0]; its padding is zero.
+ * points: (n, d) row-major. */
 int gp_matern_dense(const double* points, int64_t n, int64_t d, const double* scale_host, double nu,
                     double* K, int64_t ldk, double* dK, void* stream);
 
@@ -340,9 +343,10 @@ int gp_eig_reduce(const double* lam, int64_t n, double eta, double* out, void* s
  * Work   : A, W (npad x npad scratch each; W may be NULL when flags & 3 == 0), potrf_ws, ws.
  * flags  : bit0 (1) tr Kn^-1 via ||inv(L)||_F^2       (enough for d/d eta)
  *          bit1 (2) full inverse: tr Kn^-1, tr Kn^-2  (needed for d/d rho and the Hessian traces)
- *          bit2 (4) d/d rho reductions, needs bit1 and points/d/scale_host/nu (dK/drho is re-evaluated on the fly)
+ *          bit2 (4) d/d rho reductions, needs bit1 and points/d/scale_host/nu (dK/drho is re-evaluated on the fly; -8
+ *                   otherwise); without it points, d, scale_host and nu are not read
  *          bit3 (8) third moments T3 = R^T Kn^-3 R from one more skinny solve batch (Hessian _direct_likelihood.py:163-270,
- *                   second eta-derivative _profile_likelihood.py:138-192); needs bit0 or bit1
+ *                   second eta-derivative _profile_likelihood.py:138-192); needs bit0 or bit1 (-9 otherwise)
  * Output : out (DEVICE, gp_loglik_out_len(p) doubles):
  *          out[0] logdet(K + eta I)   out[1] tr Kn^-1   out[2] tr Kn^-2   out[3] tr(Kn^-1 dK/drho)
  *          out[4] potrf info (0 = ok) out[5..7] reserved
