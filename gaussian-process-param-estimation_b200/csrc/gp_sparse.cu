@@ -1067,6 +1067,66 @@ static void launch_blocks(int pass, bool with_dk, const SparseParams& sp, const 
     GP_COUNT(1);
 }
 
+// Per-dimension derivative streams of a built row-blocked operator: stream k holds dK/d scale[k] at the positions of bvals and
+// 0 where bvals is 0 (K > tau > 0 on the pattern, so this is the pattern whichever path built the blocks). With u_k = Delta_k /
+// scale[k], x = ||u|| and g(x) = -x K'(x) (matern_value_drho with inv_rho = 1): dK/d scale[k] = g(x) u_k^2 / (x^2 scale[k]),
+// 0 at x = 0 - the formula of gp_loglik_dense_dscale. x is computed in scaled_distance_dim's arithmetic with block_entry's
+// (i <= j) ordering; g(x) is evaluated once per entry and all d streams are written from it. One warp per row block, one
+// lane per block-column; the 16-row loop is not unrolled, for the reason given at sparse_blocks_kernel's emit.
+template <int MODE, int DIM>
+__global__ void __launch_bounds__(128)
+bcsr_dscale_kernel(const int64_t* __restrict__ bptr, const int* __restrict__ bidx, const double* __restrict__ bvals, int rows,
+                   int row_first, int64_t stream_len, const int* __restrict__ order, const double* __restrict__ pts,
+                   SparseParams sp, double* __restrict__ dvals) {
+    __shared__ double rowp_s[4][BCSR_ROWS][8];
+    __shared__ int rowid_s[4][BCSR_ROWS];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const int rb = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (rb * BCSR_ROWS >= rows) return;
+    const int dd = DIM > 0 ? DIM : sp.d;
+    constexpr int PD = DIM > 0 ? DIM : 8;
+    double (*rowp)[8] = rowp_s[w];
+    int* rowid = rowid_s[w];
+    if (lane < BCSR_ROWS) {
+        const int r = rb * BCSR_ROWS + lane;
+        const int id = (r < rows) ? order[row_first + r] : -1;
+        rowid[lane] = id;
+        for (int k = 0; k < 8; ++k) rowp[lane][k] = (id >= 0 && k < dd) ? pts[(int64_t)id * dd + k] : 0.0;
+    }
+    __syncwarp();
+    const int64_t s1 = bptr[rb + 1];
+    for (int64_t slot = bptr[rb] + lane; slot < s1; slot += 32) {
+        const int j = order[bidx[slot]];
+        double pj[PD];
+#pragma unroll
+        for (int k = 0; k < PD; ++k) pj[k] = (k < dd) ? pts[(int64_t)j * dd + k] : 0.0;
+        const int64_t o = bval_group(slot);
+#pragma unroll 1
+        for (int r = 0; r < BCSR_ROWS; ++r) {
+            const int64_t pos = bval_pos(o, r);
+            double u2[PD];
+            double s = 0.0, g = 0.0;
+#pragma unroll
+            for (int k = 0; k < PD; ++k) u2[k] = 0.0;
+            if (bvals[pos] != 0.0) {
+                const bool i_first = rowid[r] <= j;
+#pragma unroll
+                for (int k = 0; k < PD; ++k)
+                    if (k < dd) {
+                        const double t = (i_first ? rowp[r][k] - pj[k] : pj[k] - rowp[r][k]) / sp.scale[k];
+                        u2[k] = t * t;
+                        s += u2[k];
+                    }
+                double val;
+                matern_value_drho<MODE>(sqrt(s), sp.mp, &val, &g);
+            }
+#pragma unroll
+            for (int k = 0; k < PD; ++k)
+                if (k < dd) dvals[k * stream_len + pos] = (s > 0.0) ? g * (u2[k] / s) * sp.mp.inv_scale[k] : 0.0;
+        }
+    }
+}
+
 extern "C" {
 
 // Pass 0 of the direct row-blocked generation for the operator rows [row_first, row_last) (row_first a multiple of 16;
@@ -1128,6 +1188,38 @@ int gp_matern_blocks_fill(const double* points, int64_t n, int64_t d, const doub
                                             (int)(row_last - row_first), nullptr, nullptr, bptr_dev, bidx_dev, bvals_dev,
                                             bdvals_dev, s);
     });
+    GP_LAUNCH_CHECK();
+    return 0;
+}
+
+// d streams of 16 * nblocks doubles (stream k at dvals_dev + 16 * nblocks * k): dK/d scale[k] on the row blocks of the
+// operator rows [row_first, row_first + rows) (bidx: operator positions, before gp_slab_encode_columns). Any scale with
+// positive entries is accepted (never -4).
+int gp_bcsr_dscale_fill(const int64_t* bptr_dev, const int* bidx_dev, const double* bvals_dev, int64_t nblocks, int64_t row_first,
+                        int64_t rows, const int* order_dev, const double* points, int64_t n, int64_t d, const double* scale_host,
+                        double nu, double* dvals_dev, void* stream) {
+    if (!bptr_dev || !bidx_dev || !bvals_dev || !order_dev || !points || !scale_host || !dvals_dev || d < 1 || d > 8 || n <= 0 ||
+        n > INT32_MAX || nblocks < 0 || row_first < 0 || (row_first % BCSR_ROWS) || rows <= 0 || row_first + rows > n)
+        return -1;
+    SparseParams sp{};
+    int mode;
+    if (int rc = matern_params(scale_host, d, nu, false, &sp.mp, &mode)) return rc;
+    sp.mp.inv_rho = 1.0;
+    sp.d = (int)d;
+    for (int k = 0; k < d; ++k) sp.scale[k] = scale_host[k];
+    if (nblocks == 0) return 0;
+    cudaStream_t s = (cudaStream_t)stream;
+    const unsigned blocks = (unsigned)(((rows + BCSR_ROWS - 1) / BCSR_ROWS + 3) / 4);
+    with_matern_mode(mode, [&](auto tag) {
+        constexpr int MODE = decltype(tag)::value;
+        if (d == 2)
+            bcsr_dscale_kernel<MODE, 2><<<blocks, 128, 0, s>>>(bptr_dev, bidx_dev, bvals_dev, (int)rows, (int)row_first,
+                                                               16 * nblocks, order_dev, points, sp, dvals_dev);
+        else
+            bcsr_dscale_kernel<MODE, 0><<<blocks, 128, 0, s>>>(bptr_dev, bidx_dev, bvals_dev, (int)rows, (int)row_first,
+                                                               16 * nblocks, order_dev, points, sp, dvals_dev);
+    });
+    GP_COUNT(1);
     GP_LAUNCH_CHECK();
     return 0;
 }

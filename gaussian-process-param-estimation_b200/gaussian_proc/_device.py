@@ -88,6 +88,7 @@ SIGNATURES = {
     'gp_gather_rows': (_int, [_vp, _vp, _i64, _i64, _vp, _vp]),
     'gp_matern_blocks_count': (_int, [_vp, _i64, _i64, _vp, _f64, _f64, _vp, _vp, _vp, _i64, _i64, _vp, _vp, _vp]),
     'gp_matern_blocks_fill': (_int, [_vp, _i64, _i64, _vp, _f64, _f64, _vp, _vp, _vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
+    'gp_bcsr_dscale_fill': (_int, [_vp, _vp, _vp, _i64, _i64, _i64, _vp, _vp, _i64, _i64, _vp, _f64, _vp, _vp]),
     'gp_peer_handle_bytes': (_i64, []),
     'gp_peer_create': (_vp, [_i64, _i64, _i64]),
     'gp_peer_handle': (_int, [_vp, _vp]),

@@ -92,7 +92,7 @@ def evaluate_async(z, X, K_mixed, eta, traceinv=False, inverse=False, drho=False
     if K_mixed.sparse:
         # sparse K: batched CG solves + skinny Gram matrices + the engine's stochastic traces (synchronous)
         out = K_mixed.engine.fused(float(eta), X, z, traceinv=traceinv or inverse or cubic, drho=drho, cubic=cubic)
-        return (out, n, m, float(eta), -1 if cubic else -2, None, None)
+        return (out, n, m, float(eta), -1 if cubic else -2, None, K_mixed.engine.last_dscale)
     flags = 0
     if traceinv:
         flags |= FLAG_TRACEINV
@@ -117,8 +117,8 @@ def finish(handle):
     """Waits for the evaluation's stream, reads out[] back (one small D2H) and does the host algebra; raises
     numpy.linalg.LinAlgError if K + eta I was not positive definite."""
     out, n, m, eta, flags, stream, dscale = handle
-    if stream is None:
-        return FusedQuantities(out, n, m, eta, flags)      # sparse engine: already complete, breakdowns raised there
+    if stream is None:       # sparse engine: already complete, breakdowns raised there; dscale a host array
+        return FusedQuantities(out, n, m, eta, flags, dscale)
     stream.synchronize()
     q = FusedQuantities(out.cpu().numpy(), n, m, eta, flags, None if dscale is None else dscale.cpu().numpy())
     if q.info != 0:

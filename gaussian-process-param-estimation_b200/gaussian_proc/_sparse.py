@@ -65,6 +65,7 @@ class DeviceCSR(object):
         self.kernel_threshold = kernel_threshold
         self.order = order      # optional spatially local ordering of the rows (device int32), see SparseEngine
         self.sorted_rows = bool(sorted_rows)
+        self.dscale = None      # (device points, scale, nu): dK/d scale[k] per dimension, built with the row blocks
 
     def canonicalize(self):
         """sort every row by column index, in place (no-op when already sorted)"""
@@ -121,6 +122,8 @@ class DeviceRowBlocks(object):
         self.row_slab = row_slab
         self.sorted_rows = True
         self.encoded = None                    # set by the row-slab engine once the columns carry (owner, local row)
+        self.dscale = None                     # (device points, scale, nu): dK/d scale[k] per dimension (anisotropic scale)
+        self.bdvals_dims = None                # their d streams, computed by the first engine (before any column encoding)
 
     @property
     def shape(self):
@@ -186,15 +189,20 @@ def generate_sparse_correlation(points, correlation_scale, nu, density, verbose=
     DeviceCSR when ``device``). ``sort_rows``: canonical (column-sorted) rows right away; default: yes for the SciPy
     result, deferred (DeviceCSR.canonicalize) for a device handle.
     ``row_slab`` = (rank, world) (device handle only): generate only this rank's slab of rows of the spatially ordered
-    operator (gaussian_proc/_slab.py); the other rows of the handle stay empty."""
+    operator (gaussian_proc/_slab.py); the other rows of the handle stay empty.
+    ``with_derivative``: dK/drho on the pattern (``ddata``) for an isotropic scale; for an anisotropic one the device handle
+    records (device points, scale, nu) instead and the engine builds dK/d scale[k] per dimension with its row blocks (the
+    SciPy result cannot carry them: ValueError)."""
     sort_rows = (not device) if sort_rows is None else bool(sort_rows)
     torch = dev.require_cuda()
     points = numpy.ascontiguousarray(points, dtype=numpy.float64)
     scale = dev.host_f64(correlation_scale)
     n, d = points.shape
     tau = estimate_kernel_threshold(n, d, density, scale, nu) if kernel_threshold is None else float(kernel_threshold)
-    if with_derivative and not numpy.all(scale == scale[0]):
-        raise ValueError('d/d(correlation_scale) is defined for an isotropic correlation_scale.')
+    per_dim = with_derivative and not numpy.all(scale == scale[0])
+    if per_dim and not device:
+        raise ValueError('d/d(correlation_scale) of an anisotropic correlation_scale needs device=True (the derivatives '
+                         'are carried by the device operator).')
     if row_slab is not None and not device:
         raise ValueError('row_slab needs device=True (a slab is not a complete matrix).')
     s = dev.stream_ptr()
@@ -212,12 +220,14 @@ def generate_sparse_correlation(points, correlation_scale, nu, density, verbose=
                                      _p(indptr), ctypes.byref(nnz), *rows, s), 'gp_matern_sparse_count')
     indices = torch.empty(nnz.value, dtype=torch.int32, device='cuda')
     data = torch.empty(nnz.value, dtype=torch.float64, device='cuda')
-    ddata = torch.empty(nnz.value, dtype=torch.float64, device='cuda') if with_derivative else None
+    ddata = torch.empty(nnz.value, dtype=torch.float64, device='cuda') if with_derivative and not per_dim else None
     check(lib.gp_matern_sparse_fill(_p(dpts), dev.host_ptr(points), n, d, dev.host_ptr(scale), float(nu), tau, _p(ws),
                                     _p(indptr), _p(indices), _p(data), _p(ddata) if ddata is not None else None,
                                     1 if sort_rows else 0, *rows, s), 'gp_matern_sparse_fill')
     K = DeviceCSR(n, indptr, indices, data, ddata, kernel_threshold=tau, order=order, sorted_rows=sort_rows)
     K.inv_order = pos
+    if per_dim:
+        K.dscale = (dpts, scale, float(nu))
     if row_slab is not None:
         K.row_slab = (rank, world, first, last)       # only these rows of the ordered operator are present
     if verbose:
@@ -232,14 +242,14 @@ def generate_sparse_operator(points, correlation_scale, nu, density, with_deriva
     the row blocks are generated directly from the cell lists (csrc/gp_sparse.cu, sparse_blocks_kernel; same kernel
     arithmetic and pattern rule, no CSR in between), about half the time of CSR generation + block build. Falls back to that
     path (returns a DeviceCSR) for a matrix with entries inside the 8-ulp borderline band of the threshold, which the
-    reference's rule decides in host arithmetic. ``row_slab`` = (rank, world): only this rank's slab (gaussian_proc/_slab.py)."""
+    reference's rule decides in host arithmetic. ``row_slab`` = (rank, world): only this rank's slab (gaussian_proc/_slab.py).
+    ``with_derivative`` with an anisotropic scale: per-dimension derivatives, as in generate_sparse_correlation."""
     torch = dev.require_cuda()
     points = numpy.ascontiguousarray(points, dtype=numpy.float64)
     scale = dev.host_f64(correlation_scale)
     n, d = points.shape
     tau = estimate_kernel_threshold(n, d, density, scale, nu) if kernel_threshold is None else float(kernel_threshold)
-    if with_derivative and not numpy.all(scale == scale[0]):
-        raise ValueError('d/d(correlation_scale) is defined for an isotropic correlation_scale.')
+    per_dim = with_derivative and not numpy.all(scale == scale[0])
     s = dev.stream_ptr()
     dpts, order, pos = _device_points(points)
     first, last, slab = 0, n, None
@@ -263,11 +273,13 @@ def generate_sparse_operator(points, correlation_scale, nu, density, with_deriva
     total = int(bptr[-1].item())
     bidx = torch.empty(total, dtype=torch.int32, device='cuda')
     bvals = torch.empty(total * 16, dtype=torch.float64, device='cuda')
-    bdvals = torch.empty(total * 16, dtype=torch.float64, device='cuda') if with_derivative else None
+    bdvals = torch.empty(total * 16, dtype=torch.float64, device='cuda') if with_derivative and not per_dim else None
     check(lib.gp_matern_blocks_fill(_p(dpts), n, d, dev.host_ptr(scale), float(nu), tau, _p(ws), _p(order), _p(pos), first, last,
                                     _p(bptr), _p(bidx), _p(bvals), _p(bdvals) if bdvals is not None else None, s),
           'gp_matern_blocks_fill')
     K = DeviceRowBlocks(n, bptr, bidx, bvals, bdvals, order, pos, stats[0], tau, first, last, row_slab=slab)
+    if per_dim:
+        K.dscale = (dpts, scale, float(nu))
     if verbose:
         print('Generated sparse correlation operator using kernel threshold: %0.4f and sparse density: %0.2e.'
               % (tau, K.nnz / float(n) / float(last - first)))
@@ -366,6 +378,8 @@ class SparseEngine(object):
         self.order = self.inv_order = None
         self.R = 1                 # rows per block of the operator in use: 16 row-blocked, 1 plain CSR
         self.blocked = None
+        self.dims = None           # (d, 16 * blocks) per-dimension derivative streams of an anisotropic scale
+        self.last_dscale = None    # rows [tr(Kn^-1 dK_k), Q_k] of the last fused call (layout of DenseEngine.last_dscale)
         if K.order is not None:
             self._build_blocked(K)
 
@@ -410,6 +424,19 @@ class SparseEngine(object):
             if self.peer is not None and getattr(K, 'row_slab', None) is None:
                 share = self.world     # a handle with every row, of which this slab is built
         total = bidx.numel()
+        if K.dscale is not None:
+            # dK/d scale[k] on the blocks just built or generated, while the columns are still operator positions; a
+            # generated handle keeps them, so a second engine on it (its columns possibly encoded since) reuses them
+            dims = K.bdvals_dims if isinstance(K, DeviceRowBlocks) else None
+            if dims is None:
+                dpts, scale, nu = K.dscale
+                d = scale.size
+                dims = torch.empty((d, total * R), dtype=torch.float64, device='cuda')
+                check(lib.gp_bcsr_dscale_fill(_p(bptr), _p(bidx), _p(bvals), total, r0, self.rows, _p(K.order), _p(dpts), n, d,
+                                              dev.host_ptr(scale), nu, _p(dims), s), 'gp_bcsr_dscale_fill')
+                if isinstance(K, DeviceRowBlocks):
+                    K.bdvals_dims = dims
+            self.dims = dims
         if self.peer is not None:
             if encoded is None:
                 halo = (ctypes.c_int64 * 2)()   # block-columns whose row of X lives on another rank, and the distinct rows among them
@@ -444,22 +471,48 @@ class SparseEngine(object):
         arena = self.peer_side if side else self.peer
         return arena.ctx if arena is not None else None
 
-    def spmm(self, eta, X_dev, derivative=False):
-        """(K + eta I) X, or (dK/drho + eta I) X with ``derivative``, in OPERATOR space (rows in self.order when the
-        operator is permuted)"""
+    def spmm(self, eta, X_dev, derivative=False, dim=None):
+        """(K + eta I) X, (dK/drho + eta I) X with ``derivative``, or (dK/d scale[dim] + eta I) X with ``dim`` (an
+        anisotropic scale's per-dimension streams), in OPERATOR space (rows in self.order when the operator is permuted)"""
         torch = dev.torch
         B = X_dev.shape[1]
         X_dev = X_dev.contiguous()
         Y = torch.empty_like(X_dev)
+        if dim is not None:
+            self._derivative_streams(required=True)
         if self.blocked is not None:
             bptr, bidx, bvals, bdvals = self.blocked
-            check(lib.gp_bcsr_spmm(self._peer_ctx(), _p(bptr), _p(bidx), _p(bdvals if derivative else bvals), self.rows,
+            vals = self.dims[dim] if dim is not None else (bdvals if derivative else bvals)
+            check(lib.gp_bcsr_spmm(self._peer_ctx(), _p(bptr), _p(bidx), _p(vals), self.rows,
                                    float(eta), _p(X_dev), B, _p(Y), dev.stream_ptr()), 'gp_bcsr_spmm')
         else:
             K = self.K
             check(lib.gp_csr_spmm(_p(K.indptr), _p(K.indices), _p(K.ddata if derivative else K.data), self.n, float(eta),
                                   _p(X_dev), B, _p(Y), dev.stream_ptr()), 'gp_csr_spmm')
         return Y
+
+    def _derivative_streams(self, required=False):
+        """number of derivative operators K carries: 1 (dK/drho of an isotropic scale, K.ddata), d (dK/d scale[k] of an
+        anisotropic one, self.dims) or 0; ``required``: ValueError instead of 0"""
+        if self.K.dscale is not None:
+            if self.dims is not None:
+                return self.dims.shape[0]
+            if required:
+                raise ValueError('d/d(correlation_scale) per dimension needs the spatially ordered device operator of '
+                                 'generate_sparse_operator / generate_sparse_correlation(..., device=True); a plain CSR '
+                                 'or a SciPy matrix cannot carry it.')
+            return 0
+        if self.K.ddata is None:
+            if required:
+                raise ValueError('d/d(correlation_scale) needs a DeviceCSR generated with with_derivative=True')
+            return 0
+        return 1
+
+    def _dk(self, X_dev, k):
+        """dK_k X: the derivative operator k of _derivative_streams (k = 0 alone: dK/drho)"""
+        if self.dims is not None:
+            return self.spmm(0.0, X_dev, dim=k)
+        return self.spmm(0.0, X_dev, derivative=True)
 
     def to_op(self, X_dev):
         """this engine's rows, in operator order, of an (n x B) block given in the caller's row order"""
@@ -537,7 +590,7 @@ class SparseEngine(object):
         if ('probes', first, B) in self._krylov and bool(self.opt.get('shift_reuse', True)):
             return                                 # already served by a kept Lanczos run
         m = int(self.opt['lanczos_degree'])
-        with_dk = self.K.ddata is not None and bool(self.opt.get('reuse_lanczos', True))
+        with_dk = self._derivative_streams() > 0 and bool(self.opt.get('reuse_lanczos', True))
         if not hasattr(self, '_side_stream'):
             self._side_stream = torch.cuda.Stream()
         # every buffer is allocated on the main stream; the side stream only runs kernels on them
@@ -592,28 +645,30 @@ class SparseEngine(object):
     def _new_basis(self, m, B):
         return dev.torch.empty((m, self.rows, B), dtype=dev.torch.float64, device='cuda')
 
-    def _slq_samples(self, eta, first, B, with_dk=False):
-        """Per-probe quadratures [log, 1/x, 1/x^2] * n for probes first .. first+B-1. With ``with_dk`` a fourth column:
-        the Hutchinson sample v^T Kn^-1 dK v with Kn^-1 v taken from the SAME Lanczos run (x = ||v|| Q T^-1 e_1, the
-        Lanczos form of CG) when its residual beta_k |y_k| meets the CG tolerance, else from a batched CG solve."""
+    def _slq_samples(self, eta, first, B, with_dk=0):
+        """Per-probe quadratures [log, 1/x, 1/x^2] * n for probes first .. first+B-1. With ``with_dk`` derivative
+        operators (_derivative_streams) one more column each: the Hutchinson sample v^T Kn^-1 dK_k v with Kn^-1 v taken
+        from the SAME Lanczos run (x = ||v|| Q T^-1 e_1, the Lanczos form of CG) when its residual beta_k |y_k| meets the
+        CG tolerance, else from a batched CG solve."""
         torch = dev.torch
         m = int(self.opt['lanczos_degree'])
-        ent, shift = self._probe_krylov(eta, first, B, with_dk)
+        nd = int(with_dk)
+        ent, shift = self._probe_krylov(eta, first, B, nd > 0)
         a, b = ent['a'] + shift, ent['b']
-        out = numpy.empty((B, 4 if with_dk else 3))
+        out = numpy.empty((B, 3 + nd))
         vnorm = numpy.sqrt(float(self.n))          # Rademacher probes
-        quad, tmin, coef, res = lanczos_block_quadrature(a, b, vnorm if with_dk else None)
+        quad, tmin, coef, res = lanczos_block_quadrature(a, b, vnorm if nd else None)
         if not (tmin.min() > 0):
             raise numpy.linalg.LinAlgError(
                 'K + eta*I (eta=%g) is not positive definite: Lanczos found a Ritz value %.3e. The thresholded '
                 'Matern matrix is indefinite; use a larger eta (reference: _generate_sparse_correlation.pyx:516-523).'
                 % (eta, tmin.min()))
         out[:, :3] = quad * self.n
-        resid = float(res.max()) if with_dk else 0.0
-        if with_dk:
+        resid = float(res.max()) if nd else 0.0
+        if nd:
             V = ent['V'] if ent['V'] is not None else self.probes(first, B)
             if ent['Wd'] is None:
-                ent['Wd'] = self.spmm(0.0, V, derivative=True)      # dK v does not depend on eta either
+                ent['Wd'] = [self._dk(V, k) for k in range(nd)]      # dK_k v does not depend on eta either
             if resid <= float(self.opt['cg_tol']):
                 U = torch.empty_like(V)
                 cd = torch.from_numpy(coef).cuda()
@@ -623,7 +678,8 @@ class SparseEngine(object):
             else:
                 U = self.solve_dev(eta, V.clone())
                 self.last_dk_solver = 'cg'
-            out[:, 3] = self.col_dot(U, ent['Wd'])
+            for k in range(nd):
+                out[:, 3 + k] = self.col_dot(U, ent['Wd'][k])
         return out
 
     def solve_rhs_block(self, eta, Rop, key, refs=None):
@@ -752,16 +808,16 @@ class SparseEngine(object):
         return N, mean, numpy.sqrt(var), bool(cnt[1] > 0)
 
     def _slq(self, eta):
-        """SLQ estimates [logdet, tr Kn^-1, tr Kn^-2] at eta (cached). When the matrix carries dK/drho the same Lanczos
-        runs also yield the Hutchinson samples of tr(Kn^-1 dK) (kept for traceinv_dK; they do not influence the
-        stopping decision here)."""
+        """SLQ estimates [logdet, tr Kn^-1, tr Kn^-2] at eta (cached). When the matrix carries dK/drho (or dK/d scale[k]
+        per dimension) the same Lanczos runs also yield the Hutchinson samples of tr(Kn^-1 dK_k) (kept for traceinv_dK;
+        they do not influence the stopping decision here)."""
         key = float(eta)
         if key not in self._slq_cache:
-            with_dk = self.K.ddata is not None and bool(self.opt.get('reuse_lanczos', True))
+            nd = self._derivative_streams() if bool(self.opt.get('reuse_lanczos', True)) else 0
             mean, half, N, state = self._run_estimator(
-                lambda first, width: self._slq_samples(eta, first, width, with_dk), 4 if with_dk else 3, check_cols=3)
+                lambda first, width: self._slq_samples(eta, first, width, nd), 3 + nd, check_cols=3)
             self._slq_cache = {key: (mean[:3], half[:3], N)}
-            self._dk_state = {key: (state[0][:, 3:4].copy(), state[1])} if with_dk else {}
+            self._dk_state = {key: (state[0][:, 3:].copy(), state[1])} if nd else {}
         mean, half, N = self._slq_cache[key]
         self.last_info = {'num_samples': N, 'half_width': half, 'confidence_level': self.opt['confidence_level'],
                           'lanczos_degree': self.opt['lanczos_degree']}
@@ -785,26 +841,27 @@ class SparseEngine(object):
         self.last_info = {'num_samples': N, 'half_width': half}
         return float(mean[0])
 
-    def traceinv_dK(self, eta):
-        """Hutchinson estimate of tr((K + eta I)^-1 dK/d rho): mean over probes of (Kn^-1 v)^T (dK v). Samples that the
-        SLQ run at this eta already produced (same probe ids, Kn^-1 v from its Lanczos basis) are used first; further
-        rounds, if its own stopping rule asks for them, go through the same kept-Lanczos path (CG when the Lanczos
-        residual misses the tolerance or with reuse_lanczos=False)."""
-        if self.K.ddata is None:
-            raise ValueError('needs a DeviceCSR generated with with_derivative=True')
+    def _dk_samples(self, eta, first, width):
+        """Hutchinson samples (Kn^-1 v)^T (dK_k v) of probes first .. first+width-1, one column per derivative operator"""
+        nd = self._derivative_streams(required=True)
+        if bool(self.opt.get('reuse_lanczos', True)):
+            # through the (kept, shift-invariant) Lanczos run of this probe block: reused for every later eta
+            return self._slq_samples(eta, first, width, nd)[:, 3:]
+        V = self.probes(first, width)
+        U = self.solve_dev(eta, V.clone())
+        return numpy.stack([self.col_dot(U, self._dk(V, k)) for k in range(nd)], axis=1)
 
-        def fn(first, width):
-            if bool(self.opt.get('reuse_lanczos', True)):
-                # through the (kept, shift-invariant) Lanczos run of this probe block: reused for every later eta
-                return self._slq_samples(eta, first, width, True)[:, 3:4]
-            V = self.probes(first, width)
-            U = self.solve_dev(eta, V.clone())
-            Wd = self.spmm(0.0, V, derivative=True)
-            return self.col_dot(U, Wd).reshape(-1, 1)
+    def traceinv_dK(self, eta):
+        """Hutchinson estimate of tr((K + eta I)^-1 dK/d rho): mean over probes of (Kn^-1 v)^T (dK v); for an anisotropic
+        scale the array of tr(Kn^-1 dK/d scale[k]), k < d, from the same probes. Samples that the SLQ run at this eta
+        already produced (same probe ids, Kn^-1 v from its Lanczos basis) are used first; further rounds, if its own
+        stopping rule (on every column) asks for them, go through the same kept-Lanczos path (CG when the Lanczos
+        residual misses the tolerance or with reuse_lanczos=False)."""
+        nd = self._derivative_streams(required=True)
         state = getattr(self, '_dk_state', {}).get(float(eta))
-        mean, half, N, _ = self._run_estimator(fn, 1, state=state)
+        mean, half, N, _ = self._run_estimator(lambda first, width: self._dk_samples(eta, first, width), nd, state=state)
         self.last_info = {'num_samples': N, 'half_width': half}
-        return float(mean[0])
+        return mean.copy() if self.dims is not None else float(mean[0])
 
     # ---- CG ------------------------------------------------------------------------------------------------------
     def col_dot(self, X, Y):
@@ -932,7 +989,8 @@ class SparseEngine(object):
         (csrc/gp_loglik.cu): [logdet Kn, tr Kn^-1, tr Kn^-2, tr(Kn^-1 dK/drho), info, -, -, -, G, H, Q] with R = [X z],
         S = Kn^-1 R (batched CG, the reference's tol 1e-6), G = R^T S, H = S^T S, Q = S^T dK S; the traces are the
         stochastic estimates (SLQ / Hutchinson) of this engine. Reference formulas: _direct_likelihood.py:113-150,
-        _profile_likelihood.py:104-130."""
+        _profile_likelihood.py:104-130. For an anisotropic scale the d/d scale[k] pieces are the rows
+        [tr(Kn^-1 dK_k), Q_k] of self.last_dscale (out[3] and Q stay 0), as DenseEngine does."""
         n, m = X.shape
         p = m + 1
         key = (dev.host_key(X), dev.host_key(z))          # ONE content fingerprint per evaluation
@@ -943,11 +1001,18 @@ class SparseEngine(object):
         out = numpy.zeros(8 + 4 * p * p)
         out[8:8 + p * p] = self.gram(Rd, S)[:p, :p].ravel()
         out[8 + p * p:8 + 2 * p * p] = self.gram(S, S)[:p, :p].ravel()
+        self.last_dscale = None
+        dscale = None
         if drho:
-            if self.K.ddata is None:
-                raise ValueError('d/d(correlation_scale) needs a DeviceCSR generated with with_derivative=True')
-            D = self.spmm(0.0, S, derivative=True)
-            out[8 + 2 * p * p:8 + 3 * p * p] = self.gram(S, D)[:p, :p].ravel()
+            nd = self._derivative_streams(required=True)
+            if self.dims is not None:
+                # anisotropic scale: rows [tr(Kn^-1 dK_k), Q_k = S^T dK_k S] per dimension, as DenseEngine.last_dscale
+                dscale = numpy.zeros((nd, 1 + p * p))
+                for k in range(nd):
+                    dscale[k, 1:] = self.gram(S, self._dk(S, k))[:p, :p].ravel()
+            else:
+                D = self.spmm(0.0, S, derivative=True)
+                out[8 + 2 * p * p:8 + 3 * p * p] = self.gram(S, D)[:p, :p].ravel()
         if cubic:
             # third moments T3 = S^T Kn^-1 S (Hessian / second eta-derivative): one more batched CG on S
             V2 = self.solve_dev(eta, S.clone())
@@ -957,7 +1022,11 @@ class SparseEngine(object):
             out[1] = self.traceinv(eta)
             out[2] = self.traceinv(eta, exponent=2)
         if drho:
-            out[3] = self.traceinv_dK(eta)
+            if dscale is not None:
+                dscale[:, 0] = self.traceinv_dK(eta)
+                self.last_dscale = dscale
+            else:
+                out[3] = self.traceinv_dK(eta)
         return out
 
     def trace_K(self):

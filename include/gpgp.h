@@ -273,6 +273,16 @@ int gp_matern_blocks_count(const double* points, int64_t n, int64_t d, const dou
 int gp_matern_blocks_fill(const double* points, int64_t n, int64_t d, const double* scale_host, double nu, double tau, void* ws,
                           const int* order_dev, const int* inv_order_dev, int64_t row_first, int64_t row_last,
                           const int64_t* bptr_dev, int* bidx_dev, double* bvals_dev, double* bdvals_dev, void* stream);
+/* Per-dimension derivative streams of a built row-blocked operator (either build path): for the operator rows
+ * [row_first, row_first + rows) (row_first a multiple of 16) with blocks bptr / bidx (operator positions, not slab-encoded) /
+ * bvals of nblocks block-columns, writes d streams of 16 * nblocks doubles, stream k at dvals_dev + 16 * nblocks * k:
+ * dK/d scale[k] in the fragment order of bvals, zero wherever bvals is zero. Operator row r is point order_dev[r]; points is
+ * the device (n x d) array. dK/d scale[k] = g(x) u_k^2 / (x^2 scale[k]) with u_k = Delta_k / scale[k], x = ||u||,
+ * g(x) = -x K'(x); 0 at x = 0 (as gp_loglik_dense_dscale). The scale may be anisotropic (never -4); -1 for a null pointer,
+ * d outside [1, 8] or a row_first that is not a multiple of 16. */
+int gp_bcsr_dscale_fill(const int64_t* bptr_dev, const int* bidx_dev, const double* bvals_dev, int64_t nblocks, int64_t row_first,
+                        int64_t rows, const int* order_dev, const double* points, int64_t n, int64_t d, const double* scale_host,
+                        double nu, double* dvals_dev, void* stream);
 
 /* ---- row-slab sparse operator on several GPUs (csrc/gp_peer.cu, gp_sparse_la.cu) ------------------------------------------
  * One process per GPU. The reference evaluates one sparse likelihood on one host (imate SLQ + scipy CG over the whole matrix,

@@ -1,5 +1,7 @@
 """Developer check (torchrun, one rank per GPU): the row-slab sparse engine (gaussian_proc/_slab.py) against the single-GPU
-engine on the same matrix: peer all-reduce, SpMM, CG, then the whole loglik + gradient; timing of a new-rho evaluation."""
+engine on the same matrix: peer all-reduce, SpMM, CG, then the whole loglik + gradient; timing of a new-rho evaluation.
+Arguments: [n] [aniso]. With `aniso` the run compares the per-dimension gradient of an anisotropic scale after the
+operator pieces and stops there."""
 import ctypes, json, os, sys, time
 import numpy
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), '..', 'gaussian-process-param-estimation_b200'))
@@ -71,6 +73,27 @@ out['fused_head'] = [f1[:4].tolist(), f2[:4].tolist()]
 out['peer_error_after'] = lib.gp_peer_error(slab.peer.ctx, dev.stream_ptr())
 if rank == 0:
     print(json.dumps(out), flush=True)
+
+if len(sys.argv) > 2 and sys.argv[2] == 'aniso':
+    # ---- anisotropic scale: the per-dimension gradient (d/d scale[k]) on row slabs against one GPU, then stop
+    from gaussian_proc._mixed_correlation import MixedCorrelation
+    from gaussian_proc._likelihood import ProfileLikelihood
+    Ka = generate_sparse_correlation(pts, numpy.array([rho, 1.6 * rho]), 0.5, dens, device=True, with_derivative=True)
+    Ms = MixedCorrelation(Ka, imate_method='slq', imate_options=dict(opts, row_slabs=True))
+    Mo = MixedCorrelation(Ka, imate_method='slq', imate_options=dict(opts, overlap=False))
+    gs = ProfileLikelihood.log_likelihood_and_gradient(z, X, Ms, 10.0)
+    go = ProfileLikelihood.log_likelihood_and_gradient(z, X, Mo, 10.0)
+    rel = lambda a, b: float(numpy.max(numpy.abs(numpy.asarray(a) - b)) / numpy.max(numpy.abs(b)))   # noqa: E731
+    an = {'grad': [gs[0], gs[1], list(gs[2])], 'grad_one_gpu': [go[0], go[1], list(go[2])],
+          'grad_rel_diff': max(rel(gs[0], go[0]), rel(gs[1], go[1]), rel(gs[2], go[2])),
+          'dscale_rel_diff': rel(Ms.engine.last_dscale, Mo.engine.last_dscale),
+          'peer_error': lib.gp_peer_error(Ms.engine.peer.ctx, dev.stream_ptr())}
+    if rank == 0:
+        print(json.dumps({'aniso': an}), flush=True)
+    if world > 1:
+        dist.barrier()
+        dist.destroy_process_group()
+    sys.exit(0)
 
 # ---- 3. timing: fresh operator + evaluation (a new-rho step of an optimiser), slabs against one GPU
 def evaluate(cls, phases=None):
